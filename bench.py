@@ -57,7 +57,12 @@ def parse():
     ap.add_argument("--no-gpu-baseline", action="store_true", help="skip the torch-eager CUDA baseline legs")
     ap.add_argument("--no-families", action="store_true", help="skip the per-kernel-family roofline pass")
     ap.add_argument("--no-graphs", action="store_true", help="issue every kernel from the host instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed step returned (logits, loss, OFF-parameter "
+                         "gradients) as DIR/<name>.npy in float32, to compare two builds output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if a.config == 4:
         a.variant = a.variant or "rgb"
@@ -80,6 +85,26 @@ def peaks():
             return json.load(f), "measured"
     except Exception:
         return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}, "fallback"
+
+
+# element data of one --dump-outputs directory; the .npy headers come on top and the files stay under 64 MB in all
+DUMP_DATA_BYTES = 60_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as ``out_dir/<name>.npy`` in float32.  Smaller arrays are written whole first; an array larger
+    than its share of what is left of DUMP_DATA_BYTES is replaced by a fixed seeded sample of its flattened elements
+    (the same indices for the same shapes, so two runs stay comparable element for element)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left, n_left = DUMP_DATA_BYTES // 4, len(arrays)
+    for name, a in sorted(arrays.items(), key=lambda kv: kv[1].size):
+        a = np.asarray(a, dtype=np.float32)
+        share = left // n_left
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left, n_left = left - a.size, n_left - 1
 
 
 def workload(args):
@@ -389,11 +414,13 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=dev)
     B, Lg = args.batch, args.length
     graphs = not args.no_graphs
+    # the initial weights, the taps and the per-step dropout seeds all follow from this seed: the same arguments give
+    # the same inputs in every run
+    torch.manual_seed(1234 + rank)
     net = OFFSubNetwork(B, Lg, args.variant, precision=args.precision, device=dev, use_graphs=graphs).train()
     eng = net.engine
     dp = DataParallelOFF(eng, use_graphs=graphs)
     dp.broadcast_parameters()
-    torch.manual_seed(1234 + rank)
     taps_dev = net.tap_buffers()
     for t in taps_dev.values():
         t.copy_(torch.relu(torch.randn_like(t)))           # post-ReLU Inception taps (RGB_OFF.py:395)
@@ -403,22 +430,26 @@ def run_ours(args):
     taps_host = {k: torch.empty(t.shape, dtype=t.dtype, pin_memory=True).copy_(t) for k, t in taps_dev.items()}
     loss_host = torch.empty((), dtype=torch.float32, pin_memory=True)
 
-    def make_step(net, dp):
+    def make_step(net, dp, keep=None):
         def step(inputs=None):
             """One forward+backward.  inputs = None: taps already resident in HBM (device-timed `value`);
-            inputs = a prefetch handle: the end-to-end path (taps staged from pinned host memory, loss read back)."""
-            fc7, _, fc14 = net(net.tap_buffers() if inputs is None else inputs)
+            inputs = a prefetch handle: the end-to-end path (taps staged from pinned host memory, loss read back).
+            keep: a dict that receives what the step returns to its caller (for --dump-outputs)."""
+            fc7, fc28, fc14 = net(net.tap_buffers() if inputs is None else inputs)
             loss = F.cross_entropy(fc7, target) + F.cross_entropy(fc14, target)
             # backward through the module's autograd.Function; the OFF-parameter gradients land in the flat buffer
             g7, g14 = torch.autograd.grad(loss, [fc7, fc14])
-            dp.backward(g7, g14)
+            grads = dp.backward(g7, g14)
             if inputs is not None:
                 loss_host.copy_(loss.detach(), non_blocking=True)
                 torch.cuda.current_stream().synchronize()       # the user reads the loss every step
+            if keep is not None:
+                keep.update(fc7=fc7, fc28=fc28, fc14=fc14, loss=loss, grads=grads)
             return loss
         return step
 
-    step = make_step(net, dp)
+    last = {} if args.dump_outputs else None
+    step = make_step(net, dp, last)
 
     def barrier():
         if world > 1:
@@ -454,6 +485,11 @@ def run_ours(args):
         sampler.start()
     ms = timed(step, net, args.steps, False)
     sampler.stop_flag = True
+    if last is not None and rank == 0:
+        # before any further step: the gradients are views of the engine's flat buffer, which the next step overwrites
+        out = {k: last[k].detach().cpu().numpy() for k in ("fc7", "fc28", "fc14", "loss")}
+        out.update({"grad." + n: g.cpu().numpy() for n, g in last["grads"].items()})
+        dump_outputs(args.dump_outputs, out)
     timed(step, net, 2, True)                                 # warm the staged path
     n_e2e = max(3, args.steps // 2)
     ms_e2e = timed(step, net, n_e2e, True) / n_e2e * args.steps

@@ -1,7 +1,7 @@
 """Pin the oracle against the REAL reference and write tests/golden/*.npz.
 
-Runs only in the build container (needs /root/reference, read-only).  The
-reference classes are imported unmodified; the OFF section is isolated with
+Needs a checkout of the reference repository (JoeHEZHAO/Optical-Flow-Guided-Feature-Pytorch),
+read-only.  The reference classes are imported unmodified; the OFF section is isolated with
 forward-pre-hooks that replace the inputs of the 18 tap consumers
 (SURVEY.md section 8c): ``motion_conv_gen_X <- taps[X]`` and
 ``motion_spatial_down_X <- taps[X][:B*(L-1)]`` (mirrors RGB_OFF.py:609).
@@ -11,7 +11,7 @@ Shims applied at run time, never by editing the reference:
   * ``dropout``    -> a module replaying injected keep-masks in call order
     (RGB_OFF.py:612,632,651,701,719,737,755,785,791,809,827,845).
 
-Usage:  python oracle/make_golden.py      (writes tests/golden/off_*.npz)
+Usage:  python oracle/make_golden.py REFERENCE_DIR      (writes tests/golden/*)
 """
 from __future__ import annotations
 
@@ -26,7 +26,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 import off_oracle as O  # noqa: E402
 
-REF = "/root/reference"
+REF = ""                      # the reference checkout, from the command line
 GOLD = os.path.join(os.path.dirname(HERE), "tests", "golden")
 
 DROP_ORDER = ["3a", "3b", "3c", "4a", "4b", "4c", "4d", "fc28", "fc14", "5a", "5b", "fc7"]
@@ -234,4 +234,7 @@ def main():
 
 
 if __name__ == "__main__":
+    if len(sys.argv) != 2 or not os.path.isdir(sys.argv[1]):
+        sys.exit("usage: python oracle/make_golden.py REFERENCE_DIR")
+    REF = os.path.abspath(sys.argv[1])
     main()
