@@ -304,10 +304,6 @@ typedef struct offk_stencil_io {
  * host arrays of n entries; semantics per entry are those of offk_stencil_diff_fwd / _bwd. */
 int offk_stencil_diff_fwd_batch(int n, const offk_stencil_t* s, const offk_stencil_io_t* io, void* stream);
 int offk_stencil_diff_bwd_batch(int n, const offk_stencil_t* s, const offk_stencil_io_t* io, void* stream);
-/* One half of the batched backward: part = 1 the temporal half (dg: streams G and dT once), 2 the spatial half (dd, dw,
- * dbias), 3 both (= offk_stencil_diff_bwd_batch).  The halves write disjoint elements (dg / dd may be channel slices of
- * one buffer) and may run concurrently on two streams. */
-int offk_stencil_diff_bwd_batch_part(int n, const offk_stencil_t* s, const offk_stencil_io_t* io, int part, void* stream);
 
 /* Backward of the above.  dout is the gradient of the stage buffer (same
  * ctot/coff addressing as `out`).  Writes

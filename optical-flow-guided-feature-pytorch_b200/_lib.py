@@ -107,7 +107,6 @@ _PROTOS = {
                                         _P, _P, _P]),
     "offk_stencil_diff_fwd_batch": (C.c_int, [C.c_int, C.POINTER(OffkStencil), C.POINTER(OffkStencilIO), _P]),
     "offk_stencil_diff_bwd_batch": (C.c_int, [C.c_int, C.POINTER(OffkStencil), C.POINTER(OffkStencilIO), _P]),
-    "offk_stencil_diff_bwd_batch_part": (C.c_int, [C.c_int, C.POINTER(OffkStencil), C.POINTER(OffkStencilIO), C.c_int, _P]),
     "offk_avgpool_drop_fwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_uint64, _P,
                                         C.c_float, C.c_float, _P, _P]),
     "offk_avgpool_drop_bwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_uint64, _P,

@@ -1,18 +1,8 @@
 // extern "C" surface of liboffk.so that is not tied to one kernel family.
-#include <stdlib.h>
 #include "offk_gemm.cuh"
 
 namespace offk {
 thread_local char g_err[512] = "";
-
-bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("OFFK_NO_PDL");
-    v = (e && e[0] == '1') ? 0 : 1;
-  }
-  return v != 0;
-}
 
 int sm_count() {
   static int cached = 0;

@@ -104,7 +104,6 @@ __device__ __forceinline__ void pdl_sync() {
   asm volatile("griddepcontrol.wait;" ::: "memory");
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 }
-bool pdl_enabled();  // OFFK_NO_PDL=1 turns the launch attribute off
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
@@ -112,7 +111,7 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.attrs = attr; cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 

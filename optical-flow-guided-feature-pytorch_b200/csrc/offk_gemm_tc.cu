@@ -20,7 +20,6 @@
 //              mbarrier (and to "accum_full" after the last K-block).
 // One output tile per CTA; two CTAs co-reside per SM (<=110 KB smem, <=256 TMEM columns each) so one
 // CTA's epilogue overlaps the other's main loop.
-#include <stdlib.h>
 #include "offk_tc.cuh"
 
 namespace offk {
@@ -656,15 +655,7 @@ static int launch_tc_t(const offk_gemm_t& g, int bn, int stages, int kb_per, int
     if (e != cudaSuccess) return cuda_check(e, "cudaFuncSetAttribute(gather_gemm_tc)");
     attr_set = true;
   }
-  static int pdl = -1;
-  if (pdl < 0) { const char* e = getenv("OFFK_NO_PDL"); pdl = (e && e[0] == '1') ? 0 : 1; }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid; cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, g, bn, stages, kb_per, tmem_cols, la, n_main);
+  cudaError_t e = launch_pdl(kern, grid, dim3(TC_THREADS), smem, st, g, bn, stages, kb_per, tmem_cols, la, n_main);
   if (e != cudaSuccess) return cuda_check(e, "gather_gemm_tc launch");
   return OFFK_LAUNCH_CHECK("gather_gemm_tc");
 }

@@ -43,7 +43,6 @@
 // One output tile per CTA; two CTAs co-reside per SM in the tf32 mode so one CTA's epilogue overlaps the other's main loop
 // (the 3xTF32 stages and TMEM budget take the whole SM).  tools/timeline.py + -DOFFK_TIMELINE stamp every phase per CTA.
 #include <cuda.h>
-#include <stdlib.h>
 #include "offk_tc.cuh"
 
 namespace offk {
@@ -574,26 +573,8 @@ tma_gemm_kernel(const __grid_constant__ CUtensorMap tma, const __grid_constant__
       // Linear output rows (offk.h: out_ld): 32-column slabs of the tile go to shared memory in the SWIZZLE_128B box
       // layout (row r at r * 128 bytes, 16-byte chunk j at j ^ (r & 7)) and leave as TMA tile stores -- or float adds
       // for split-K partial sums -- which clip at the matrix / frame edge.  Three slabs rotate: the store of slab c - 2
-      // has released its buffer (wait_group.read) before anyone passed the barrier of slab c - 1.
-      // Pass 1 (one accumulator row per thread): bias and the leading ReLU.  Pass 2, only for layers with a ReLU' gate or
-      // a residual addend: the slab is revisited in place with row-contiguous (coalesced) loads of those operands.
-      const bool extra = (g.gate || g.addend) && !atomic;
-      const int rsub = lane >> 3, cq = lane & 7;
-      const int oc0 = __ldg(g.out_col);
-      const int gc0 = g.gate ? (g.gate_col ? __ldg(g.gate_col) : oc0) : 0;
-      const int ac0 = g.addend ? (g.add_col ? __ldg(g.add_col) : oc0) : 0;
-      int r_gate[TC_BM / 32], r_add[TC_BM / 32];
-      bool r_ok[TC_BM / 32];
-#pragma unroll
-      for (int it = 0; it < TC_BM / 32; ++it) {
-        const int m = m0 + it * 32 + ew * 4 + rsub;
-        r_ok[it] = extra && m < m_lim;
-        r_gate[it] = r_add[it] = 0;
-        if (r_ok[it]) {
-          const EpiRow er = epi_row(g, m);
-          r_gate[it] = er.gate; r_add[it] = er.add;
-        }
-      }
+      // has released its buffer (wait_group.read) before anyone passed the barrier of slab c - 1.  One accumulator row per
+      // thread: bias and ReLU only (host: no gate, addend, finisher or second output on this path).
       if (g.bias && !atomic)
         for (int i = tid - 64; i < bn; i += TM_THREADS - 64) sh->bias[i] = n0 + i < g.N ? __ldg(g.bias + n0 + i) : 0.f;
       asm volatile("bar.sync 1, 256;" ::: "memory");             // bias values are read before the first slab barrier
@@ -607,20 +588,6 @@ tma_gemm_kernel(const __grid_constant__ CUtensorMap tma, const __grid_constant__
       int slab = 0;
       for (int c = 0; c < nchunks; ++c) {
         const uint32_t buf = smem_base + (uint32_t)slab * (TC_BM * 128);
-        const int n = n0 + c * 32 + cq * 4;                      // pass 2: this thread's 4 columns
-        const bool gated = g.gate && n >= g.gate_col0;
-        float4 gt[TC_BM / 32], ad[TC_BM / 32];
-        if (extra) {                                             // in flight across the TMEM drain and the first barrier
-#pragma unroll
-          for (int it = 0; it < TC_BM / 32; ++it) {
-            gt[it] = make_float4(1.f, 1.f, 1.f, 1.f);
-            ad[it] = f4zero();
-            if (r_ok[it] && n < g.N) {
-              if (gated) gt[it] = ldg128(g.gate + (r_gate[it] + gc0 + n));
-              if (g.addend) ad[it] = ldg128(g.addend + (r_add[it] + ac0 + n));
-            }
-          }
-        }
         float v[16];
         tmem_ld16_sum(tmem_d + ((uint32_t)(quad * 32) << 16) + (uint32_t)(c * 32 + half * 16), n_acc, acc_stride, v);
         const int nl = c * 32 + half * 16;                       // first of this thread's 16 columns inside the tile
@@ -632,33 +599,12 @@ tma_gemm_kernel(const __grid_constant__ CUtensorMap tma, const __grid_constant__
               const float4 b = *reinterpret_cast<const float4*>(&sh->bias[nl + j]);
               x.x += b.x; x.y += b.y; x.z += b.z; x.w += b.w;
             }
-            if (n0 + nl + j < g.relu_pre_cols || (g.relu_post && !extra)) x = f4relu(x);
+            if (n0 + nl + j < g.relu_pre_cols || g.relu_post) x = f4relu(x);
           }
           sts128(buf + (uint32_t)trow * 128u + (uint32_t)((((half * 4 + (j >> 2))) ^ (trow & 7)) << 4), x.x, x.y, x.z, x.w);
         }
-        if (!extra) fence_proxy_async_smem();                    // generic-proxy writes -> visible to the TMA
+        fence_proxy_async_smem();                                // generic-proxy writes -> visible to the TMA
         asm volatile("bar.sync 1, 256;" ::: "memory");
-        if (extra) {
-#pragma unroll
-          for (int it = 0; it < TC_BM / 32; ++it) {
-            if (!r_ok[it] || n >= g.N) continue;
-            const int row = it * 32 + ew * 4 + rsub;
-            const uint32_t addr = buf + (uint32_t)row * 128u + (uint32_t)((cq ^ (row & 7)) << 4);
-            float4 x = lds128(addr);
-            const float4 t = gt[it];
-            if (gated && g.gate_first) {
-              x.x = t.x > 0.f ? x.x : 0.f; x.y = t.y > 0.f ? x.y : 0.f; x.z = t.z > 0.f ? x.z : 0.f; x.w = t.w > 0.f ? x.w : 0.f;
-            }
-            x.x += ad[it].x; x.y += ad[it].y; x.z += ad[it].z; x.w += ad[it].w;
-            if (gated && !g.gate_first) {
-              x.x = t.x > 0.f ? x.x : 0.f; x.y = t.y > 0.f ? x.y : 0.f; x.z = t.z > 0.f ? x.z : 0.f; x.w = t.w > 0.f ? x.w : 0.f;
-            }
-            if (g.relu_post) x = f4relu(x);
-            sts128(addr, x.x, x.y, x.z, x.w);
-          }
-          fence_proxy_async_smem();
-          asm volatile("bar.sync 1, 256;" ::: "memory");
-        }
         if (warp == 2 && elect_one_sync()) {
           if (c_mode == 2) tma_store_3d(&tmc, buf, n0 + c * 32, pix0, img_t, atomic);
           else tma_store_2d(&tmc, buf, n0 + c * 32, m0, atomic);
@@ -937,15 +883,8 @@ static int launch_tm_t(const CUtensorMap& ta, const CUtensorMap& tb, const CUten
     if (e != cudaSuccess) return cuda_check(e, "cudaFuncSetAttribute(tma_gemm)");
     attr_set = true;
   }
-  static int pdl = -1;
-  if (pdl < 0) { const char* e = getenv("OFFK_NO_PDL"); pdl = (e && e[0] == '1') ? 0 : 1; }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid; cfg.blockDim = dim3(TM_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, ta, tb, tc, g, geo, bn, stages, kb_per, tmem_cols, n_main, bk, b_presplit, a_tmem, c_mode);
+  cudaError_t e = launch_pdl(kern, grid, dim3(TM_THREADS), smem, st, ta, tb, tc, g, geo, bn, stages, kb_per, tmem_cols, n_main,
+                             bk, b_presplit, a_tmem, c_mode);
   if (e != cudaSuccess) return cuda_check(e, "tma_gemm launch");
   return OFFK_LAUNCH_CHECK("tma_gemm");
 }
@@ -1086,18 +1025,15 @@ extern "C" int offk_tma_gemm(const offk_tgemm_t* t, void* stream) {
   const int presplit = (x3 && t->b_kind == OFFK_TMA_B_DENSE && t->b_lo_delta != 0) ? 1 : 0;
   // 3xTF32 with the A operand in tensor memory (kernel comment): possible when the accumulators leave room for at least
   // two (A_hi, A_lo) column pairs; the wide tiles (N tile > 192) keep both operands in shared memory.  One CTA per SM.
-  static int atm_env = -1;
-  if (atm_env < 0) { const char* e = getenv("OFFK_X3_ATM"); atm_env = (e && e[0] == '0') ? 0 : 1; }
   const int acc_stride = (bn + 31) / 32 * 32;
   const int a_cols = t->a_kind == OFFK_TMA_A_IM2COL_T ? bk : TC_BK;
   const int mmas = kb_per * (bk / 8);                      // K = 8 steps per output tile
   int atm = 0, atm_main = 0, atm_slots = 0;
-  if (x3 && atm_env) {
-    // chains of at most OFFK_X3_CHAIN (64) MMAs per main accumulator where tensor memory has the room (measured: the
-    // chain policy does not move the step time -- profiles/env_r02x.log -- but single 800-MMA chains took the fc14
-    // error from 3.7e-6 to 6.7e-6)
-    static int chain = -1;
-    if (chain < 0) { const char* e = getenv("OFFK_X3_CHAIN"); chain = e ? atoi(e) : 64; if (chain < 64) chain = 64; }
+  if (x3) {
+    // chains of at most 64 MMAs per main accumulator where tensor memory has the room (measured: the chain policy does
+    // not move the step time -- profiles/env_r02x.log -- but single 800-MMA chains took the fc14 error from 3.7e-6 to
+    // 6.7e-6)
+    constexpr int chain = 64;
     const int want = x3_main_accumulators(4, (mmas * 64 + chain - 1) / chain);
     for (int nm = want; nm >= 1 && !atm; --nm) {
       const int slots = (512 - (1 + nm) * acc_stride) / (2 * a_cols);
@@ -1139,15 +1075,12 @@ extern "C" int offk_tma_gemm(const offk_tgemm_t* t, void* stream) {
   memcpy(&ta, t->tmap_a, sizeof(ta));
   memcpy(&tb, t->tmap_b, sizeof(tb));
   memcpy(&tc, t->tmap_c, sizeof(tc));
-  // TMA stores (offk.h: out_ld): only with the epilogue the output map was prepared for
-  static int tst_env = -1;
-  if (tst_env < 0) { const char* e = getenv("OFFK_TMA_STORE"); tst_env = e ? atoi(e) : 1; }
-  // 0 = off, 1 = plain epilogues (bias / ReLU, split-K partial sums), 2 = also the layers with a ReLU' gate or a residual
-  // addend (second pass over the slab).  1 is the default: measured -3.4 % (fp32) / -2.5 % (tf32) of the step against 0,
-  // while 2 buys nothing on top (profiles/env_r03f-i.log) -- the extra barrier and shared-memory pass cost what the
-  // faster stores save.
-  const int c_mode = (tst_env && t->c_mode && g.out_vec == 1 && !g.finish_counter && !g.aux_out && bn % 32 == 0 &&
-                      (tst_env > 1 || (!g.gate && !g.addend))) ? t->c_mode : 0;
+  // TMA stores (offk.h: out_ld) for plain epilogues only: bias / ReLU, or split-K partial sums.  Measured -3.4 % (fp32) /
+  // -2.5 % (tf32) of the step against st.global everywhere; a second pass over the slab for the ReLU' gate and residual
+  // addend bought nothing on top (profiles/env_r03f-i.log): its barrier and shared-memory pass cost what the faster
+  // stores save.
+  const int c_mode = (t->c_mode && g.out_vec == 1 && !g.finish_counter && !g.aux_out && bn % 32 == 0 && !g.gate && !g.addend)
+                         ? t->c_mode : 0;
   // same formula as the kernel: the shared structure follows max(pipeline stages, epilogue staging)
   const size_t epi_bytes = c_mode ? 3 * TC_BM * 128 : 2 * TC_BM * TM_EPI_PITCH * 4;
   if (pipe_bytes < epi_bytes) pipe_bytes = epi_bytes;

@@ -20,14 +20,11 @@
 // dw[a,b] += D(y,x) * dS(y-a+1, x-b+1) (the tap gradient re-indexed so that it needs D only at the centre pixel).
 // Tap / bias gradients are accumulated in registers over a few consecutive items, reduced with warp shuffles and
 // shared-memory atomics, then one global atomicAdd per tap and block.
-#include <stdlib.h>
 #include "offk_common.cuh"
 
 namespace offk {
 
-#ifndef ST_FWD_MINB
-#define ST_FWD_MINB 3      // resident blocks per SM the kernels are compiled for (register cap 80)
-#endif
+constexpr int ST_FWD_MINB = 3;   // resident blocks per SM the kernels are compiled for (register cap 80; 4 spills, DESIGN 3.1)
 constexpr int ST_THREADS = 256;
 constexpr int ST_WARPS = ST_THREADS / 32;
 constexpr int ST_MAX_LEVELS = 12;
@@ -559,25 +556,6 @@ stencil_diff_bwd_kernel(const __grid_constant__ StBatch bt) {
   }
 }
 
-// The two halves of the backward as separate launches (offk_stencil_diff_bwd_batch_part): the temporal half is a pure
-// stream (64 registers, 4 blocks per SM), the spatial half is instruction-heavy and moves a tenth of the bytes; on two
-// streams the block scheduler mixes them instead of spatial blocks holding a third of the resident-block slots.
-__global__ void __launch_bounds__(ST_THREADS, 4)
-stencil_diff_bwd_temporal_kernel(const __grid_constant__ StBatch bt) {
-  pdl_sync();
-  const StLevel& lv = find_level(bt, (int)blockIdx.x);
-  const int r2 = (int)blockIdx.x - lv.blk0;
-  if (lv.s.L == 3) temporal_bwd<3>(lv, r2, threadIdx.x);
-  else temporal_bwd<0>(lv, r2, threadIdx.x);
-}
-__global__ void __launch_bounds__(ST_THREADS, ST_FWD_MINB)
-stencil_diff_bwd_spatial_kernel(const __grid_constant__ StBatch bt) {
-  pdl_sync();
-  extern __shared__ __align__(16) float4 st_smem[];
-  const StLevel& lv = find_level(bt, (int)blockIdx.x);
-  spatial_bwd(lv, (int)blockIdx.x - lv.blk0, threadIdx.x, st_smem);
-}
-
 // ---------------------------------------------------------------------------------------------- host
 static int check_stencil(const offk_stencil_t* s) {
   OFFK_REQUIRE(s != nullptr, "stencil: null descriptor");
@@ -633,15 +611,8 @@ static int plan_spatial(StLevel& lv, bool backward) {
   // backward: a block keeps the tap-gradient partial sums in registers over up to ST_ITEMS consecutive items (fewer
   // block reductions / atomics); small levels keep one item per block so their blocks stay short
   // measured at config 2 (B200): items / (0.5 * SMs) capped at 8 -> 121 us; 2.0 / 4 -> 149 us; 0.2 / 32 -> 250 us (tail)
-  static int div10 = 0, cap = 0;                                   // bring-up knobs (environment)
-  if (!div10) {
-    const char* e = getenv("OFFK_ST_IPB_DIV10");
-    div10 = e ? atoi(e) : 5;
-    const char* c = getenv("OFFK_ST_IPB_CAP");
-    cap = c ? atoi(c) : ST_ITEMS;
-  }
-  long long ipb = items * 10 / ((long long)div10 * sm_count());
-  lv.ipb = backward ? (int)(ipb < 1 ? 1 : (ipb > cap ? cap : ipb)) : 1;
+  const long long ipb = items * 2 / sm_count();
+  lv.ipb = backward ? (int)(ipb < 1 ? 1 : (ipb > ST_ITEMS ? ST_ITEMS : ipb)) : 1;
   lv.n_sblocks = (int)((items + lv.ipb - 1) / lv.ipb);
   const int tile_bytes = (lv.band_rows + 2) * row_bytes;
   const int tap_bytes = s.K * 9 * ST_WQ * 16;
@@ -651,8 +622,7 @@ static int plan_spatial(StLevel& lv, bool backward) {
   return tile_bytes + tap_bytes + extra;
 }
 
-static int launch_batch(int n, const offk_stencil_t* s, const offk_stencil_io_t* io, bool backward, void* stream, int part = 3) {
-  OFFK_REQUIRE(part >= 1 && part <= 3 && (backward || part == 3), "stencil batch: part must be 1 (temporal), 2 (spatial) or 3 (both)");
+static int launch_batch(int n, const offk_stencil_t* s, const offk_stencil_io_t* io, bool backward, void* stream) {
   OFFK_REQUIRE(n >= 1 && n <= ST_MAX_LEVELS, "stencil batch: 1 <= n <= %d (got %d)", ST_MAX_LEVELS, n);
   OFFK_REQUIRE(s != nullptr && io != nullptr, "stencil batch: null arrays");
   StBatch bt;
@@ -677,13 +647,12 @@ static int launch_batch(int n, const offk_stencil_t* s, const offk_stencil_io_t*
       OFFK_REQUIRE(s[i].Cs == 0 || (lv.w && lv.dd && aligned16(lv.dd) && lv.dd_fs % 4 == 0), "stencil_bwd: w/dd missing");
       OFFK_REQUIRE(lv.dw == nullptr || (lv.d != nullptr && aligned16(lv.d)), "stencil_bwd: tap gradient needs d");
     }
-    int need = plan_spatial(lv, backward);
-    if (!(part & 2)) { lv.n_sblocks = 0; need = 0; }               // temporal half only
+    const int need = plan_spatial(lv, backward);
     OFFK_REQUIRE(need <= ST_SMEM_MAX, "stencil: halo tile of %d bytes exceeds %d (W=%d, Cs=%d)", need, ST_SMEM_MAX, s[i].W, s[i].Cs);
     if (need > smem) smem = need;
     const int HW = s[i].H * s[i].W;
     lv.t_chunks = s[i].Cg > 0 ? (HW + ST_TPIX - 1) / ST_TPIX : 1;
-    const long long n_t = (s[i].Cg > 0 && (part & 1)) ? (long long)lv.t_chunks * s[i].B : 0;
+    const long long n_t = s[i].Cg > 0 ? (long long)lv.t_chunks * s[i].B : 0;
     lv.n_tblocks = (int)n_t;
     // spatial blocks at every 2^lstride-th position of the level's range
     lv.lstride = 0;
@@ -699,8 +668,6 @@ static int launch_batch(int n, const offk_stencil_t* s, const offk_stencil_io_t*
     cudaError_t e = cudaFuncSetAttribute(stencil_diff_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM_MAX);
     if (e == cudaSuccess)
       e = cudaFuncSetAttribute(stencil_diff_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM_MAX);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(stencil_diff_bwd_spatial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM_MAX);
     if (e != cudaSuccess) return cuda_check(e, "cudaFuncSetAttribute(stencil)");
     attr_set = true;
   }
@@ -708,9 +675,7 @@ static int launch_batch(int n, const offk_stencil_t* s, const offk_stencil_io_t*
     (void)launch_pdl(stencil_diff_fwd_kernel, dim3((unsigned)blk), dim3(ST_THREADS), (size_t)smem, as_stream(stream), bt);
     return OFFK_LAUNCH_CHECK("stencil_diff_fwd");
   }
-  if (part == 1) (void)launch_pdl(stencil_diff_bwd_temporal_kernel, dim3((unsigned)blk), dim3(ST_THREADS), (size_t)0, as_stream(stream), bt);
-  else if (part == 2) (void)launch_pdl(stencil_diff_bwd_spatial_kernel, dim3((unsigned)blk), dim3(ST_THREADS), (size_t)smem, as_stream(stream), bt);
-  else (void)launch_pdl(stencil_diff_bwd_kernel, dim3((unsigned)blk), dim3(ST_THREADS), (size_t)smem, as_stream(stream), bt);
+  (void)launch_pdl(stencil_diff_bwd_kernel, dim3((unsigned)blk), dim3(ST_THREADS), (size_t)smem, as_stream(stream), bt);
   return OFFK_LAUNCH_CHECK("stencil_diff_bwd");
 }
 
@@ -724,10 +689,6 @@ extern "C" int offk_stencil_diff_fwd_batch(int n, const offk_stencil_t* s, const
 
 extern "C" int offk_stencil_diff_bwd_batch(int n, const offk_stencil_t* s, const offk_stencil_io_t* io, void* stream) {
   return launch_batch(n, s, io, true, stream);
-}
-
-extern "C" int offk_stencil_diff_bwd_batch_part(int n, const offk_stencil_t* s, const offk_stencil_io_t* io, int part, void* stream) {
-  return launch_batch(n, s, io, true, stream, part);
 }
 
 extern "C" int offk_stencil_diff_fwd(const offk_stencil_t* s, const float* g, const float* d, const float* w,

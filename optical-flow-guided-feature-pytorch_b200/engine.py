@@ -14,7 +14,6 @@ from __future__ import annotations
 
 import ctypes as C
 import math
-import os
 from collections import OrderedDict
 
 import numpy as np
@@ -25,8 +24,11 @@ from . import spec as S
 from . import tables as T
 
 _SM_TARGET = 148
-_PICK_A = float(os.environ.get("OFFK_PICK_A", "128"))      # _pick_tile_n: per-CTA cost ~ _PICK_A + bn (A rows + B rows of a K-block)
-_X3_MAX_BN = int(os.environ.get("OFFK_X3_MAX_BN", "256"))     # widest N tile of a TMA-fed GEMM in the 3xTF32 mode
+_PICK_A = 128           # _pick_tile_n: per-CTA cost ~ _PICK_A + bn (A rows + B rows of a K-block)
+_WGRAD_FIXED_KB = 10    # _wgrad_split: fixed cost of a weight-gradient CTA, in K-blocks of 32 pixels
+_TF32_WANT_CTAS = _SM_TARGET    # _auto_tile_n: CTAs a TMA-fed GEMM without split-K aims for in the tf32 mode
+_X3_WANT_CTAS = 40      # ... and in the 3xTF32 mode
+_FINISH_MIN_TILES = 100     # output tiles from which a split-K conv finishes in-kernel (_conv_fwd)
 _TC_PRECS = (L.PREC_TF32, L.PREC_TF32X3)      # tcgen05 modes: 1 MMA per product / error-compensated 3xTF32
 
 
@@ -62,7 +64,7 @@ def _wgrad_split(tiles: int, kb: int, slots: int, bk: int = 32) -> int:
     minimises rounds x (K-blocks per CTA + fixed cost), rounds = ceil(CTAs / resident CTA slots); an under-filled round is
     charged as idle SMs.  The fixed cost (prologue, first TMA round trip, adding the tile into dW) is worth ~10 K-blocks of
     32 pixels (profiles/timeline_*_r02z.txt); the result is insensitive to it between 5 and 20 (profiles/env_r03j.log)."""
-    fixed = float(os.environ.get("OFFK_WGRAD_FIXED_KB", "10")) * 32 / bk
+    fixed = _WGRAD_FIXED_KB * 32 / bk
     cost = lambda s_: math.ceil(tiles * s_ / slots) * (math.ceil(kb / s_) + fixed) * max(1.0, _SM_TARGET / (tiles * s_))
     return min(range(1, max(1, kb // 4) + 1), key=lambda s_: (cost(s_), s_))
 
@@ -96,12 +98,6 @@ class Gemm:
         d.ones_row_out = ones_out.data_ptr() if ones_out is not None else None
         if tile_n == 0 and split_k == 1:
             tile_n = _auto_tile_n(spc.M, spc.N, isinstance(self, TGemm), eng.prec == L.PREC_TF32X3)
-        if isinstance(self, TGemm) and eng.prec == L.PREC_TF32X3 and _X3_MAX_BN < 256:
-            # 3xTF32 keeps the A operand in tensor memory when the accumulators leave room (N tile <= 192, offk_gemm_tma.cu);
-            # a wide tile would fall back to both operands in shared memory and two pipeline stages
-            bn = tile_n if tile_n else (256 if spc.N > 256 else (spc.N + 15) // 16 * 16)
-            if bn > 192:
-                tile_n = min(_X3_MAX_BN, (math.ceil(spc.N / math.ceil(spc.N / _X3_MAX_BN)) + 15) // 16 * 16)
         d.split_k, d.tile_n = split_k, tile_n
         d.out_vec = spc.out_vec if out_vec is None else out_vec
         counter = None
@@ -239,23 +235,6 @@ class OFFEngine:
         self.consensus = (variant != "rgb") if consensus is None else bool(consensus)
         self.tap_grads = tap_grads
         self.single_stream = False       # True: issue every lane on the caller's stream (profiling / debugging)
-        self.use_tma = os.environ.get("OFFK_NO_TMA", "0") != "1"     # bring-up switch: gather-fed GEMMs everywhere
-        # weight gradients with TMA-fed operands: on for the NCHW taps (measured 81 -> 54 us at level 3a); off by default
-        # for channels-last convs, where 32-pixel im2col boxes lose to the cp.async gather on the big KxK layers
-        # (motion_conv_trans_28: 388 vs 211 us) and tie elsewhere -- OFFK_TMA_WGRAD=all forces them on, =none disables both
-        self.tma_wgrad = os.environ.get("OFFK_TMA_WGRAD", "taps")
-        self.tma_strided_dgrad = os.environ.get("OFFK_NO_TMA_SDGRAD", "0") != "1"
-        # channels-last weight gradients through TMA im2col with DEEP K-blocks (bk output pixels per stage: 64 / 128 instead
-        # of 32 -> fewer, larger TMA boxes).  OFFK_WGRAD_TMA: which layers ("big" = the three stage-entry KxK convs, "kxk" =
-        # every KxK conv, "all"); OFFK_WGRAD_BK: the depth
-        # Measured at config 2 (profiles/wgrad_sweep_r02x.txt).  tf32 mode: the cp.async gather kernel is faster everywhere
-        # except on motion_conv_trans_28, where 128-pixel boxes win (197 us gather, 389 / 204 / 169 us TMA at bk = 32 / 64 / 128;
-        # motion_conv_trans_14: 97 vs 136, motion_conv_trans: 60 vs 77).  fp32 (3xTF32) mode, where the gather kernel's producers
-        # also write the residual tiles: the TMA-fed kernel wins on every KxK layer (784 -> 501, 344 -> 296, 194 -> 177 us at the
-        # deepest K-block that still leaves two pipeline stages).  Defaults follow the measurement.
-        x3 = self.prec == L.PREC_TF32X3
-        self.wgrad_tma = os.environ.get("OFFK_WGRAD_TMA", "all" if x3 else "t28")
-        self.wgrad_bk = int(os.environ.get("OFFK_WGRAD_BK", "64" if x3 else "128"))
         self._tab_cache = {}
         self._keep = []
         self.generation = 0
@@ -265,7 +244,7 @@ class OFFEngine:
         # fp32 (3xTF32) mode: the tf32 residuals of the weights are produced once per step into a twin buffer directly behind
         # the parameters, so that the GEMMs receive both weight tiles by TMA (offk.h: b_lo_delta) instead of splitting them in
         # shared memory in every CTA and K-block
-        self.presplit = self.prec == L.PREC_TF32X3 and os.environ.get("OFFK_NO_PRESPLIT", "0") != "1"
+        self.presplit = self.prec == L.PREC_TF32X3
         self._params_all = torch.zeros(self.n_flat * (2 if self.presplit else 1), device=self.device)
         self.params_flat = self._params_all[:self.n_flat]
         self.params_lo = self._params_all[self.n_flat:] if self.presplit else None
@@ -418,8 +397,6 @@ class OFFEngine:
         spc = T.conv_fwd_spec(geom, x_layout, "nhwc")
         m_tiles, kb = math.ceil(spc.M / 128), math.ceil(spc.K / 32)
         n_tiles = max(1, math.ceil(spc.N / 256))
-        if self.prec == L.PREC_TF32X3 and self.use_tma and spc.N > 192:
-            n_tiles = math.ceil(spc.N / _X3_MAX_BN)      # Gemm.__init__ re-tiles wide 3xTF32 GEMMs
         split = 1
         if self.tc and addend is None and m_tiles * n_tiles < 200 and kb >= 32:
             # split-K factor: minimise rounds x K-blocks per CTA, rounds = ceil(CTAs / resident CTA slots) (two CTAs per SM in
@@ -429,19 +406,17 @@ class OFFEngine:
             tiles = m_tiles * n_tiles
             split = min(range(1, max(1, kb // 8) + 1),
                         key=lambda s_: (math.ceil(tiles * s_ / slots) * math.ceil(kb / s_) * (1 if tiles * s_ >= 0.9 * _SM_TARGET else 4), s_))
-            forced = dict(kv.split("=") for kv in os.environ.get("OFFK_FWD_SPLIT", "").split(",") if "=" in kv)
-            split = int(forced.get(name, split))          # tuning hook: OFFK_FWD_SPLIT=motion_conv_trans_28=3,...
         cols = (geom.cout if relu else 0) if relu_cols is None else relu_cols
-        tma = self.use_tma and TGemm.eligible(geom, self.prec, a_relu, x_layout)
+        tma = TGemm.eligible(geom, self.prec, a_relu, x_layout)
         mk = (lambda *a, **k: TGemm(*a, geom=geom, x_layout=x_layout, **k)) if tma else Gemm
         if (tma and x_layout == "nchw") or no_split:
             split = 1                     # per-frame M tiles already fill the machine (N * ceil(hw/128) CTAs)
-        fuse = tma and spc.out_vec and os.environ.get("OFFK_NO_FINISHER", "0") != "1"
+        fuse = tma and spc.out_vec
         # in-kernel finishing pays when there are enough output tiles for the finishing CTAs to keep the machine busy
         # (motion_conv_trans_28: 147 tiles, same time as the bare split-K GEMM, bias_act and ReLU copy for free); with the
         # 37-tile 7x7 layers the fences + a finishing pass by 37 CTAs cost 9-27 us more than a separate full-grid bias_act
         # pass (measured, profiles/launches_tf32_r02g*.txt), so those keep the two-kernel form
-        fin_ok = fuse and m_tiles * n_tiles >= int(os.environ.get("OFFK_FINISH_MIN_TILES", "100"))
+        fin_ok = fuse and m_tiles * n_tiles >= _FINISH_MIN_TILES
         if split > 1 and fin_ok:
             # split-K partial tiles are added into the zeroed output; the last CTA of each tile applies bias / ReLU (and
             # writes the second output) in place: no separate bias_act pass
@@ -483,43 +458,40 @@ class OFFEngine:
         self.flops_fwd += g.flops
         return g
 
-    def _conv_wgrad(self, name, x, dy, geom, dw, db, *, a_relu=False, x_layout="nhwc", force_tma=False):
+    def _conv_wgrad(self, name, x, dy, geom, dw, db, *, a_relu=False, x_layout="nhwc", tap_copy=False):
+        """tap_copy: x is the channels-last copy of a unit's tap (the 7x7 levels), which is TMA-fed like the NCHW tap."""
         # dW is accumulated in the k order of the implicit GEMM (OHWI: consecutive accumulator rows = consecutive
         # addresses, so the split-K reductions coalesce) and un-permuted once at the end; writing OIHW directly
         # (dw_layout="oihw") was measured slower: the strided atomics cost more than the permute pass
         spc = T.conv_wgrad_spec(geom, x_layout, "nhwc")
-        tma = (self.use_tma and (self.tma_wgrad == "all" or (self.tma_wgrad == "taps" and (x_layout == "nchw" or force_tma)))
-               and TGemm.wgrad_eligible(geom, self.prec, a_relu, x_layout))
+        x3 = self.prec == L.PREC_TF32X3
+        # the units' weight gradients are TMA-fed from the tap (measured 81 -> 54 us at level 3a)
+        tma = TGemm.wgrad_eligible(geom, self.prec, a_relu, x_layout)
         bk = 0
-        base = name.split(".")[0]
-        deep = {"t28": base == "motion_conv_trans_28",
-                "big": base in ("motion_conv_trans_28", "motion_conv_trans_14", "motion_conv_trans"),
-                "kxk": geom.kh > 1, "all": True}.get(self.wgrad_tma, False)
-        if (deep and self.use_tma and x_layout == "nhwc" and not force_tma and self.wgrad_bk in (32, 64, 128)
-                and TGemm.wgrad_eligible(geom, self.prec, a_relu, x_layout)):
-            # deepest K-block <= the requested one whose pipeline stage (A: 4 stacks of {32 rows x bk pixels}, B: one per 32
-            # columns of the N tile; twice that with the 3xTF32 residual tiles) still leaves room for two stages per SM
+        if tma and x_layout == "nhwc" and not tap_copy:
+            # stage convs: TMA im2col with DEEP K-blocks (bk output pixels per stage: 64 / 128 instead of 32 -> fewer, larger
+            # TMA boxes) where that was measured faster than the cp.async gather kernel (config 2,
+            # profiles/wgrad_sweep_r02x.txt).  tf32 mode: only motion_conv_trans_28, where 128-pixel boxes win (197 us
+            # gather, 389 / 204 / 169 us TMA at bk = 32 / 64 / 128; motion_conv_trans_14: 97 vs 136, motion_conv_trans:
+            # 60 vs 77).  fp32 (3xTF32) mode, where the gather kernel's producers also write the residual tiles: every
+            # layer, and the TMA-fed kernel wins on every KxK one (784 -> 501, 344 -> 296, 194 -> 177 us) at bk <= 64.
+            max_bk = 64 if x3 else (128 if name == "motion_conv_trans_28" else 0)
+            # deepest K-block <= max_bk whose pipeline stage (A: 4 stacks of {32 rows x bk pixels}, B: one per 32 columns
+            # of the N tile; twice that with the 3xTF32 residual tiles) still leaves room for two stages per SM
             bn = 256 if spc.N > 256 else (spc.N + 15) // 16 * 16
-            mul = 2 if self.prec == L.PREC_TF32X3 else 1
-            fits = [b for b in (128, 64, 32) if b <= self.wgrad_bk and mul * (b * 512 + math.ceil(bn / 32) * b * 128) <= 108 * 1024]
-            if fits:
-                tma, bk = True, fits[0]
+            mul = 2 if x3 else 1
+            fits = [b for b in (128, 64, 32) if b <= max_bk and mul * (b * 512 + math.ceil(bn / 32) * b * 128) <= 108 * 1024]
+            tma, bk = bool(fits), (fits[0] if fits else 0)
         m_tiles, kb = math.ceil(spc.M / 128), math.ceil(spc.K / (bk or 32))
         n_tiles = max(1, math.ceil(spc.N / 256))
         # split-K factor: minimise rounds x (K-blocks per CTA + fixed cost), rounds = ceil(CTAs / resident CTA slots) -- two CTAs
         # per SM in the tf32 mode, one in the 3xTF32 mode.  The fixed cost (prologue, first TMA round trip, the epilogue that
         # adds the CTA's whole tile into dW) is worth ~10 K-blocks (profiles/timeline_*_r02z.txt); an under-filled round is
-        # charged as idle SMs.  OFFK_WGRAD_CTAS=n restores the plain "n CTAs" rule.
-        tiles = m_tiles * n_tiles
-        fixed_ctas = int(os.environ.get("OFFK_WGRAD_CTAS", "0"))
-        if fixed_ctas:
-            split = max(1, min(math.ceil(fixed_ctas / tiles), max(1, kb // 4)))
-        else:
-            split = _wgrad_split(tiles, kb, _SM_TARGET * (1 if self.prec == L.PREC_TF32X3 else 2), bk or 32)
+        # charged as idle SMs.
+        split = _wgrad_split(m_tiles * n_tiles, kb, _SM_TARGET * (1 if x3 else 2), bk or 32)
         mk = (lambda *a, **k: TGemm(*a, geom=geom, x_layout=x_layout, wgrad=True, bk=bk, **k)) if tma else Gemm
         # dW[n][m]: consecutive accumulator rows are consecutive addresses -> transposed float4 adds (offk.h: out_vec = 2)
-        rows_vec = (self.tc and dw.data_ptr() % 16 == 0 and geom.kdim % 4 == 0
-                    and os.environ.get("OFFK_WGRAD_VEC", "1") != "0")
+        rows_vec = self.tc and dw.data_ptr() % 16 == 0 and geom.kdim % 4 == 0
         g = mk(self, spc, ("wgrad", x_layout, _gkey(geom)), a_src=x, b_src=dy, out=dw, ones_out=db, a_relu=a_relu,
                atomic=True, split_k=split, name=name + ".wgrad", out_vec=2 if rows_vec else None)
         self.flops_bwd += g.flops
@@ -541,11 +513,11 @@ class OFFEngine:
             gd = T.ConvGeom(geom.n_img, geom.cout, geom.hout, geom.wout, geom.cin, geom.kh, geom.kw, 1,
                             geom.kh - 1 - geom.pad, geom.y_ctot, geom.y_coff, geom.x_ctot, geom.x_coff) if geom.stride == 1 else None
             ex = spc.extra
-            if (self.use_tma and x_layout == "nhwc" and gd is not None and name in self.wd and geom.kh == geom.kw
+            if (x_layout == "nhwc" and gd is not None and name in self.wd and geom.kh == geom.kw
                     and TGemm.eligible(gd, self.prec) and (gd.hout, gd.wout) == (geom.hin, geom.win)):
                 kw_["b_src"] = self.wd[name]
                 g = TGemm(self, spc, ("dgrad", x_layout, _gkey(geom), i), geom=gd, **kw_)
-            elif (self.use_tma and self.tma_strided_dgrad and x_layout == "nhwc" and geom.stride > 1
+            elif (x_layout == "nhwc" and geom.stride > 1
                   and (name, ex["a"], ex["b"]) in self.wd and self.tc and geom.cout % 32 == 0
                   and geom.y_ctot % 4 == 0 and geom.y_coff % 4 == 0 and ex["pad_h"] >= 0 and ex["pad_w"] >= 0):
                 # one stride-parity class = a stride-1 correlation over dY with the class's R x Q taps (free geometry)
@@ -566,7 +538,7 @@ class OFFEngine:
         P, N, B, Lg = self.P, self.N, self.B, self.Lseg
         bf, pr, gr = self.buf, self.params, self.grads
         self.flops_fwd = self.flops_bwd = 0.0
-        fwd, bwd_units, bwd_stage = [], [], []
+        fwd, bwd_stage = [], []
         lib = self.lib
 
         # ============ OFF units (RGB_OFF.py:596-616 and the eight copies)
@@ -578,7 +550,6 @@ class OFFEngine:
         self._st_desc = (L.OffkStencil * n_lv)()      # one contiguous array: stage batches are slices of it
         self._st_io = (L.OffkStencilIO * n_lv)()
         k4_steps = []
-        k4_by_stage = {st: [] for st in S.STAGES}
         for li, (tag, (cin, s)) in enumerate(S.LEVELS.items()):
             st = S.LEVEL_STAGE[tag]
             fl = fwd_lane[st]
@@ -589,8 +560,7 @@ class OFFEngine:
             # K1: gen (ReLU) and down (linear) 1x1 convs as ONE GEMM with 160 output channels
             # 7x7 taps: a 196-byte channel stride is not a legal TMA stride -> one channels-last copy of the tap per
             # step feeds both the forward GEMM (dense tensor map) and the weight gradient (im2col_t), all TMA-fed
-            via_copy = (self.tc and self.use_tma and (s * s) % 4 != 0 and cin % 32 == 0
-                        and os.environ.get("OFFK_NO_TAP_COPY", "0") != "1")
+            via_copy = self.tc and (s * s) % 4 != 0 and cin % 32 == 0
             if via_copy:
                 tapT = self._buf("tapT_" + tag, N, s, s, cin)
 
@@ -628,7 +598,7 @@ class OFFEngine:
             # K4: weight / bias gradient of the fused 1x1 (no dX for the frozen taps unless asked, train_off.py:39-46)
             if via_copy:
                 k4 = self._conv_wgrad("unit_" + tag, tapT, dgd, geom, self._unit_w(self.grads_flat, tag),
-                                      self._unit_b(self.grads_flat, tag), x_layout="nhwc", force_tma=True)
+                                      self._unit_b(self.grads_flat, tag), x_layout="nhwc", tap_copy=True)
             else:
                 k4 = self._conv_wgrad("unit_" + tag, self.taps[tag], dgd, geom,
                                       self._unit_w(self.grads_flat, tag), self._unit_b(self.grads_flat, tag), x_layout="nchw")
@@ -639,15 +609,12 @@ class OFFEngine:
                 grp += [_on(g, li % 3) for g in self._conv_dgrad("unit_" + tag, dgd, self._unit_w(self.params_flat, tag),
                                                                   self.tap_grad[tag], geom, x_layout="nchw")]
             k4_steps += grp
-            k4_by_stage[st] += grp
-        # K2: ONE stencil launch per stage-fusion buffer (its units' GEMMs precede it on the same lane)
+        # K2: the forward stencil in two batched launches: the 28-stage units on their own (they open the critical path);
+        # the 14- and 7-stage units together (the 7x7 levels are 7 MB each: on their own they run at a fifth of the
+        # bandwidth)
         tags = list(S.LEVELS)
-        # forward stencil launches: the 28-stage units on their own (they open the critical path); the 14- and 7-stage
-        # units together (the 7x7 levels are 7 MB each: on their own they run at a fifth of the bandwidth)
-        merge = os.environ.get("OFFK_STENCIL_FWD_MERGE", "1") == "1"
-        groups = [("28", ["28"]), ("14+7", ["14", "7"])] if merge else [(st, [st]) for st in S.STAGES]
         self.stencil_fwd_tags = OrderedDict()         # launch name -> level tags (bench.py: algorithmic bytes)
-        for gname, sts in groups:
+        for gname, sts in (("28", ["28"]), ("14+7", ["14", "7"])):
             lv_tags = [t for st in sts for t in stage_levels[st]]
             i0, n = tags.index(lv_tags[0]), len(lv_tags)
             assert tags[i0:i0 + n] == lv_tags
@@ -660,50 +627,17 @@ class OFFEngine:
             fwd.append(step)
             self.stencil_fwd_steps[gname] = step
             self.stencil_fwd_tags[gname] = lv_tags
-        # K3: the backward of all nine units in ONE launch (every stage gradient dF* is complete by then)
+        # K3: the backward of all nine units in ONE launch (every stage gradient dF* is complete by then), then their weight
+        # gradients.  Running the 7- and 14-stage units' backward early on side lanes, under the rest of the stage chain, was
+        # measured slower at config 2 (2.90 vs 2.84 ms/step): the HBM-bound unit kernels slow the chain more than the
+        # overlap saves.
         grad3 = [gr[f"motion_spatial_grad_{t}.{k}"] for t in tags for k in ("weight", "bias")] if self.variant == "rgb" else []
-
-        # two launches on two lanes: the temporal half streams (dG), the spatial half (dD, tap gradients) is
-        # instruction-heavy; they write disjoint channels of dgd_X, so the pair is exempt from the hazard analysis
-        def k3t(stream):
-            L.check(lib.offk_stencil_diff_bwd_batch_part(n_lv, self._st_desc, self._st_io, 1, stream), "stencil_bwd_temporal")
-
-        def k3s(stream):
-            L.check(lib.offk_stencil_diff_bwd_batch_part(n_lv, self._st_desc, self._st_io, 2, stream), "stencil_bwd_spatial")
-        rd3 = [bf["dF" + st] for st in S.STAGES] + [bf["gd_" + t] for t in tags]
-        k3t = _nm(k3t, "stencil_bwd_temporal", reads=rd3, writes=[bf["dgd_" + t] for t in tags], lane=0)
-        k3s = _nm(k3s, "stencil_bwd_spatial", reads=rd3, writes=[bf["dgd_" + t] for t in tags] + grad3, lane=1)
-        k3s.independent_of = (k3t,)
 
         def k3(stream):
             L.check(lib.offk_stencil_diff_bwd_batch(n_lv, self._st_desc, self._st_io, stream), "stencil_bwd")
-        k3 = _nm(k3, "stencil_bwd", reads=rd3, writes=[bf["dgd_" + t] for t in tags] + grad3, lane=0)
-        # Early unit backward (optional): dF7[:, :320] is final right after motion_conv_trans' data gradient and
-        # dF14[:, :800] after motion_conv_trans_14's, so the 7- and 14-stage units' stencil backward + weight gradients
-        # can run on side lanes under the rest of the stage chain.  Measured at config 2: 2.90 ms/step vs 2.84 ms with
-        # all nine units at the tail -- the HBM-bound unit kernels slow the chain more than the overlap saves -- so off.
-        self.unit_bwd_early = os.environ.get("OFFK_UNIT_BWD_EARLY", "0") == "1"
-        unit_bwd = {}
-        for st, lv_tags in stage_levels.items():
-            i0, n = tags.index(lv_tags[0]), len(lv_tags)
-            g3 = [gr[f"motion_spatial_grad_{t}.{k}"] for t in lv_tags for k in ("weight", "bias")] if self.variant == "rgb" else []
-
-            def k3st(stream, i0=i0, n=n, st=st):
-                L.check(lib.offk_stencil_diff_bwd_batch(n, C.byref(self._st_desc[i0]), C.byref(self._st_io[i0]), stream),
-                        "stencil_bwd_" + st)
-            lane3 = 0 if st == "28" else 2
-            stp = _nm(k3st, "stencil_bwd_" + st, reads=[bf["dF" + st]] + [bf["gd_" + t] for t in lv_tags],
-                      writes=[bf["dgd_" + t] for t in lv_tags] + g3, lane=lane3)
-            grp = list(k4_by_stage[st])
-            if self.unit_bwd_early:
-                for j, g_ in enumerate(grp):                       # early groups stay off lane 0 (the dgrad chain)
-                    g_.lane = (2, 1)[j % 2] if st != "28" else (0, 2, 1)[j % 3]
-            unit_bwd[st] = [stp] + grp
-        if self.unit_bwd_early:
-            bwd_units += unit_bwd["28"]
-        else:
-            bwd_units += [k3t, k3s] if os.environ.get("OFFK_STENCIL_BWD_SPLIT", "0") == "1" else [k3]
-            bwd_units += k4_steps
+        k3 = _nm(k3, "stencil_bwd", reads=[bf["dF" + st] for st in S.STAGES] + [bf["gd_" + t] for t in tags],
+                 writes=[bf["dgd_" + t] for t in tags] + grad3, lane=0)
+        bwd_units = [k3] + k4_steps
 
         # ============ stage convs
         def geom_of(name, n_img, s_in, x_ctot=0, x_coff=0, y_ctot=0, y_coff=0):
@@ -813,8 +747,6 @@ class OFFEngine:
         dgrad("motion_conv_trans", d("t7"), bf["dF7"], g_t7)
         # d sum_14b = (dF7[:,320:] + head-14 pool gradient) * [sum_14b > 0]   (in place in the dF7 slice)
         bs.extend(self._head_bwd("14", self.d_out14, bf["dF7"], 512, 832, 320, "fc_action_motion_14", act=bf["F7"], accumulate=True))
-        if self.unit_bwd_early:          # after the in-place update of dF7[:, 320:], so the main lane never waits on these
-            bs.extend(unit_bwd["7"])
         # ---- 14b:  sum_14b = relu(s14a + relu(conv3_14b(h2b)))
         bs.append(_nm(lambda stream: L.check(lib.offk_gate_copy(_ptr(bf["dF7"]), 832, 320, _ptr(bf["h3_14b"]), 512, 0,
                                                                 _ptr(d("h3_14b")), 512, 0, P, 512, 49, stream), "gate_h3b"),
@@ -839,8 +771,6 @@ class OFFEngine:
         back("motion_conv_trans_14", bf["F14"], d("t14"), g_t14)
         # dF14; channels >= 800 are sum_28c = relu(.) -> gate them here (fc28 contributes nothing)
         dgrad("motion_conv_trans_14", d("t14"), bf["dF14"], g_t14, gate=bf["F14"], gate_col0=800)
-        if self.unit_bwd_early:
-            bs.extend(unit_bwd["14"])
         # ---- 28c / 28b (identity residuals): the incoming gradient of 28c is the dF14 slice [800,1056)
         g_dy_c3c = g_c3c
         back("motion_conv3_trans_28c", bf["h2_28c"], bf["dF14"], g_dy_c3c)
@@ -872,9 +802,8 @@ class OFFEngine:
 
         # weight re-layouts before the forward (one launch), OHWI -> OIHW weight gradients after the backward
         wc, wci, pflat = self.wc_flat, self.wc_idx, self.params_flat
-        wc_lane = int(os.environ.get("OFFK_WC_LANE", "2"))
         pre = [_nm(lambda stream: L.check(lib.offk_gather_copy(_ptr(pflat), _ptr(wci), _ptr(wc), wc.numel(), stream),
-                                          "weight copies"), "weight_copies", writes=[wc], lane=wc_lane)]
+                                          "weight copies"), "weight_copies", writes=[wc], lane=2)]
         if self.presplit:
             # 3xTF32 residuals of every weight, once per step (the GEMMs then get both weight tiles by TMA)
             plo, wlo = self.params_lo, self.wc_lo
@@ -882,7 +811,7 @@ class OFFEngine:
                                                   "weight residuals"), "weight_residuals_params", writes=[plo], lane=0))
             pre.append(_nm(lambda stream: L.check(lib.offk_tf32_residual(_ptr(wc), _ptr(wlo), wc.numel(), stream),
                                                   "weight residuals"), "weight_residuals_copies", reads=[wc], writes=[wlo],
-                           lane=wc_lane))
+                           lane=2))
         # OHWI -> OIHW accumulation of every KxK weight gradient: one launch
         kxk = [(name, cout, cin, k) for name, cout, cin, k, _, _ in S.STAGE_CONVS if k > 1]
         self._unperm = (L.OffkPermute * len(kxk))()
@@ -1147,12 +1076,12 @@ def _auto_tile_n(M: int, N: int, tma: bool = False, x3: bool = False) -> int:
     bn0 = (N + 15) // 16 * 16 if N <= 256 else 256
     want, enough = (120, 140)
     if tma:         # (2 x 148 before the MMA issue path was fixed: narrow tiles were issue-bound then; profiles/env_r03t.log)
-        want = enough = int(os.environ.get("OFFK_TF32_WANT_CTAS", str(_SM_TARGET)))
+        want = enough = _TF32_WANT_CTAS
     if tma and x3:
         # 3xTF32: one CTA per SM, and every extra N tile repeats the A tile AND its residual pass (motion_conv_trans_28,
         # 147 x 1 tiles of 64: two tiles of 32 took 586 us against 371 us; unit_5a, 56 M tiles: five tiles of 32 columns
         # 38 us against ~20 for one of 160).  Only the 37-tile 7x7 layers are narrowed (sweep: profiles/env_r03s.log)
-        want = enough = int(os.environ.get("OFFK_X3_WANT_CTAS", "40"))
+        want = enough = _X3_WANT_CTAS
     if mt * math.ceil(N / bn0) >= want:
         return 0
     best = 0
@@ -1220,8 +1149,6 @@ class Schedule:
             for j in range(i):
                 if lanes[j] == lanes[i] or j <= covered[lanes[i]][lanes[j]]:
                     continue
-                if self.steps[j] in getattr(self.steps[i], "independent_of", ()):
-                    continue                      # declared to touch disjoint elements of the same buffers
                 if hit(wr[j], rd[i]) or hit(wr[j], wr[i]) or hit(rd[j], wr[i]):
                     need[lanes[j]] = j
             for lane_j, j in need.items():

@@ -511,19 +511,6 @@ def test_stencil_batch_equals_single_launches(dev):
     for gd, w, bias, bufs in keep:
         assert torch.equal(bufs["b"][0], bufs["s"][0])                                   # dG, dD: bit-exact
         assert _rel(bufs["b"][1], bufs["s"][1].cpu()) < 1e-5 and _rel(bufs["b"][2], bufs["s"][2].cpu()) < 1e-5  # atomics: order
-    # the two halves as separate launches (offk_stencil_diff_bwd_batch_part) = the one-launch backward
-    parts = []
-    for i in range(n):
-        gd, w, bias, bufs = keep[i]
-        dgd, dw, db = torch.full_like(gd, float("nan")), torch.zeros_like(w), torch.zeros_like(bias)
-        ios[i].dg, ios[i].dd, ios[i].dw, ios[i].dbias = dgd.data_ptr(), dgd.data_ptr() + 4 * Cg, dw.data_ptr(), db.data_ptr()
-        parts.append((dgd, dw, db))
-    L.check(lib.offk_stencil_diff_bwd_batch_part(n, descs, ios, 2, None), "bwd spatial half")
-    L.check(lib.offk_stencil_diff_bwd_batch_part(n, descs, ios, 1, None), "bwd temporal half")
-    torch.cuda.synchronize()
-    for (gd, w, bias, bufs), (dgd, dw, db) in zip(keep, parts):
-        assert torch.equal(dgd, bufs["b"][0])
-        assert _rel(dw, bufs["b"][1].cpu()) < 1e-5 and _rel(db, bufs["b"][2].cpu()) < 1e-5
 
 
 def test_layout_helpers(dev):

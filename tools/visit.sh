@@ -20,11 +20,6 @@ for w in "$@"; do
       timeout -k 5 900 python bench.py --config 4 --no-cpu-baseline --no-gpu-baseline > $OUT/bench_cfg4_$TAG.json 2> $OUT/bench_cfg4_$TAG.err; echo "bench cfg4 exit $?"; cut -c1-330 $OUT/bench_cfg4_$TAG.json; tail -3 $OUT/bench_cfg4_$TAG.err;;
     launches_tf32) bash tools/visit_l.sh $TAG tf32 | tail -24;;
     launches_fp32) bash tools/visit_l.sh $TAG fp32 | tail -24;;
-    split_sweep)
-      rm -f $OUT/split_sweep_$TAG.log
-      for sp in 1 2 3 4; do echo "== motion_conv_trans_28 split $sp (fp32)" >> $OUT/split_sweep_$TAG.log
-        OFFK_FWD_SPLIT=motion_conv_trans_28=$sp timeout -k 5 300 python tools/issue_time.py 48 3 fp32 2>&1 | grep -E "GRAPH replay both" >> $OUT/split_sweep_$TAG.log; done
-      cat $OUT/split_sweep_$TAG.log;;
     smoke)
       timeout 600 python -c 'import __graft_entry__ as g; g.smoke()' > $OUT/smoke_$TAG.log 2>&1; echo "smoke exit $?"; tail -3 $OUT/smoke_$TAG.log;;
   esac
