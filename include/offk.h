@@ -35,7 +35,6 @@ extern "C" {
 #define OFFK_E_LIMIT    (-3)  /* size beyond what the kernel supports        */
 
 /* arithmetic of the dense contractions */
-#define OFFK_PREC_FP32   0 /* CUDA-core FFMA, fp32 accumulate: slow cross-check of the tensor-core modes (tests)       */
 #define OFFK_PREC_TF32   1 /* tcgen05.mma kind::tf32, operands in smem, fp32 accumulate in TMEM                        */
 #define OFFK_PREC_TF32X3 2 /* fp32-parity mode on the tensor cores (the reference computes in fp32, RGB_OFF.py:597):
                               every operand tile x is used as hi = trunc_tf32(x) (what kind::tf32 reads anyway) plus a
@@ -62,11 +61,15 @@ int offk_device_info(int* sm_count, int* cc_major, int* cc_minor, long long* l2_
 /* ------------------------------------------------------------------------
  * Gather-GEMM:  D[m,n] = sum_k A(m,k) * B(n,k),  then a fused epilogue.
  *
- * Every dense contraction on the path is this one kernel: the 1x1
- * channel-reduction convs of the nine OFF units (RGB_OFF.py:597,610 ...),
- * the stage-entry 7x7/5x5/3x3 convs (:657,:762,:833), the residual-block
- * convs (:659-685,:764-780,:835-841), the three FC heads (:787,:793,:847) and
- * the data-/weight-gradient of all of them (autograd, train_off.py:136-146).
+ * The contractions whose operands no TMA tensor map describes (offk_tma_gemm below carries every forward conv and
+ * every stage-conv data gradient).  The engine launches it for
+ *   - the weight gradients of the stage convs (RGB_OFF.py:657-685,762-780,833-841; autograd, train_off.py:136-146) in
+ *     the tf32 mode, except motion_conv_trans_28: A = im2col(x)^T and B = dY, both OFFK_LOAD_VEC_ROW, out_vec = 2
+ *     (dW rows contiguous) and the all-ones row for the bias gradient, with or without split-K;
+ *   - the data gradients of the nine OFF units' fused 1x1 conv (RGB_OFF.py:597,610 ...) into the NCHW taps, when the
+ *     caller asks for tap gradients: A = dY (OFFK_LOAD_VEC_K), B = the weights (OFFK_LOAD_VEC_ROW), a plain store
+ *     through the out tables.
+ * The other two pairings of the load modes are accepted as well; tables.py picks a mode from each operand's layout.
  * What differs per layer is only WHERE element (m,k) / (n,k) / (m,n) lives;
  * that is described by separable index tables built once per layer geometry
  * (by the host: optical-flow-guided-feature-pytorch_b200/tables.py builds them with numpy for forward,
@@ -93,10 +96,9 @@ int offk_device_info(int* sm_count, int* cc_major, int* cc_minor, long long* l2_
  * a_col carry y = -16384 (the box test is always on; pass a_h = a_w = 32767 for "no box"), padding entries of
  * b_row / b_col are 0.  The entry of a_ones_row is never gathered.
  * ---------------------------------------------------------------------- */
-/* Operand fetch modes.  The tables are always element-granular; a vector mode is a promise by the caller
- * that groups of 4 consecutive indices are contiguous in memory, 16-byte aligned and share validity. */
-#define OFFK_LOAD_SCALAR_ROW 0 /* 4-byte loads, lanes walk rows (source contiguous along m / n)                 */
-#define OFFK_LOAD_SCALAR_K   1 /* 4-byte loads, lanes walk k    (source contiguous along k)                     */
+/* Operand fetch modes.  The tables are always element-granular; a load mode is a promise by the caller
+ * that groups of 4 consecutive indices are contiguous in memory, 16-byte aligned and share validity
+ * (a_src and b_src 16-byte aligned).  An operand without such groups cannot be launched. */
 #define OFFK_LOAD_VEC_K      2 /* 16-byte loads of 4 consecutive k (K % 4 == 0): NHWC activations, dense weights */
 #define OFFK_LOAD_VEC_ROW    3 /* 16-byte cp.async of 4 consecutive rows straight into the MN-major swizzled tile (the
                                   operand is then marked MN-major for tcgen05.mma; nothing is transposed): NCHW taps
@@ -115,7 +117,6 @@ typedef struct offk_gemm {
   const offk_idx_t* a_row; /* [M] */
   const offk_idx_t* a_col; /* [K] */
   int32_t a_h, a_w;        /* validity box (>= 1); 32767 = every real element is valid */
-  int32_t a_relu;          /* max(.,0) on load (consumer of a pre-activation tensor, RGB_OFF.py:658) */
   int32_t a_ones_row;      /* -1, or the row whose A values are all 1 */
   int32_t a_mode;          /* OFFK_LOAD_*: how the producer warps may fetch this operand */
   /* B operand */

@@ -12,10 +12,10 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("OFFK_LIB") or os.path.join(_HERE, "liboffk.so")   # OFFK_LIB: bring-up builds only
 
-PREC_FP32, PREC_TF32, PREC_TF32X3 = 0, 1, 2
+PREC_TF32, PREC_TF32X3 = 1, 2
 INDEX_REFERENCE_FLAT, INDEX_ALIGNED = 0, 1
 DROP_NONE, DROP_MASK, DROP_SEED = 0, 1, 2
-LOAD_SCALAR_ROW, LOAD_SCALAR_K, LOAD_VEC_K, LOAD_VEC_ROW = 0, 1, 2, 3
+LOAD_VEC_K, LOAD_VEC_ROW = 2, 3
 
 
 class OffkIdx(C.Structure):
@@ -27,8 +27,7 @@ class OffkGemm(C.Structure):
     _fields_ = [
         ("M", C.c_int32), ("N", C.c_int32), ("K", C.c_int32),
         ("a_src", C.c_void_p), ("a_row", C.c_void_p), ("a_col", C.c_void_p),
-        ("a_h", C.c_int32), ("a_w", C.c_int32), ("a_relu", C.c_int32), ("a_ones_row", C.c_int32),
-        ("a_mode", C.c_int32),
+        ("a_h", C.c_int32), ("a_w", C.c_int32), ("a_ones_row", C.c_int32), ("a_mode", C.c_int32),
         ("b_src", C.c_void_p), ("b_row", C.c_void_p), ("b_col", C.c_void_p), ("b_mode", C.c_int32),
         ("out", C.c_void_p), ("out_row", C.c_void_p), ("out_col", C.c_void_p),
         ("bias", C.c_void_p), ("relu_pre_cols", C.c_int32),

@@ -9,7 +9,7 @@ mkdir -p "$ODIR"
 NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
 FLAGS=(-O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -Xcompiler -fPIC -Xptxas -v
        -I"$ROOT/include" -I"$HERE" ${OFFK_EXTRA_FLAGS:-})
-SRCS=(offk_api offk_gemm_simt offk_gemm_tc offk_gemm_tma offk_stencil offk_head offk_train)
+SRCS=(offk_api offk_gemm_tc offk_gemm_tma offk_stencil offk_head offk_train)
 OBJS=()
 PIDS=()
 for f in "${SRCS[@]}"; do

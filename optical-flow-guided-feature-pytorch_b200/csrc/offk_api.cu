@@ -42,15 +42,15 @@ extern "C" int offk_gather_gemm(const offk_gemm_t* g, int precision, void* strea
   OFFK_REQUIRE(g->a_src && g->a_row && g->a_col && g->b_src && g->b_row && g->b_col, "gather_gemm: operand tables");
   OFFK_REQUIRE(g->out && g->out_row && g->out_col, "gather_gemm: output tables");
   OFFK_REQUIRE(g->a_ones_row < 0 || g->a_ones_row < g->M, "gather_gemm: a_ones_row out of range");
-  OFFK_REQUIRE(g->a_mode >= 0 && g->a_mode <= 3 && g->b_mode >= 0 && g->b_mode <= 3, "gather_gemm: bad load mode");
-  if (g->a_mode >= OFFK_LOAD_VEC_K) OFFK_REQUIRE((reinterpret_cast<uintptr_t>(g->a_src) & 15u) == 0, "gather_gemm: a_src alignment");
-  if (g->b_mode >= OFFK_LOAD_VEC_K) OFFK_REQUIRE((reinterpret_cast<uintptr_t>(g->b_src) & 15u) == 0, "gather_gemm: b_src alignment");
+  OFFK_REQUIRE(g->a_mode >= OFFK_LOAD_VEC_K && g->a_mode <= OFFK_LOAD_VEC_ROW && g->b_mode >= OFFK_LOAD_VEC_K &&
+               g->b_mode <= OFFK_LOAD_VEC_ROW, "gather_gemm: bad load mode");
+  OFFK_REQUIRE((reinterpret_cast<uintptr_t>(g->a_src) & 15u) == 0, "gather_gemm: a_src alignment");
+  OFFK_REQUIRE((reinterpret_cast<uintptr_t>(g->b_src) & 15u) == 0, "gather_gemm: b_src alignment");
   if (g->a_mode == OFFK_LOAD_VEC_K || g->b_mode == OFFK_LOAD_VEC_K) OFFK_REQUIRE((g->K & 3) == 0, "gather_gemm: VEC_K needs K %% 4 == 0");
   if (g->out_vec == 1) OFFK_REQUIRE((g->N & 3) == 0 && (reinterpret_cast<uintptr_t>(g->out) & 15u) == 0, "gather_gemm: out_vec alignment");
   if (g->out_vec == 2)
-    OFFK_REQUIRE((reinterpret_cast<uintptr_t>(g->out) & 15u) == 0 && !g->bias && !g->gate && !g->addend && !g->relu_pre_cols && !g->relu_post &&
-                 precision != OFFK_PREC_FP32, "gather_gemm: out_vec = 2 needs a tensor-core precision, a 16-byte aligned `out` and a plain epilogue");
-  if (precision == OFFK_PREC_FP32) return launch_gemm_simt(*g, as_stream(stream));
+    OFFK_REQUIRE((reinterpret_cast<uintptr_t>(g->out) & 15u) == 0 && !g->bias && !g->gate && !g->addend && !g->relu_pre_cols && !g->relu_post,
+                 "gather_gemm: out_vec = 2 needs a 16-byte aligned `out` and a plain epilogue");
   if (precision == OFFK_PREC_TF32) return launch_gemm_tc(*g, as_stream(stream), false);
   if (precision == OFFK_PREC_TF32X3) return launch_gemm_tc(*g, as_stream(stream), true);
   return fail(OFFK_E_BADARG, "gather_gemm: unknown precision %d", precision);

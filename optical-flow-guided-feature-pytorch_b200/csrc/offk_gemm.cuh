@@ -1,21 +1,8 @@
-// Gather-GEMM pieces shared by the fp32 CUDA-core kernel and the tcgen05 kernel.
+// Gather-GEMM epilogue pieces shared by the gather-fed and the TMA-fed tcgen05 kernels.
 #pragma once
 #include "offk_common.cuh"
 
 namespace offk {
-
-// A(m,k) for the scalar paths.  r/c are the table entries of row m and column k.
-__device__ __forceinline__ float gemm_load_a(const offk_gemm_t& g, offk_idx_t r, offk_idx_t c, bool ones) {
-  if (ones) return 1.0f;
-  const int y = (int)r.y + (int)c.y, x = (int)r.x + (int)c.x;
-  const bool ok = (g.a_h == 0) || ((unsigned)y < (unsigned)g.a_h && (unsigned)x < (unsigned)g.a_w);
-  float v = 0.f;
-  if (ok) {
-    v = __ldg(g.a_src + (r.off + c.off));
-    if (g.a_relu) v = fmaxf(v, 0.f);
-  }
-  return v;
-}
 
 // Per-row state of the epilogue (one accumulator row m).
 struct EpiRow {
@@ -54,7 +41,6 @@ __device__ __forceinline__ void epi_store(const offk_gemm_t& g, const EpiRow& r,
   g.out[r.out + oc] = v;
 }
 
-int launch_gemm_simt(const offk_gemm_t& g, cudaStream_t st);
 int launch_gemm_tc(const offk_gemm_t& g, cudaStream_t st, bool x3);
 
 }  // namespace offk

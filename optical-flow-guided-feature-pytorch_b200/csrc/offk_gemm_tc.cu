@@ -1,16 +1,14 @@
-// tcgen05 gather-GEMM (OFFK_PREC_TF32) for sm_100a.
+// tcgen05 gather-GEMM (OFFK_PREC_TF32 / OFFK_PREC_TF32X3) for sm_100a: the operands that no TMA tensor map describes
+// (offk.h lists what the engine launches it for).
 //
 //   D[128 x BN] (fp32, TMEM) += A[128 x 32] (tf32, smem) * B[BN x 32]^T (tf32, smem)   per K-block
 //
 // Warp roles (288 threads):
-//   warps 0-7  producers: gather A and B through the index tables (NHWC implicit-GEMM im2col / col2im,
-//              NCHW taps, pixel-major weight-gradient operands), with 16-byte loads wherever the
-//              caller promises contiguity: 16-byte cp.async straight into shared memory, never through
-//              registers.  OFFK_LOAD_VEC_K (source contiguous along k) fills the canonical K-major
-//              SWIZZLE_128B tile; OFFK_LOAD_VEC_ROW (source contiguous along m / n: NCHW taps as A(m = pixel),
-//              channels-last tensors in weight- and data-gradient GEMMs) fills the canonical MN-major
-//              SWIZZLE_128B tile and the instruction descriptor marks that operand MN-major, so no transpose
-//              is ever executed.  The scalar modes go through registers.  Producers then fence to the async
+//   warps 0-7  producers: gather A and B through the index tables with 16-byte cp.async straight into
+//              shared memory, never through registers.  OFFK_LOAD_VEC_K (source contiguous along k) fills
+//              the canonical K-major SWIZZLE_128B tile; OFFK_LOAD_VEC_ROW (source contiguous along m / n)
+//              fills the canonical MN-major SWIZZLE_128B tile and the instruction descriptor marks that
+//              operand MN-major, so no transpose is ever executed.  Producers then fence to the async
 //              proxy and arrive on the stage's "full" mbarrier.  After the main loop the same
 //              warps run the epilogue: tcgen05.ld the accumulator rows out of TMEM, apply
 //              bias / ReLU / gate / residual, store coalesced along pixels (or atomically for
@@ -55,16 +53,16 @@ __device__ __forceinline__ Idx2 ld_idx(const offk_idx_t* p) {
   return Idx2{(int)v.x, v.y};
 }
 
-// ============================ A operand (validity box, ReLU-on-load, ones row)
+// ============================ A operand (validity box, ones row)
 // VEC_K  : thread = (row (tid>>3)+32i, chunk tid&7), i < 4.   cp.async, zero-fill for invalid.   K-major tile.
 // VEC_ROW: thread = (row-quad tid&31, column (tid>>5)+8i), i < 4.   cp.async, zero-fill.          MN-major tile.
 template <int MODE>
 struct LoaderA {
+  static_assert(MODE == OFFK_LOAD_VEC_K || MODE == OFFK_LOAD_VEC_ROW, "gather-GEMM operands are 16-byte vector loads");
   Idx2 r[4];
   uint32_t dst[4];
   uint32_t ones;       // VEC_K: bit i; VEC_ROW: bit 0
   Idx2 c_cur[4], c_nxt[4];
-  float4 d_cur[4], d_nxt[4];
   __device__ __forceinline__ void init(const offk_gemm_t& g, int m0, int tid) {
     const int warp = tid >> 5, lane = tid & 31;
     ones = 0;
@@ -76,89 +74,27 @@ struct LoaderA {
         dst[i] = swz(tr, tid & 7);
         ones |= (m0 + tr == g.a_ones_row ? 1u : 0u) << i;
       }
-    } else if (MODE == OFFK_LOAD_VEC_ROW) {
+    } else {
       r[0] = ld_idx(g.a_row + m0 + 4 * lane);
 #pragma unroll
       for (int i = 0; i < 4; ++i) dst[i] = swz_mn(lane, warp + 8 * i, TC_BM / 32);
       ones = (m0 + 4 * lane == g.a_ones_row) ? 1u : 0u;
-    } else if (MODE == OFFK_LOAD_SCALAR_ROW) {
-      r[0] = ld_idx(g.a_row + m0 + (tid & 127));
-      ones = (m0 + (tid & 127) == g.a_ones_row) ? 1u : 0u;
     }
   }
   __device__ __forceinline__ void fetch_cols(const offk_gemm_t& g, int k0, int tid, Idx2 (&c)[4]) const {
     if (MODE == OFFK_LOAD_VEC_K) {
       c[0] = ld_idx(g.a_col + k0 + 4 * (tid & 7));
-    } else if (MODE == OFFK_LOAD_VEC_ROW) {
+    } else {
 #pragma unroll
       for (int i = 0; i < 4; ++i) c[i] = ld_idx(g.a_col + k0 + (tid >> 5) + 8 * i);
     }
   }
-  // register-staged load of the K-block whose column entries are `c` (scalar modes)
-  __device__ __forceinline__ void load(const offk_gemm_t& g, const Idx2 (&c)[4], int m0, int k0, int tid,
-                                       float4 (&v)[4]) const {
-    if (MODE == OFFK_LOAD_SCALAR_ROW) {
-      const int half = tid >> 7;
-      float t[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const Idx2 cc = ld_idx(g.a_col + k0 + half * 16 + i);
-        float x = 0.f;
-        if (ones) x = (short)(cc.yx & 0xFFFFu) > -8192 ? 1.f : 0.f;
-        else if (box_ok(g, r[0].yx, cc.yx)) x = __ldg(g.a_src + (r[0].off + cc.off));
-        t[i] = x;
-      }
-#pragma unroll
-      for (int i = 0; i < 4; ++i) v[i] = make_float4(t[4 * i], t[4 * i + 1], t[4 * i + 2], t[4 * i + 3]);
-    } else if (MODE == OFFK_LOAD_SCALAR_K) {   // lane owns column k0+lane, warp w owns tile rows w + 8*i
-      const int warp = tid >> 5, lane = tid & 31;
-      const Idx2 cc = ld_idx(g.a_col + k0 + lane);
-      float t[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const int m = m0 + warp + 8 * i;
-        const Idx2 rr = ld_idx(g.a_row + m);
-        float x = 0.f;
-        if (m == g.a_ones_row) x = (short)(cc.yx & 0xFFFFu) > -8192 ? 1.f : 0.f;
-        else if (box_ok(g, rr.yx, cc.yx)) x = __ldg(g.a_src + (rr.off + cc.off));
-        t[i] = x;
-      }
-#pragma unroll
-      for (int i = 0; i < 4; ++i) v[i] = make_float4(t[4 * i], t[4 * i + 1], t[4 * i + 2], t[4 * i + 3]);
-    }
-  }
-  // lo_off != 0 (3xTF32): the tf32 residual of every element goes to the twin tile lo_off bytes further
-  __device__ __forceinline__ void store(const offk_gemm_t& g, uint32_t tile, int tid, float4 (&v)[4], uint32_t lo_off) const {
-    if (g.a_relu) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) v[i] = f4relu(v[i]);
-    }
-    if (MODE == OFFK_LOAD_SCALAR_ROW) {
-      const int tr = tid & 127, half = tid >> 7;
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        const uint32_t d = tile + swz(tr, half * 4 + c);
-        sts128(d, v[c].x, v[c].y, v[c].z, v[c].w);
-        if (lo_off) sts128(d + lo_off, tf32_lo(v[c].x), tf32_lo(v[c].y), tf32_lo(v[c].z), tf32_lo(v[c].w));
-      }
-    } else if (MODE == OFFK_LOAD_SCALAR_K) {
-      const int warp = tid >> 5, lane = tid & 31;
-      const float t[16] = {v[0].x, v[0].y, v[0].z, v[0].w, v[1].x, v[1].y, v[1].z, v[1].w,
-                           v[2].x, v[2].y, v[2].z, v[2].w, v[3].x, v[3].y, v[3].z, v[3].w};
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const uint32_t d = tile + swz(warp + 8 * i, lane >> 2) + (lane & 3) * 4;
-        sts32(d, t[i]);
-        if (lo_off) sts32(d + lo_off, tf32_lo(t[i]));
-      }
-    }
-  }
-  // 3xTF32, cp.async modes: residuals of the chunks THIS thread copied (they have landed: cp.async.wait_group)
+  // 3xTF32: residuals of the chunks THIS thread copied (they have landed: cp.async.wait_group)
   __device__ __forceinline__ void split_async(uint32_t tile, uint32_t lo_off) const {
 #pragma unroll
     for (int i = 0; i < 4; ++i) split_chunk(tile + dst[i], lo_off);
   }
-  // VEC_K / VEC_ROW: straight to shared memory.  Returns true when st.shared was used (ones row).
+  // straight to shared memory.  Returns true when st.shared was used (ones row).
   __device__ __forceinline__ bool issue_async(const offk_gemm_t& g, const Idx2 (&c)[4], uint32_t tile) const {
     bool stored = false;
     if (MODE == OFFK_LOAD_VEC_K) {
@@ -189,49 +125,24 @@ struct LoaderA {
     }
     return stored;
   }
-  static constexpr bool kAsync = (MODE == OFFK_LOAD_VEC_K || MODE == OFFK_LOAD_VEC_ROW);
   static constexpr bool kMN = (MODE == OFFK_LOAD_VEC_ROW);
-  static constexpr bool kVec = (MODE == OFFK_LOAD_VEC_K || MODE == OFFK_LOAD_VEC_ROW);
-  __device__ __forceinline__ void prologue(const offk_gemm_t& g, int m0, int k_first, int tid) {
-    if (kVec) fetch_cols(g, k_first, tid, c_cur);
-    if (!kAsync) {
-      load(g, c_cur, m0, k_first, tid, d_cur);
-      if (kVec) fetch_cols(g, k_first + TC_BK, tid, c_cur);
-    }
-  }
-  __device__ __forceinline__ void pre_wait(const offk_gemm_t& g, int m0, int k0, int tid, bool has_next) {
-    if (kAsync) {
-      fetch_cols(g, k0 + TC_BK, tid, c_nxt);
-    } else {
-      if (has_next) load(g, c_cur, m0, k0 + TC_BK, tid, d_nxt);
-      if (kVec) fetch_cols(g, k0 + 2 * TC_BK, tid, c_nxt);
-    }
-  }
-  __device__ __forceinline__ bool post_wait(const offk_gemm_t& g, uint32_t tile, int tid, uint32_t lo_off = 0) {
-    bool stored;
-    if (kAsync) {
-      stored = issue_async(g, c_cur, tile);
-    } else {
-      store(g, tile, tid, d_cur, lo_off);
-      stored = true;
+  __device__ __forceinline__ void prologue(const offk_gemm_t& g, int k_first, int tid) { fetch_cols(g, k_first, tid, c_cur); }
+  __device__ __forceinline__ void pre_wait(const offk_gemm_t& g, int k0, int tid) { fetch_cols(g, k0 + TC_BK, tid, c_nxt); }
+  __device__ __forceinline__ bool post_wait(const offk_gemm_t& g, uint32_t tile) {
+    const bool stored = issue_async(g, c_cur, tile);
 #pragma unroll
-      for (int q = 0; q < 4; ++q) d_cur[q] = d_nxt[q];
-    }
-    if (kVec) {
-#pragma unroll
-      for (int q = 0; q < 4; ++q) c_cur[q] = c_nxt[q];
-    }
+    for (int q = 0; q < 4; ++q) c_cur[q] = c_nxt[q];
     return stored;
   }
 };
 
-// ============================ B operand (plain gather, up to 256 rows = two 128-row passes)
+// ============================ B operand (plain gather, up to 256 rows)
 template <int MODE>
 struct LoaderB {
+  static_assert(MODE == OFFK_LOAD_VEC_K || MODE == OFFK_LOAD_VEC_ROW, "gather-GEMM operands are 16-byte vector loads");
   int r[8];            // VEC_K: rows (tid>>3)+32i, i<8;  VEC_ROW: row-quads of pass 0 / pass 1 in r[0], r[1]
   uint32_t dst[8];
   int c_cur[4], c_nxt[4];
-  float4 d_cur[4], d_nxt[4];
   int bn;
   __device__ __forceinline__ void init(const offk_gemm_t& g, int n0, int bn_, int tid) {
     bn = bn_;
@@ -243,7 +154,7 @@ struct LoaderB {
         r[i] = __ldg(g.b_row + n0 + (tr < bn ? tr : 0));
         dst[i] = swz(tr, tid & 7);
       }
-    } else if (MODE == OFFK_LOAD_VEC_ROW) {
+    } else {
       // MN-major tile: thread = (row-quad lane of pass p, column warp+8i); atoms ordered [k-group][n-atom]
       const int atoms = (bn + 31) >> 5;
 #pragma unroll
@@ -258,69 +169,19 @@ struct LoaderB {
   __device__ __forceinline__ void fetch_cols(const offk_gemm_t& g, int k0, int tid, int (&c)[4]) const {
     if (MODE == OFFK_LOAD_VEC_K) {
       c[0] = __ldg(g.b_col + k0 + 4 * (tid & 7));
-    } else if (MODE == OFFK_LOAD_VEC_ROW) {
+    } else {
 #pragma unroll
       for (int i = 0; i < 4; ++i) c[i] = __ldg(g.b_col + k0 + (tid >> 5) + 8 * i);
     }
   }
-  __device__ __forceinline__ void load(const offk_gemm_t& g, const int (&c)[4], int n0, int k0, int tid, int pass,
-                                       float4 (&v)[4]) const {
-    if (MODE == OFFK_LOAD_SCALAR_ROW) {
-      // thread = row (tid & 127) of this pass, k-half (tid >> 7): 16 scalar gathers
-      const int tr = 128 * pass + (tid & 127), half = tid >> 7;
-      const int rb = __ldg(g.b_row + n0 + (tr < bn ? tr : 0));
-      float t[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) t[i] = tr < bn ? __ldg(g.b_src + (rb + __ldg(g.b_col + k0 + half * 16 + i))) : 0.f;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) v[i] = make_float4(t[4 * i], t[4 * i + 1], t[4 * i + 2], t[4 * i + 3]);
-    } else if (MODE == OFFK_LOAD_SCALAR_K) {
-      const int warp = tid >> 5, lane = tid & 31;
-      const int cc = __ldg(g.b_col + k0 + lane);
-      float t[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const int tr = 128 * pass + warp + 8 * i;
-        t[i] = tr < bn ? __ldg(g.b_src + (__ldg(g.b_row + n0 + tr) + cc)) : 0.f;
-      }
-#pragma unroll
-      for (int i = 0; i < 4; ++i) v[i] = make_float4(t[4 * i], t[4 * i + 1], t[4 * i + 2], t[4 * i + 3]);
-    }
-  }
-  __device__ __forceinline__ void store(uint32_t tile, int tid, int pass, const float4 (&v)[4], uint32_t lo_off) const {
-    if (MODE == OFFK_LOAD_SCALAR_ROW) {
-      const int tr = 128 * pass + (tid & 127), half = tid >> 7;
-      if (tr < bn) {
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          const uint32_t d = tile + swz(tr, half * 4 + c);
-          sts128(d, v[c].x, v[c].y, v[c].z, v[c].w);
-          if (lo_off) sts128(d + lo_off, tf32_lo(v[c].x), tf32_lo(v[c].y), tf32_lo(v[c].z), tf32_lo(v[c].w));
-        }
-      }
-    } else if (MODE == OFFK_LOAD_SCALAR_K) {
-      const int warp = tid >> 5, lane = tid & 31;
-      const float t[16] = {v[0].x, v[0].y, v[0].z, v[0].w, v[1].x, v[1].y, v[1].z, v[1].w,
-                           v[2].x, v[2].y, v[2].z, v[2].w, v[3].x, v[3].y, v[3].z, v[3].w};
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const int tr = 128 * pass + warp + 8 * i;
-        if (tr < bn) {
-          const uint32_t d = tile + swz(tr, lane >> 2) + (lane & 3) * 4;
-          sts32(d, t[i]);
-          if (lo_off) sts32(d + lo_off, tf32_lo(t[i]));
-        }
-      }
-    }
-  }
-  // 3xTF32, cp.async modes: residuals of the chunks THIS thread copied (same predicates as post_wait)
+  // 3xTF32: residuals of the chunks THIS thread copied (same predicates as post_wait)
   __device__ __forceinline__ void split_async(uint32_t tile, int tid, uint32_t lo_off) const {
     if (MODE == OFFK_LOAD_VEC_K) {
       const int nrow = (bn + 31) >> 5;
 #pragma unroll
       for (int i = 0; i < 8; ++i)
         if (i < nrow && (tid >> 3) + 32 * i < bn) split_chunk(tile + dst[i], lo_off);
-    } else if (MODE == OFFK_LOAD_VEC_ROW) {
+    } else {
 #pragma unroll
       for (int p = 0; p < 2; ++p)
         if (128 * p + 4 * (tid & 31) < bn) {
@@ -329,53 +190,25 @@ struct LoaderB {
         }
     }
   }
-  static constexpr bool kAsync = (MODE == OFFK_LOAD_VEC_K || MODE == OFFK_LOAD_VEC_ROW);
   static constexpr bool kMN = (MODE == OFFK_LOAD_VEC_ROW);
-  static constexpr bool kVec = (MODE == OFFK_LOAD_VEC_K || MODE == OFFK_LOAD_VEC_ROW);
-  __device__ __forceinline__ void prologue(const offk_gemm_t& g, int n0, int k_first, int tid) {
-    if (kVec) fetch_cols(g, k_first, tid, c_cur);
-    if (!kAsync) {
-      load(g, c_cur, n0, k_first, tid, 0, d_cur);
-      if (kVec) fetch_cols(g, k_first + TC_BK, tid, c_cur);
-    }
-  }
-  __device__ __forceinline__ void pre_wait(const offk_gemm_t& g, int n0, int k0, int tid, bool has_next) {
-    if (kAsync) {
-      fetch_cols(g, k0 + TC_BK, tid, c_nxt);
-    } else {
-      if (has_next) load(g, c_cur, n0, k0 + TC_BK, tid, 0, d_nxt);
-      if (kVec) fetch_cols(g, k0 + 2 * TC_BK, tid, c_nxt);
-    }
-  }
-  __device__ __forceinline__ void post_wait(const offk_gemm_t& g, uint32_t tile, int n0, int k0, int tid, uint32_t lo_off = 0) {
+  __device__ __forceinline__ void prologue(const offk_gemm_t& g, int k_first, int tid) { fetch_cols(g, k_first, tid, c_cur); }
+  __device__ __forceinline__ void pre_wait(const offk_gemm_t& g, int k0, int tid) { fetch_cols(g, k0 + TC_BK, tid, c_nxt); }
+  __device__ __forceinline__ void post_wait(const offk_gemm_t& g, uint32_t tile, int tid) {
     if (MODE == OFFK_LOAD_VEC_K) {
       const int nrow = (bn + 31) >> 5;          // 32 rows per i
 #pragma unroll
       for (int i = 0; i < 8; ++i)
         if (i < nrow && (tid >> 3) + 32 * i < bn) cp_async16_cg(tile + dst[i], g.b_src + (r[i] + c_cur[0]), 16u);
-    } else if (MODE == OFFK_LOAD_VEC_ROW) {
+    } else {
 #pragma unroll
       for (int p = 0; p < 2; ++p)
         if (128 * p + 4 * (tid & 31) < bn) {
 #pragma unroll
           for (int i = 0; i < 4; ++i) cp_async16_cg(tile + dst[p] + i * dst[2], g.b_src + (r[p] + c_cur[i]), 16u);
         }
-    } else {
-      store(tile, tid, 0, d_cur, lo_off);
-      if (bn > 128) {   // second pass of a wide tile: not prefetched (only gradient GEMMs wider than 128)
-        int ct[4];
-        float4 vt[4];
-        if (kVec) fetch_cols(g, k0, tid, ct);
-        load(g, ct, n0, k0, tid, 1, vt);
-        store(tile, tid, 1, vt, lo_off);
-      }
-#pragma unroll
-      for (int q = 0; q < 4; ++q) d_cur[q] = d_nxt[q];
     }
-    if (kVec) {
 #pragma unroll
-      for (int q = 0; q < 4; ++q) c_cur[q] = c_nxt[q];
-    }
+    for (int q = 0; q < 4; ++q) c_cur[q] = c_nxt[q];
   }
 };
 
@@ -424,15 +257,15 @@ gather_gemm_tc_kernel(const offk_gemm_t g, int bn, int stages, int kb_per_split,
 
   if (warp < 8) {
     // ================= producers =================
-    // VEC_K operands go global->smem with cp.async (up to `stages` K-blocks in flight, no registers); the other
-    // modes are staged through registers with the NEXT K-block's loads issued before this K-block is stored.
+    // both operands go global->smem with cp.async (up to `stages` K-blocks in flight, no registers); the column table
+    // entries of the NEXT K-block are loaded before the empty-wait of this one.
     LoaderA<A_MODE> pa;
     LoaderB<B_MODE> pb;
     pa.init(g, m0, tid);
     pb.init(g, n0, bn, tid);
     if (nkb > 0) {
-      pa.prologue(g, m0, kb_begin * TC_BK, tid);
-      pb.prologue(g, n0, kb_begin * TC_BK, tid);
+      pa.prologue(g, kb_begin * TC_BK, tid);
+      pb.prologue(g, kb_begin * TC_BK, tid);
     }
     int s = 0;
     uint32_t parity = 1;                                       // empty-barrier parity of the current round
@@ -444,19 +277,19 @@ gather_gemm_tc_kernel(const offk_gemm_t g, int bn, int stages, int kb_per_split,
         if (it < nkb) {
           const int k0 = (kb_begin + it) * TC_BK;
           const uint32_t a_base = smem_base + s * stage_bytes;
-          pa.pre_wait(g, m0, k0, tid, it + 1 < nkb);
-          pb.pre_wait(g, n0, k0, tid, it + 1 < nkb);
+          pa.pre_wait(g, k0, tid);
+          pb.pre_wait(g, k0, tid);
           mbar_wait(smem_u32(&sh->empty[s]), parity);
-          pa.post_wait(g, a_base, tid, hi_bytes);
-          pb.post_wait(g, a_base + TC_A_BYTES, n0, k0, tid, hi_bytes);
+          pa.post_wait(g, a_base);
+          pb.post_wait(g, a_base + TC_A_BYTES, tid);
           if (++s == stages) { s = 0; parity ^= 1u; }
         }
         cp_async_commit();                                     // one group per iteration (empty past the last K-block)
         if (it >= la) {
           if (la == 1) cp_async_wait_group<1>(); else if (la == 2) cp_async_wait_group<2>(); else cp_async_wait_group<3>();
           const uint32_t a_base = smem_base + s2 * stage_bytes;
-          if (LoaderA<A_MODE>::kAsync) pa.split_async(a_base, hi_bytes);
-          if (LoaderB<B_MODE>::kAsync) pb.split_async(a_base + TC_A_BYTES, tid, hi_bytes);
+          pa.split_async(a_base, hi_bytes);
+          pb.split_async(a_base + TC_A_BYTES, tid, hi_bytes);
           fence_proxy_async_smem();                            // generic-proxy st.shared -> visible to the tensor core
           mbar_arrive(smem_u32(&sh->full[s2]));
           if (++s2 == stages) s2 = 0;
@@ -467,12 +300,12 @@ gather_gemm_tc_kernel(const offk_gemm_t g, int bn, int stages, int kb_per_split,
       const int k0 = (kb_begin + i) * TC_BK;
       const uint32_t a_base = smem_base + s * stage_bytes;
       const uint32_t b_base = a_base + TC_A_BYTES;
-      pa.pre_wait(g, m0, k0, tid, i + 1 < nkb);
-      pb.pre_wait(g, n0, k0, tid, i + 1 < nkb);
+      pa.pre_wait(g, k0, tid);
+      pb.pre_wait(g, k0, tid);
       mbar_wait(smem_u32(&sh->empty[s]), parity);              // slot free (first round passes at once)
-      const bool stored = pa.post_wait(g, a_base, tid) | !LoaderB<B_MODE>::kAsync;
-      pb.post_wait(g, b_base, n0, k0, tid);
-      if (stored) fence_proxy_async_smem();   // generic-proxy st.shared -> visible to the tensor core (async proxy)
+      const bool stored = pa.post_wait(g, a_base);
+      pb.post_wait(g, b_base, tid);
+      if (stored) fence_proxy_async_smem();   // ones row: generic-proxy st.shared -> visible to the tensor core (async proxy)
       cp_async_mbar_arrive_noinc(smem_u32(&sh->full[s]));
       if (++s == stages) { s = 0; parity ^= 1u; }
     }
@@ -688,18 +521,14 @@ int launch_gemm_tc(const offk_gemm_t& g, cudaStream_t st, bool x3) {
   }
   dim3 grid((g.M + TC_BM - 1) / TC_BM, (g.N + bn - 1) / bn, (num_kb + kb_per - 1) / kb_per);
   if (grid.y > 65535 || grid.z > 65535) return fail(OFFK_E_LIMIT, "gather_gemm: grid too large");
-  // cp.async cannot apply ReLU-on-load: such operands (one small 1x1 conv) take the scalar register path
-  const int a_mode = (g.a_relu && g.a_mode >= OFFK_LOAD_VEC_K) ? OFFK_LOAD_SCALAR_ROW : g.a_mode;
 #define OFFK_TC_CASE(AM, BM)                                                                        \
-  if (a_mode == AM && g.b_mode == BM)                                                               \
+  if (g.a_mode == AM && g.b_mode == BM)                                                             \
     return x3 ? launch_tc_t<AM, BM, true>(g, bn, stages, kb_per, tmem_cols, grid, smem, st)         \
               : launch_tc_t<AM, BM, false>(g, bn, stages, kb_per, tmem_cols, grid, smem, st);
-  OFFK_TC_CASE(0, 0) OFFK_TC_CASE(0, 1) OFFK_TC_CASE(0, 2) OFFK_TC_CASE(0, 3)
-  OFFK_TC_CASE(1, 0) OFFK_TC_CASE(1, 1) OFFK_TC_CASE(1, 2) OFFK_TC_CASE(1, 3)
-  OFFK_TC_CASE(2, 0) OFFK_TC_CASE(2, 1) OFFK_TC_CASE(2, 2) OFFK_TC_CASE(2, 3)
-  OFFK_TC_CASE(3, 0) OFFK_TC_CASE(3, 1) OFFK_TC_CASE(3, 2) OFFK_TC_CASE(3, 3)
+  OFFK_TC_CASE(OFFK_LOAD_VEC_K, OFFK_LOAD_VEC_K) OFFK_TC_CASE(OFFK_LOAD_VEC_K, OFFK_LOAD_VEC_ROW)
+  OFFK_TC_CASE(OFFK_LOAD_VEC_ROW, OFFK_LOAD_VEC_K) OFFK_TC_CASE(OFFK_LOAD_VEC_ROW, OFFK_LOAD_VEC_ROW)
 #undef OFFK_TC_CASE
-  return fail(OFFK_E_BADARG, "gather_gemm: unsupported load modes %d/%d", a_mode, g.b_mode);
+  return fail(OFFK_E_BADARG, "gather_gemm: unsupported load modes %d/%d", g.a_mode, g.b_mode);
 }
 
 }  // namespace offk

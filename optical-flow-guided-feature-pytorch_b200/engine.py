@@ -29,7 +29,6 @@ _WGRAD_FIXED_KB = 10    # _wgrad_split: fixed cost of a weight-gradient CTA, in 
 _TF32_WANT_CTAS = _SM_TARGET    # _auto_tile_n: CTAs a TMA-fed GEMM without split-K aims for in the tf32 mode
 _X3_WANT_CTAS = 40      # ... and in the 3xTF32 mode
 _FINISH_MIN_TILES = 100     # output tiles from which a split-K conv finishes in-kernel (_conv_fwd)
-_TC_PRECS = (L.PREC_TF32, L.PREC_TF32X3)      # tcgen05 modes: 1 MMA per product / error-compensated 3xTF32
 
 
 def _ptr(t):
@@ -73,16 +72,18 @@ class Gemm:
     """One bound gather-GEMM launch (descriptor + device tables kept alive)."""
 
     def __init__(self, eng: "OFFEngine", spc: T.GemmSpec, key, *, a_src, b_src, out, bias=None, relu_pre_cols=0,
-                 a_relu=False, gate=None, gate_tabs=None, gate_col0=0, gate_first=False, addend=None,
+                 gate=None, gate_tabs=None, gate_col0=0, gate_first=False, addend=None,
                  add_tabs=None, relu_post=False, atomic=False, ones_out=None, split_k=1, tile_n=0, name="",
                  finish=False, aux=None, out_vec=None):
+        if spc.a_mode is None or spc.b_mode is None:
+            raise ValueError(f"{name}: an operand of this {spc.kind} GEMM has no 16-byte load form (tables.GemmSpec)")
         self.eng, self.name, self.spec = eng, name, spc
         tabs = eng._tables(key, spc)
         d = L.OffkGemm()
         d.M, d.N, d.K = spc.M, spc.N, spc.K
         d.a_src, d.a_row, d.a_col = a_src.data_ptr(), tabs["a_row"].data_ptr(), tabs["a_col"].data_ptr()
         d.a_h, d.a_w = (spc.a_h, spc.a_w) if spc.a_h else (T.NO_BOX, T.NO_BOX)
-        d.a_relu, d.a_ones_row, d.a_mode = int(a_relu), spc.a_ones_row, spc.a_mode
+        d.a_ones_row, d.a_mode = spc.a_ones_row, spc.a_mode
         d.b_src, d.b_row, d.b_col, d.b_mode = b_src.data_ptr(), tabs["b_row"].data_ptr(), tabs["b_col"].data_ptr(), spc.b_mode
         d.out, d.out_row, d.out_col = out.data_ptr(), tabs["out_row"].data_ptr(), tabs["out_col"].data_ptr()
         d.bias = bias.data_ptr() if bias is not None else None
@@ -132,22 +133,20 @@ class TGemm(Gemm):
     output tables as the gather-GEMM it stands in for."""
 
     @staticmethod
-    def eligible(geom: T.ConvGeom, prec, a_relu=False, x_layout="nhwc") -> bool:
+    def eligible(geom: T.ConvGeom, x_layout="nhwc") -> bool:
         if x_layout == "nchw":      # the taps, read in place as an MN-major operand: 1x1 conv over whole frames
-            return (prec in _TC_PRECS and not a_relu and T._is1x1(geom) and geom.cin % 32 == 0 and geom.x_coff == 0
-                    and geom.x_ctot == geom.cin and (geom.hin * geom.win) % 4 == 0)
-        return (prec in _TC_PRECS and not a_relu and geom.cin % 32 == 0 and geom.x_ctot % 4 == 0 and geom.x_coff % 4 == 0
-                and geom.kdim % 4 == 0)
+            return (T._is1x1(geom) and geom.cin % 32 == 0 and geom.x_coff == 0 and geom.x_ctot == geom.cin
+                    and (geom.hin * geom.win) % 4 == 0)
+        return geom.cin % 32 == 0 and geom.x_ctot % 4 == 0 and geom.x_coff % 4 == 0 and geom.kdim % 4 == 0
 
     @staticmethod
-    def wgrad_eligible(geom: T.ConvGeom, prec, a_relu=False, x_layout="nhwc") -> bool:
+    def wgrad_eligible(geom: T.ConvGeom, x_layout="nhwc") -> bool:
         """Weight gradient with both operands TMA-fed: A = im2col(x)^T (channels-last) or the NCHW tap, B = dY."""
         y_ok = geom.y_ctot % 4 == 0 and geom.y_coff % 4 == 0 and geom.cout % 4 == 0
         if x_layout == "nchw":
-            return (prec in _TC_PRECS and not a_relu and y_ok and T._is1x1(geom) and geom.x_coff == 0
-                    and geom.x_ctot == geom.cin and (geom.hin * geom.win) % 4 == 0)
-        return (prec in _TC_PRECS and not a_relu and y_ok and geom.cin % 32 == 0 and geom.x_ctot % 4 == 0
-                and geom.x_coff % 4 == 0)
+            return (y_ok and T._is1x1(geom) and geom.x_coff == 0 and geom.x_ctot == geom.cin
+                    and (geom.hin * geom.win) % 4 == 0)
+        return y_ok and geom.cin % 32 == 0 and geom.x_ctot % 4 == 0 and geom.x_coff % 4 == 0
 
     def __init__(self, eng, spc, key, geom: T.ConvGeom, x_layout="nhwc", wgrad=False, bk=0, **kw):
         super().__init__(eng, spc, key, **kw)
@@ -218,7 +217,7 @@ class OFFEngine:
              'flow' fixed diagonal Sobel, segment consensus over the L-1 pairs (Flow_OFF.py / RGB_OFF_v2.py)
     precision: 'fp32' = fp32-parity mode ON THE TENSOR CORES (OFFK_PREC_TF32X3: error-compensated 3xTF32 tcgen05 MMAs,
                fp32 accumulate; the reference's arithmetic is fp32, RGB_OFF.py:597), 'tf32' = one kind::tf32 MMA per
-               product (the fast mode, tolerance stated separately), 'fp32_simt' = CUDA-core FFMA cross-check (tests only)
+               product (the fast mode, tolerance stated separately)
     """
 
     def __init__(self, batch: int, length: int, variant: str = "rgb", device="cuda", precision: str = "tf32",
@@ -228,8 +227,7 @@ class OFFEngine:
         self.B, self.Lseg, self.variant = batch, length, variant
         self.N, self.P = batch * length, batch * (length - 1)
         self.device = torch.device(device)
-        self.prec = {"fp32": L.PREC_TF32X3, "tf32": L.PREC_TF32, "fp32_simt": L.PREC_FP32}[precision]
-        self.tc = self.prec in _TC_PRECS
+        self.prec = {"fp32": L.PREC_TF32X3, "tf32": L.PREC_TF32}[precision]
         self.precision = precision
         self.index_mode = {"reference_flat": L.INDEX_REFERENCE_FLAT, "aligned": L.INDEX_ALIGNED}[index_mode]
         self.consensus = (variant != "rgb") if consensus is None else bool(consensus)
@@ -390,15 +388,17 @@ class OFFEngine:
         self._cap_stream = None
 
     # ------------------------------------------------------------------ plan
-    def _conv_fwd(self, name, x, y, geom, w, b, *, relu=False, relu_cols=None, a_relu=False, addend=None,
+    def _conv_fwd(self, name, x, y, geom, w, b, *, relu=False, relu_cols=None, addend=None,
                   add_tabs=None, relu_post=False, x_layout="nhwc", no_split=False, aux=None):
-        """aux = (aux_out, aux_row table | None, aux_col0, aux_addend | None): second output max(v + aux_addend, 0) written by
-        the GEMM epilogue (offk.h); only honoured on the TMA-fed path -- the returned step has .aux_fused = True then."""
+        """One TMA-fed launch (TGemm); a geometry without a TMA-fed form is an error.
+        aux = (aux_out, aux_row table | None, aux_col0, aux_addend | None): second output max(v + aux_addend, 0) written by
+        the GEMM epilogue (offk.h); only honoured with the float4 epilogue (out_vec) -- the returned step has
+        .aux_fused = True then."""
         spc = T.conv_fwd_spec(geom, x_layout, "nhwc")
         m_tiles, kb = math.ceil(spc.M / 128), math.ceil(spc.K / 32)
         n_tiles = max(1, math.ceil(spc.N / 256))
         split = 1
-        if self.tc and addend is None and m_tiles * n_tiles < 200 and kb >= 32:
+        if addend is None and m_tiles * n_tiles < 200 and kb >= 32:
             # split-K factor: minimise rounds x K-blocks per CTA, rounds = ceil(CTAs / resident CTA slots) (two CTAs per SM in
             # the tf32 mode, one in the 3xTF32 mode whose stages are twice as large); ties go to the smaller factor.
             # 147 tiles: 2 splits = 294 CTAs = one round (3 splits were 1.49 rounds at 31 % tensor-pipe activity).
@@ -407,11 +407,12 @@ class OFFEngine:
             split = min(range(1, max(1, kb // 8) + 1),
                         key=lambda s_: (math.ceil(tiles * s_ / slots) * math.ceil(kb / s_) * (1 if tiles * s_ >= 0.9 * _SM_TARGET else 4), s_))
         cols = (geom.cout if relu else 0) if relu_cols is None else relu_cols
-        tma = TGemm.eligible(geom, self.prec, a_relu, x_layout)
-        mk = (lambda *a, **k: TGemm(*a, geom=geom, x_layout=x_layout, **k)) if tma else Gemm
-        if (tma and x_layout == "nchw") or no_split:
+        if not TGemm.eligible(geom, x_layout):
+            raise ValueError(f"{name}: this conv geometry has no TMA-fed form (TGemm.eligible)")
+        mk = lambda *a, **k: TGemm(*a, geom=geom, x_layout=x_layout, **k)
+        if x_layout == "nchw" or no_split:
             split = 1                     # per-frame M tiles already fill the machine (N * ceil(hw/128) CTAs)
-        fuse = tma and spc.out_vec
+        fuse = spc.out_vec
         # in-kernel finishing pays when there are enough output tiles for the finishing CTAs to keep the machine busy
         # (motion_conv_trans_28: 147 tiles, same time as the bare split-K GEMM, bias_act and ReLU copy for free); with the
         # 37-tile 7x7 layers the fences + a finishing pass by 37 CTAs cost 9-27 us more than a separate full-grid bias_act
@@ -420,7 +421,7 @@ class OFFEngine:
         if split > 1 and fin_ok:
             # split-K partial tiles are added into the zeroed output; the last CTA of each tile applies bias / ReLU (and
             # writes the second output) in place: no separate bias_act pass
-            g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, bias=b, relu_pre_cols=cols, a_relu=a_relu,
+            g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, bias=b, relu_pre_cols=cols,
                    split_k=split, name=name, finish=True, aux=aux)
 
             def run(stream, g=g, y=y):
@@ -433,7 +434,7 @@ class OFFEngine:
             run.reads, run.writes, run.lane = g.reads, g.writes, 0
             return run
         if split > 1:
-            g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, a_relu=a_relu, split_k=split, name=name)
+            g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, split_k=split, name=name)
             hw = geom.hout * geom.wout
 
             def run(stream, g=g, y=y, b=b, geom=geom, hw=hw, cols=cols):
@@ -451,14 +452,14 @@ class OFFEngine:
             run.reads, run.writes, run.lane = g.reads, g.writes, 0
             return run
         # nchw TMA: one N tile (re-reading the tap per N tile would multiply the HBM traffic of an HBM-bound GEMM)
-        tn = (spc.N + 15) // 16 * 16 if (tma and x_layout == "nchw" and spc.N <= 256) else 0
-        g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, bias=b, relu_pre_cols=cols, a_relu=a_relu,
+        tn = (spc.N + 15) // 16 * 16 if (x_layout == "nchw" and spc.N <= 256) else 0
+        g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, bias=b, relu_pre_cols=cols,
                addend=addend, add_tabs=add_tabs, relu_post=relu_post, tile_n=tn, name=name, aux=aux if fuse else None)
         g.aux_fused = bool(fuse and aux is not None)
         self.flops_fwd += g.flops
         return g
 
-    def _conv_wgrad(self, name, x, dy, geom, dw, db, *, a_relu=False, x_layout="nhwc", tap_copy=False):
+    def _conv_wgrad(self, name, x, dy, geom, dw, db, *, x_layout="nhwc", tap_copy=False):
         """tap_copy: x is the channels-last copy of a unit's tap (the 7x7 levels), which is TMA-fed like the NCHW tap."""
         # dW is accumulated in the k order of the implicit GEMM (OHWI: consecutive accumulator rows = consecutive
         # addresses, so the split-K reductions coalesce) and un-permuted once at the end; writing OIHW directly
@@ -466,7 +467,7 @@ class OFFEngine:
         spc = T.conv_wgrad_spec(geom, x_layout, "nhwc")
         x3 = self.prec == L.PREC_TF32X3
         # the units' weight gradients are TMA-fed from the tap (measured 81 -> 54 us at level 3a)
-        tma = TGemm.wgrad_eligible(geom, self.prec, a_relu, x_layout)
+        tma = TGemm.wgrad_eligible(geom, x_layout)
         bk = 0
         if tma and x_layout == "nhwc" and not tap_copy:
             # stage convs: TMA im2col with DEEP K-blocks (bk output pixels per stage: 64 / 128 instead of 32 -> fewer, larger
@@ -491,8 +492,8 @@ class OFFEngine:
         split = _wgrad_split(m_tiles * n_tiles, kb, _SM_TARGET * (1 if x3 else 2), bk or 32)
         mk = (lambda *a, **k: TGemm(*a, geom=geom, x_layout=x_layout, wgrad=True, bk=bk, **k)) if tma else Gemm
         # dW[n][m]: consecutive accumulator rows are consecutive addresses -> transposed float4 adds (offk.h: out_vec = 2)
-        rows_vec = self.tc and dw.data_ptr() % 16 == 0 and geom.kdim % 4 == 0
-        g = mk(self, spc, ("wgrad", x_layout, _gkey(geom)), a_src=x, b_src=dy, out=dw, ones_out=db, a_relu=a_relu,
+        rows_vec = dw.data_ptr() % 16 == 0 and geom.kdim % 4 == 0
+        g = mk(self, spc, ("wgrad", x_layout, _gkey(geom)), a_src=x, b_src=dy, out=dw, ones_out=db,
                atomic=True, split_k=split, name=name + ".wgrad", out_vec=2 if rows_vec else None)
         self.flops_bwd += g.flops
         return g
@@ -509,27 +510,31 @@ class OFFEngine:
                 add_tabs = (t["out_row"], t["out_col"])
             kw_ = dict(a_src=dy, b_src=w, out=dx, gate=gate, gate_col0=gate_col0, gate_first=gate_first, addend=addend,
                        add_tabs=add_tabs, name=f"{name}.dgrad{i}")
-            # dX of a stride-1 conv = a forward conv over dY with flipped taps and pad' = k-1-pad: TMA-fed
-            gd = T.ConvGeom(geom.n_img, geom.cout, geom.hout, geom.wout, geom.cin, geom.kh, geom.kw, 1,
-                            geom.kh - 1 - geom.pad, geom.y_ctot, geom.y_coff, geom.x_ctot, geom.x_coff) if geom.stride == 1 else None
-            ex = spc.extra
-            if (x_layout == "nhwc" and gd is not None and name in self.wd and geom.kh == geom.kw
-                    and TGemm.eligible(gd, self.prec) and (gd.hout, gd.wout) == (geom.hin, geom.win)):
+            key, ex = ("dgrad", x_layout, _gkey(geom), i), spc.extra
+            if x_layout == "nchw":
+                # the units' tap gradients: dX is NCHW, written through the out tables by the gather-fed kernel
+                g = Gemm(self, spc, key, **kw_)
+            elif geom.stride == 1:
+                # dX of a stride-1 conv = a forward conv over dY with flipped taps and pad' = k-1-pad: TMA-fed
+                gd = T.ConvGeom(geom.n_img, geom.cout, geom.hout, geom.wout, geom.cin, geom.kh, geom.kw, 1,
+                                geom.kh - 1 - geom.pad, geom.y_ctot, geom.y_coff, geom.x_ctot, geom.x_coff)
+                if not (name in self.wd and geom.kh == geom.kw and TGemm.eligible(gd)
+                        and (gd.hout, gd.wout) == (geom.hin, geom.win)):
+                    raise ValueError(f"{name}.dgrad{i}: this data gradient has no TMA-fed form")
                 kw_["b_src"] = self.wd[name]
-                g = TGemm(self, spc, ("dgrad", x_layout, _gkey(geom), i), geom=gd, **kw_)
-            elif (x_layout == "nhwc" and geom.stride > 1
-                  and (name, ex["a"], ex["b"]) in self.wd and self.tc and geom.cout % 32 == 0
-                  and geom.y_ctot % 4 == 0 and geom.y_coff % 4 == 0 and ex["pad_h"] >= 0 and ex["pad_w"] >= 0):
+                g = TGemm(self, spc, key, geom=gd, **kw_)
+            else:
                 # one stride-parity class = a stride-1 correlation over dY with the class's R x Q taps (free geometry)
+                if not ((name, ex["a"], ex["b"]) in self.wd and geom.cout % 32 == 0 and geom.y_ctot % 4 == 0
+                        and geom.y_coff % 4 == 0 and ex["pad_h"] >= 0 and ex["pad_w"] >= 0):
+                    raise ValueError(f"{name}.dgrad{i}: this data gradient has no TMA-fed form")
                 R, Q = len(ex["rs"]), len(ex["qs"])
                 fg = _FreeGeom(n_img=geom.n_img, cin=geom.cout, hin=geom.hout, win=geom.wout, cout=geom.cin, kh=R, kw=Q,
                                stride=1, pad=ex["pad_h"], pad_w=ex["pad_w"], x_ctot=geom.y_ctot, x_coff=geom.y_coff,
                                hout=ex["hc"], wout=ex["wc"], kdim=R * Q * geom.cout)
                 kw_["b_src"] = self.wd[(name, ex["a"], ex["b"])]
                 kw_["tile_n"] = _pick_tile_n(spc.M, spc.N, _SM_TARGET * (1 if self.prec == L.PREC_TF32X3 else 2))
-                g = TGemm(self, spc, ("dgrad", x_layout, _gkey(geom), i), geom=fg, **kw_)
-            else:
-                g = Gemm(self, spc, ("dgrad", x_layout, _gkey(geom), i), **kw_)
+                g = TGemm(self, spc, key, geom=fg, **kw_)
             self.flops_bwd += g.flops
             out.append(g)
         return out
@@ -560,7 +565,7 @@ class OFFEngine:
             # K1: gen (ReLU) and down (linear) 1x1 convs as ONE GEMM with 160 output channels
             # 7x7 taps: a 196-byte channel stride is not a legal TMA stride -> one channels-last copy of the tap per
             # step feeds both the forward GEMM (dense tensor map) and the weight gradient (im2col_t), all TMA-fed
-            via_copy = self.tc and (s * s) % 4 != 0 and cin % 32 == 0
+            via_copy = (s * s) % 4 != 0 and cin % 32 == 0
             if via_copy:
                 tapT = self._buf("tapT_" + tag, N, s, s, cin)
 
@@ -649,11 +654,11 @@ class OFFEngine:
         def dW(n): return self.dwp[n] if n in self.dwp else gr[n + ".weight"]
         def dB(n): return gr[n + ".bias"]
 
-        def layer(name, x, y, s_in, *, relu=False, a_relu=False, addend=None, relu_post=False,
+        def layer(name, x, y, s_in, *, relu=False, addend=None, relu_post=False,
                   x_ctot=0, x_coff=0, y_ctot=0, y_coff=0, lane=0, aux=None):
             """forward conv; returns geom for the gradient wiring."""
             geom = geom_of(name, P, s_in, x_ctot, x_coff, y_ctot, y_coff)
-            fwd.append(_on(self._conv_fwd(name, x, y, geom, W(name), Bv(name), relu=relu, a_relu=a_relu, addend=addend,
+            fwd.append(_on(self._conv_fwd(name, x, y, geom, W(name), Bv(name), relu=relu, addend=addend,
                                           relu_post=relu_post, aux=aux), lane))
             return geom
 
@@ -728,8 +733,8 @@ class OFFEngine:
         # ds7 = avgpool'(dropout'(Linear'(d_out7))) in one pass
         bs.extend(self._head_bwd("7", self.d_out7, d("s7"), 1024, 1024, 0, "fc_action_motion", act=None, accumulate=False))
 
-        def back(name, x, dy, geom, *, a_relu=False):
-            bs.append(_on(self._conv_wgrad(name, x, dy, geom, dW(name), dB(name), a_relu=a_relu), 1))   # wgrad lane
+        def back(name, x, dy, geom):
+            bs.append(_on(self._conv_wgrad(name, x, dy, geom, dW(name), dB(name)), 1))   # wgrad lane
 
         def dgrad(name, dy, dx, geom, lane=0, **kw):
             bs.extend(_on(g, lane) for g in self._conv_dgrad(name, dy, W(name), dx, geom, **kw))

@@ -116,7 +116,7 @@ class OFFSubNetwork(nn.Module):
     logits ``[batch*(length-1), 101]``; variant='flow' (also RGB_OFF_v2): fixed diagonal Sobel and segment consensus
     ``[batch, 101]``.  Dropout follows ``self.training`` (p = 0.8, RGB_OFF.py:356); pass ``masks`` to inject keep-masks.
     ``precision``: 'fp32' = fp32-parity arithmetic on the tensor cores (3xTF32), 'tf32' = single-MMA tf32 (the default here,
-    the fast mode), 'fp32_simt' = CUDA-core cross-check.  ``use_graphs``: replay each pass as one captured CUDA graph.
+    the fast mode).  ``use_graphs``: replay each pass as one captured CUDA graph.
     """
 
     def __init__(self, batch: int, length: int, variant: str = "rgb", precision: str = "tf32",

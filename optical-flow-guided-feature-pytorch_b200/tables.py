@@ -59,7 +59,9 @@ class ConvGeom:
 
 @dataclass
 class GemmSpec:
-    """Host-side description of one gather-GEMM (numpy tables; pointers are bound later)."""
+    """Host-side description of one gather-GEMM (numpy tables; pointers are bound later).  a_mode / b_mode: the
+    16-byte load form the operand's layout allows (LOAD_VEC_K / LOAD_VEC_ROW), or None when it has none -- such a spec
+    can be emulated on the CPU but not launched."""
     M: int
     N: int
     K: int
@@ -72,14 +74,14 @@ class GemmSpec:
     a_h: int = 0
     a_w: int = 0
     a_ones_row: int = -1
-    a_mode: int = 0
-    b_mode: int = 0
+    a_mode: Optional[int] = None
+    b_mode: Optional[int] = None
     out_vec: int = 0
     kind: str = ""
     extra: dict = field(default_factory=dict)
 
 
-LOAD_SCALAR_ROW, LOAD_SCALAR_K, LOAD_VEC_K, LOAD_VEC_ROW = 0, 1, 2, 3
+LOAD_VEC_K, LOAD_VEC_ROW = 2, 3          # offk.h OFFK_LOAD_*
 
 
 def _idx(off, y, x):
@@ -134,9 +136,9 @@ def conv_fwd_spec(g: ConvGeom, x_layout: str = "nchw", y_layout: str = "nchw") -
     hw, hwo = g.hin * g.win, g.hout * g.wout
     box = not (g.kh == 1 and g.kw == 1 and g.pad == 0)
     if x_layout == "nhwc":
-        a_mode = LOAD_VEC_K if (g.cin % 4 == 0 and g.x_ctot % 4 == 0 and g.x_coff % 4 == 0) else LOAD_SCALAR_ROW
+        a_mode = LOAD_VEC_K if (g.cin % 4 == 0 and g.x_ctot % 4 == 0 and g.x_coff % 4 == 0) else None
     else:
-        a_mode = LOAD_VEC_ROW if (_is1x1(g) and hw % 4 == 0) else LOAD_SCALAR_ROW
+        a_mode = LOAD_VEC_ROW if (_is1x1(g) and hw % 4 == 0) else None
     if y_layout == "nhwc":
         out_col = np.arange(g.cout)
         out_vec = int(g.cout % 4 == 0 and g.y_ctot % 4 == 0 and g.y_coff % 4 == 0)
@@ -146,7 +148,7 @@ def conv_fwd_spec(g: ConvGeom, x_layout: str = "nchw", y_layout: str = "nchw") -
         M=g.n_img * hwo, N=g.cout, K=K, a_row=a_row, a_col=_filter_tables(g, x_layout),
         b_row=_i32(np.arange(g.cout) * K), b_col=_i32(np.arange(K)), out_row=y_off, out_col=_i32(out_col),
         a_h=g.hin if box else 0, a_w=g.win if box else 0, a_mode=a_mode,
-        b_mode=LOAD_VEC_K if K % 4 == 0 else LOAD_SCALAR_K, out_vec=out_vec, kind="fwd")
+        b_mode=LOAD_VEC_K if K % 4 == 0 else None, out_vec=out_vec, kind="fwd")
 
 
 def conv_wgrad_spec(g: ConvGeom, x_layout: str = "nchw", y_layout: str = "nchw", dw_layout: str = None) -> GemmSpec:
@@ -162,15 +164,15 @@ def conv_wgrad_spec(g: ConvGeom, x_layout: str = "nchw", y_layout: str = "nchw",
     img = np.repeat(np.arange(g.n_img), hwo)
     p = np.tile(np.arange(hwo), g.n_img)
     if x_layout == "nhwc":
-        a_mode = LOAD_VEC_ROW if (g.cin % 4 == 0 and g.x_ctot % 4 == 0 and g.x_coff % 4 == 0) else LOAD_SCALAR_ROW
+        a_mode = LOAD_VEC_ROW if (g.cin % 4 == 0 and g.x_ctot % 4 == 0 and g.x_coff % 4 == 0) else None
     else:
-        a_mode = LOAD_VEC_K if (_is1x1(g) and hw % 4 == 0) else LOAD_SCALAR_K
+        a_mode = LOAD_VEC_K if (_is1x1(g) and hw % 4 == 0) else None
     if y_layout == "nhwc":
         b_row, b_col = np.arange(g.cout) + g.y_coff, (img * hwo + p) * g.y_ctot
-        b_mode = LOAD_VEC_ROW if (g.cout % 4 == 0 and g.y_ctot % 4 == 0 and g.y_coff % 4 == 0) else LOAD_SCALAR_ROW
+        b_mode = LOAD_VEC_ROW if (g.cout % 4 == 0 and g.y_ctot % 4 == 0 and g.y_coff % 4 == 0) else None
     else:
         b_row, b_col = (np.arange(g.cout) + g.y_coff) * hwo, img * g.y_ctot * hwo + p
-        b_mode = LOAD_VEC_K if hwo % 4 == 0 else LOAD_SCALAR_K
+        b_mode = LOAD_VEC_K if hwo % 4 == 0 else None
     out_row = np.arange(K_w + 1)
     if dw_layout == "oihw" and x_layout == "nhwc":
         r, q, c = np.meshgrid(np.arange(g.kh), np.arange(g.kw), np.arange(g.cin), indexing="ij")
@@ -206,21 +208,21 @@ def conv_dgrad_specs(g: ConvGeom, x_layout: str = "nchw", y_layout: str = "nchw"
                 a_row = _idx((img * g.y_ctot + g.y_coff) * hwo + oy * g.wout + ox, oy, ox)
                 co, rr, qq = np.meshgrid(np.arange(g.cout), np.arange(len(rs)), np.arange(len(qs)), indexing="ij")
                 a_col = _idx(co * hwo - rr * g.wout - qq, -rr, -qq)
-                a_mode = LOAD_SCALAR_ROW
+                a_mode = None
             else:
                 a_row = _idx(((img * g.hout + oy) * g.wout + ox) * g.y_ctot + g.y_coff, oy, ox)
                 rr, qq, co = np.meshgrid(np.arange(len(rs)), np.arange(len(qs)), np.arange(g.cout), indexing="ij")
                 a_col = _idx((-rr * g.wout - qq) * g.y_ctot + co, -rr, -qq)
-                a_mode = LOAD_VEC_K if (g.cout % 4 == 0 and g.y_ctot % 4 == 0 and g.y_coff % 4 == 0) else LOAD_SCALAR_ROW
+                a_mode = LOAD_VEC_K if (g.cout % 4 == 0 and g.y_ctot % 4 == 0 and g.y_coff % 4 == 0) else None
             r_full, q_full = r0 + s * rr, q0 + s * qq
             if w_layout == "nchw":
                 b_row = np.arange(g.cin) * (g.kh * g.kw)
                 b_col = co * kw_tot + r_full * g.kw + q_full
-                b_mode = LOAD_SCALAR_ROW
+                b_mode = None
             else:
                 b_row = np.arange(g.cin)
                 b_col = co * kw_tot + (r_full * g.kw + q_full) * g.cin
-                b_mode = LOAD_VEC_ROW if g.cin % 4 == 0 else LOAD_SCALAR_ROW
+                b_mode = LOAD_VEC_ROW if g.cin % 4 == 0 else None
             iy, ix = s * ih + a, s * iw + b
             if x_layout == "nchw":
                 out_row = (img * g.x_ctot + g.x_coff) * hwi + iy * g.win + ix
@@ -332,7 +334,7 @@ def padded_tables(spec: GemmSpec):
     return {k: np.ascontiguousarray(v).view(np.int32).reshape(-1) for k, v in tabs.items()}
 
 
-def emulate(spec: GemmSpec, a_src: np.ndarray, b_src: np.ndarray, a_relu: bool = False) -> np.ndarray:
+def emulate(spec: GemmSpec, a_src: np.ndarray, b_src: np.ndarray) -> np.ndarray:
     """Dense D[M,N] of a spec, evaluated with numpy (float64).  CPU-side check of the tables only."""
     a_src = a_src.reshape(-1).astype(np.float64)
     b_src = b_src.reshape(-1).astype(np.float64)
@@ -350,8 +352,6 @@ def emulate(spec: GemmSpec, a_src: np.ndarray, b_src: np.ndarray, a_relu: bool =
         else:
             ok = np.ones(off.shape, bool)
         A = np.where(ok, a_src[np.where(ok, off, 0)], 0.0)
-        if a_relu:
-            A = np.maximum(A, 0.0)
         if spec.a_ones_row >= 0 and m0 <= spec.a_ones_row < m0 + step:
             A[spec.a_ones_row - m0] = 1.0
         D[m0:m0 + step] = A @ B.T

@@ -1,7 +1,7 @@
 """GPU: parity of the sm_100a path with the CPU oracle, through the C ABI (liboffk.so).
 
 Tolerances (stated per mode, as BASELINE.json's north_star asks):
-  fp32 mode (CUDA-core FFMA, fp32 accumulate): <= 2e-5 max-abs relative to the tensor's max, per level / head;
+  fp32 mode (3xTF32 tcgen05, fp32 accumulate): <= 2e-5 max-abs relative to the tensor's max, per level / head;
   tf32 mode (tcgen05 kind::tf32, fp32 accumulate): <= 5e-3 on the stage-fusion tensors, <= 1e-2 on the logits;
   gradients are compared in relative L2 norm (a single ReLU whose pre-activation sits within round-off of 0 may flip
   between fp32 and the fp64 oracle, which moves individual entries but not the norm): fp32 <= 2e-3, tf32 <= 0.2.
@@ -58,20 +58,21 @@ def _run_spec(spc, a_src, b_src, out_shape, prec, dev, bias=None, ones=None, spl
 
 GEMM_CASES = [
     # n, cin, h, w, cout, k, s, p, x_ctot, x_coff, y_ctot, y_coff, x_layout, y_layout
-    (3, 8, 7, 7, 8, 1, 1, 0, 8, 0, 8, 0, "nchw", "nhwc"),          # unit conv, 7x7 taps (scalar NCHW loader)
+    (3, 8, 7, 7, 8, 1, 1, 0, 8, 0, 8, 0, "nchw", "nhwc"),          # unit conv, 7x7 taps: data gradient only
     (5, 64, 14, 14, 160, 1, 1, 0, 64, 0, 160, 0, "nchw", "nhwc"),  # unit conv, vectorised transposing loader
     (4, 64, 14, 14, 64, 3, 1, 1, 64, 0, 64, 0, "nhwc", "nhwc"),
     (2, 32, 28, 28, 64, 7, 2, 3, 32, 0, 64, 0, "nhwc", "nhwc"),  # motion_conv_trans_28 geometry
     (2, 24, 14, 14, 128, 5, 2, 2, 40, 8, 160, 32, "nhwc", "nhwc"),  # 5x5 s2 on channel slices
     (3, 128, 7, 7, 512, 3, 1, 1, 128, 0, 512, 0, "nhwc", "nhwc"),  # N > 256: two N tiles
-    (8, 1024, 1, 1, 101, 1, 1, 0, 1024, 0, 101, 0, "nhwc", "nhwc"),  # FC head, N not a multiple of 4
-    (2, 6, 9, 8, 4, 3, 1, 1, 10, 3, 7, 2, "nchw", "nchw"),       # ragged everything (scalar paths)
+    (8, 1024, 1, 1, 101, 1, 1, 0, 1024, 0, 101, 0, "nhwc", "nhwc"),  # FC head, N not a multiple of 4: forward only
 ]
 
 
-@pytest.mark.parametrize("prec,tol", [(0, 5e-6), (1, 3e-3), (2, 1e-5)], ids=["fp32simt", "tf32", "tf32x3"])
+@pytest.mark.parametrize("prec,tol", [(1, 3e-3), (2, 1e-5)], ids=["tf32", "tf32x3"])
 @pytest.mark.parametrize("case", GEMM_CASES, ids=[f"{c[1]}x{c[2]}k{c[5]}s{c[6]}{c[12]}" for c in GEMM_CASES])
 def test_gather_gemm_conv_parity(dev, case, prec, tol):
+    """Forward, weight gradient and data gradient of a conv through offk_gather_gemm against autograd of conv2d; a GEMM
+    whose operand layout has no 16-byte load form (tables.GemmSpec mode None) cannot be launched and is skipped."""
     from off_b200 import tables as T
     n, cin, h, w, cout, k, s, p, xct, xco, yct, yco, xl, yl = case
     g = T.ConvGeom(n, cin, h, w, cout, k, k, s, p, xct, xco, yct, yco)
@@ -88,21 +89,34 @@ def test_gather_gemm_conv_parity(dev, case, prec, tol):
     back = lambda a, lay: a.permute(0, 3, 1, 2) if lay == "nhwc" else a
     xb, dyb = to(x, xl), to(dy, yl)
     wl = wt.permute(0, 2, 3, 1).contiguous() if xl == "nhwc" else wt
-    out = back(_run_spec(T.conv_fwd_spec(g, xl, yl), xb, wl, tuple(dyb.shape), prec, dev, bias=b), yl)
-    assert _rel(out[:, yco:yco + cout], y.detach().cpu()) < tol
-    other = torch.cat([out[:, :yco], out[:, yco + cout:]], 1)
-    assert other.abs().max().item() == 0 if other.numel() else True           # channel slice only
-    out2 = back(_run_spec(T.conv_fwd_spec(g, xl, yl), xb, wl, tuple(dyb.shape), prec, dev, split_k=3), yl)
-    assert _rel(out2[:, yco:yco + cout], (y - b.double().view(1, -1, 1, 1)).detach().cpu()) < tol
-    db = torch.zeros(cout, device=dev)
-    dw = _run_spec(T.conv_wgrad_spec(g, xl, yl), xb, dyb, tuple(wl.shape), prec, dev, ones=db, split_k=4, atomic=True)
-    dwc = dw.permute(0, 3, 1, 2) if xl == "nhwc" else dw
-    assert _rel(dwc, wd.grad.cpu()) < tol
-    assert _rel(db, dy[:, yco:yco + cout].double().sum((0, 2, 3)).cpu()) < tol
-    dx = torch.zeros_like(xb)
-    for spc in T.conv_dgrad_specs(g, xl, yl, xl):
-        dx += _run_spec(spc, dyb, wl, tuple(xb.shape), prec, dev)
-    assert _rel(back(dx, xl)[:, xco:xco + cin], xs.grad.cpu()) < tol
+    launchable = lambda spc: spc.a_mode is not None and spc.b_mode is not None
+    ran = 0
+    fwd = T.conv_fwd_spec(g, xl, yl)
+    if launchable(fwd):
+        out = back(_run_spec(fwd, xb, wl, tuple(dyb.shape), prec, dev, bias=b), yl)
+        assert _rel(out[:, yco:yco + cout], y.detach().cpu()) < tol
+        other = torch.cat([out[:, :yco], out[:, yco + cout:]], 1)
+        assert other.abs().max().item() == 0 if other.numel() else True           # channel slice only
+        out2 = back(_run_spec(fwd, xb, wl, tuple(dyb.shape), prec, dev, split_k=3), yl)
+        assert _rel(out2[:, yco:yco + cout], (y - b.double().view(1, -1, 1, 1)).detach().cpu()) < tol
+        ran += 1
+    wgrad = T.conv_wgrad_spec(g, xl, yl)
+    if launchable(wgrad):
+        db = torch.zeros(cout, device=dev)
+        dw = _run_spec(wgrad, xb, dyb, tuple(wl.shape), prec, dev, ones=db, split_k=4, atomic=True)
+        dwc = dw.permute(0, 3, 1, 2) if xl == "nhwc" else dw
+        assert _rel(dwc, wd.grad.cpu()) < tol
+        assert _rel(db, dy[:, yco:yco + cout].double().sum((0, 2, 3)).cpu()) < tol
+        ran += 1
+    # a 1x1 weight is the same memory in OIHW and OHWI: the NCHW cases take the weight layout of the engine's tap gradients
+    dgrads = T.conv_dgrad_specs(g, xl, yl, "nhwc" if k == 1 else xl)
+    if all(launchable(spc) for spc in dgrads):
+        dx = torch.zeros_like(xb)
+        for spc in dgrads:
+            dx += _run_spec(spc, dyb, wl, tuple(xb.shape), prec, dev)
+        assert _rel(back(dx, xl)[:, xco:xco + cin], xs.grad.cpu()) < tol
+        ran += 1
+    assert ran > 0
 
 
 TMA_CASES = [
@@ -549,8 +563,8 @@ import functools
 # flipped gate moves a weight gradient by O(1/sqrt(#elements)).  The reference's own fp32 CPU arithmetic shows the same
 # against fp64 (B=1, L=3: worst relative L2 1.4e-2; 1.8e-6 once the gates are matched -- measured with oracle/off_oracle.py),
 # so the exact-oracle gate only bounds the flip rate and the arithmetic is pinned by the gate-matched run.
-# Measured on the B200 (profiles/parity_r02b.txt): fp32 mode forward 4e-7 .. 2.5e-6 (the CUDA-core FFMA twin: 4e-7 .. 9e-7),
-# gate-matched gradients 3.5e-6 .. 5.1e-6 (FFMA twin 1.7e-6), exact-oracle gradients 3.5e-6 (no flip) .. 3.7e-3 (B = 48).
+# Measured on the B200 (profiles/parity_r02b.txt): fp32 mode forward 4e-7 .. 2.5e-6, gate-matched gradients 3.5e-6 .. 5.1e-6,
+# exact-oracle gradients 3.5e-6 (no flip) .. 3.7e-3 (B = 48).
 TOL_FP32 = (5e-6, 1e-5, 5e-2)
 TOL_FP32_GATED = (5e-6, 1e-5, 2e-5)
 
@@ -622,18 +636,12 @@ def _engine_vs_oracle(dev, precision, variant, B, Lg, train, tol_fuse, tol_logit
 
 @pytest.mark.parametrize("variant,B,Lg,train", [("rgb", 2, 3, False), ("flow", 2, 3, False), ("rgb", 2, 2, True),
                                                 ("flow", 1, 4, False), ("rgb", 1, 3, False),
-                                                ("rgb", 2, 7, False), ("flow", 1, 7, True)])   # config 4 geometry: 7 segments
+                                                ("rgb", 2, 7, False), ("flow", 1, 7, True),   # config 4 geometry: 7 segments
+                                                ("flow", 1, 4, True)])
 def test_engine_fp32_mode_matches_oracle(dev, variant, B, Lg, train):
     """precision='fp32' = the fp32-parity mode on the tensor cores (3xTF32 tcgen05, OFFK_PREC_TF32X3)."""
     _engine_vs_oracle(dev, "fp32", variant, B, Lg, train, *TOL_FP32)
     _engine_vs_oracle(dev, "fp32", variant, B, Lg, train, *TOL_FP32_GATED, gate_matched=True)
-
-
-@pytest.mark.parametrize("variant,B,Lg,train", [("rgb", 2, 3, False), ("flow", 1, 4, True)])
-def test_engine_fp32_simt_cross_check(dev, variant, B, Lg, train):
-    """The CUDA-core FFMA twin of every contraction (OFFK_PREC_FP32): an independent check of the index tables."""
-    _engine_vs_oracle(dev, "fp32_simt", variant, B, Lg, train, *TOL_FP32)
-    _engine_vs_oracle(dev, "fp32_simt", variant, B, Lg, train, *TOL_FP32_GATED, gate_matched=True)
 
 
 TF32_CASES = [("rgb", 2, 3, False), ("flow", 2, 3, False), ("rgb", 2, 2, True), ("rgb", 2, 7, True)]

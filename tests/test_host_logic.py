@@ -105,7 +105,7 @@ def test_engine_plan_builds_without_a_gpu():
     # forward FLOPs follow the survey's scaling law 0.28897*N + 1.29305*P GFLOP (+ the down rows of the N-P extra frames)
     gf = 0.28897 * eng.N + 1.29305 * eng.P + 0.07235 * (eng.N - eng.P)
     assert abs(eng.flops_fwd / 1e9 - gf) / gf < 0.01
-    flow = E.OFFEngine(1, 4, "flow", "cpu", "fp32_simt", tap_grads=True)
+    flow = E.OFFEngine(1, 4, "flow", "cpu", "tf32", tap_grads=True)
     assert flow.consensus and "motion_spatial_grad_3a.weight" not in flow.params
     # tf32 plan: the 7x7 taps go through a channels-last copy, every stride-2 data-gradient class has its own weight
     # block, the forward stencil is two launches and all KxK weight gradients are un-permuted by one
@@ -115,7 +115,13 @@ def test_engine_plan_builds_without_a_gpu():
     assert names.count("unpermute_kxk_weight_grads") == 1 and "stencil_bwd" in names
     for conv in ("motion_conv_trans_28", "motion_conv_trans_14"):
         assert all((conv, a, b) in eng.wd for a in (0, 1) for b in (0, 1))
-    assert "tapT_5a" not in flow.launch_names()          # the CUDA-core cross-check mode reads the NCHW taps through the gather kernel
+    # tap gradients: every unit's data gradient into its NCHW tap is launched; the 7x7 units read a channels-last tap copy
+    flow_names = flow.launch_names()
+    for tag in S.LEVELS:
+        assert any(n.startswith(f"unit_{tag}.dgrad") for n in flow_names), tag
+    assert "tapT_5a" in flow_names and "tapT_5b" in flow_names
+    with pytest.raises(KeyError):
+        E.OFFEngine(1, 4, "flow", "cpu", "fp32_simt")
     # precision='fp32' is the 3xTF32 tensor-core mode: the same TMA-fed plan as 'tf32', launch for launch, plus the two
     # per-step weight-residual passes (the GEMMs then receive both weight tiles by TMA)
     x3 = E.OFFEngine(2, 3, "rgb", "cpu", "fp32")

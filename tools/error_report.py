@@ -6,7 +6,7 @@ error reported per level; tf32 GEMM tolerance stated separately").
 For every OFF unit (level 3a..5b) the 160-channel slice it writes into its stage-fusion buffer -- 32 spatial-gradient
 channels (RGB_OFF.py:611 / Flow_OFF.py:622) and 128 temporal-difference channels (:599-604) -- then the three
 stage-fusion tensors as a whole, the heads, and the parameter gradients per layer family.  Columns: max |got - ref|,
-the same divided by max |ref| of that tensor, for the fp32 mode (CUDA-core FFMA) and the tf32 mode (tcgen05
+the same divided by max |ref| of that tensor, for the fp32 mode (3xTF32 tcgen05) and the tf32 mode (tcgen05
 kind::tf32).  The last column is the error of the reference's OWN fp32 CPU arithmetic (oracle run in float32, i.e. the
 ATen CPU kernels the reference calls) against the same fp64 truth: the noise floor any fp32 implementation has.
 """
