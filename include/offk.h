@@ -352,9 +352,21 @@ int offk_head_bwd(const float* dout, int P, int C, int HW, int ctot, int coff, i
                   uint64_t seed, const uint64_t* seed_dev, float drop_p, float keep_scale, const float* weight,
                   int num_classes, int T, const float* pooled, const float* act, int accumulate, float* dx,
                   float* dweight, float* dbias, void* stream);
-/* 3x3 stride-2 ceil-mode max pool (motion_pool_trans_28, RGB_OFF.py:353,:783) */
-int offk_maxpool3s2_fwd(const float* x, int P, int C, int H, int W, int x_ctot, int x_coff, float* out,
-                        void* stream);
+/* 3x3 pool with ceil-mode output size between channel slices of channels-last tensors:
+ *   x [n_img, H, W, x_ctot], channels [x_coff, x_coff + C)  ->  y [n_img, Ho, Wo, y_ctot], channels [y_coff, y_coff + C)
+ *   Ho = ceil((H + 2 pad - 3) / stride) + 1, minus one if that last window would start at or past H + pad (the rule of
+ *   F.max_pool2d / F.avg_pool2d with ceil_mode=True); likewise Wo.  pad <= 1.
+ *   OFFK_POOL_MAX: max over the window elements inside the input (a window cut by the edge takes the max of the rest)
+ *   OFFK_POOL_AVG: sum over the window elements inside the input / 9 (count_include_pad=True); every window must lie
+ *                  inside the padded input, which holds for stride 1, pad 1
+ * C, x_ctot, x_coff, y_ctot, y_coff multiples of 4, x and y 16-byte aligned.  Used for motion_pool_trans_28
+ * (RGB_OFF.py:353,:783: max, stride 2, pad 0) and every pool of the BN-Inception extractor (RGB_OFF.py:43-263,362-594:
+ * pool1 / pool2 and the stride-2 modules 3c / 4e: max, stride 2, pad 0; the normal modules: avg, stride 1, pad 1; 5b:
+ * max, stride 1, pad 1). */
+#define OFFK_POOL_MAX 0
+#define OFFK_POOL_AVG 1
+int offk_pool3_nhwc(const float* x, int n_img, int H, int W, int x_ctot, int x_coff, int C, int stride, int pad, int kind,
+                    float* y, int y_ctot, int y_coff, void* stream);
 /* ConsensusModule('avg', dim=1): out[b,:] = mean_t x[b,t,:]  (basic_ops.py:21-22) and its backward (:30-31) */
 int offk_segment_mean_fwd(const float* x, int B, int T, int C, float* out, void* stream);
 int offk_segment_mean_bwd(const float* dout, int B, int T, int C, float* dx, void* stream);
@@ -401,6 +413,11 @@ int offk_gather_copy(const float* src, const int32_t* idx, float* dst, long long
  * RGB_OFF.py:567,590): their 196-byte channel stride is not a legal TMA stride, so the unit's 1x1 conv and its weight
  * gradient read this copy through dense / im2col tensor maps instead. */
 int offk_nchw_to_nhwc(const float* src, float* dst, int n_img, int C, int HW, void* stream);
+
+/* dst[n, p, c'] = c' < c ? src[n, c', p] : 0, p < hw, c' < c_pad: the NCHW image batch of the BN-Inception extractor as a
+ * channels-last tensor whose channel count c_pad (a multiple of 4: 4 for RGB, 12 for the 10-channel flow stack) gives the
+ * stem conv 16-byte channel groups.  dst 16-byte aligned. */
+int offk_image_to_nhwc(const float* src, float* dst, int n_img, int c, int hw, int c_pad, void* stream);
 
 /* ------------------------------------------------------------------------
  * The training step around the path (train_off.py:72,133-151), on the flat parameter / gradient buffers.

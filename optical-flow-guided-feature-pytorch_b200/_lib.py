@@ -15,6 +15,7 @@ LIB_PATH = os.environ.get("OFFK_LIB") or os.path.join(_HERE, "liboffk.so")   # O
 PREC_TF32, PREC_TF32X3 = 1, 2
 INDEX_REFERENCE_FLAT, INDEX_ALIGNED = 0, 1
 DROP_NONE, DROP_MASK, DROP_SEED = 0, 1, 2
+POOL_MAX, POOL_AVG = 0, 1
 LOAD_VEC_K, LOAD_VEC_ROW = 2, 3
 
 
@@ -116,7 +117,8 @@ _PROTOS = {
                                 C.c_float, _P, C.c_int, C.c_int, _P, _P, C.c_int, _P, _P, _P, _P]),
     "offk_seed_set": (C.c_int, [_P, C.c_uint64, _P]),
     "offk_seed_advance": (C.c_int, [_P, _P]),
-    "offk_maxpool3s2_fwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "offk_pool3_nhwc": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                  _P, C.c_int, C.c_int, _P]),
     "offk_segment_mean_fwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "offk_segment_mean_bwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "offk_fill_zero": (C.c_int, [_P, C.c_longlong, _P]),
@@ -126,6 +128,7 @@ _PROTOS = {
     "offk_bias_act": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "offk_add_relu_slice": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "offk_nchw_to_nhwc": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P]),
+    "offk_image_to_nhwc": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "offk_gather_copy": (C.c_int, [_P, _P, _P, C.c_longlong, _P]),
     "offk_tf32_residual": (C.c_int, [_P, _P, C.c_longlong, _P]),
     "offk_permute_weight_batch": (C.c_int, [C.c_int, C.POINTER(OffkPermute), C.c_int, _P]),

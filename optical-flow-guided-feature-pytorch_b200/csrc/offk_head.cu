@@ -1,5 +1,5 @@
 // Head-side kernels of the OFF sub-network (channels-last tensors [P, HW, C]): global average pool (+dropout) forward/backward,
-// 3x3/s2 ceil-mode max pool, segment consensus (mean over segments) and small element-wise passes.
+// the channels-last 3x3 pools (also those of the BN-Inception extractor), the image conversion of the extractor, segment consensus (mean over segments) and small element-wise passes.
 // All are bandwidth-trivial ([P,C,7,7] tensors); they exist so that no ATen op is left on the path.
 #include "offk_common.cuh"
 
@@ -55,28 +55,64 @@ __global__ void avgpool_drop_bwd_kernel(const float* __restrict__ dpooled, int P
   dx[o] = v;
 }
 
-__global__ void maxpool3s2_fwd_kernel(const float* __restrict__ x, int P, int C, int H, int W, int ctot, int coff,
-                                      int Ho, int Wo, float* __restrict__ out) {
+// 3x3 pool over a channel slice of a channels-last tensor, ceil-mode output, one thread per (output pixel, channel quad):
+// kind 0 = max over the valid window elements (F.max_pool2d), 1 = sum / 9 (F.avg_pool2d, count_include_pad=True, for
+// windows that stay inside the padded input -- every pool the plans use)
+__global__ void __launch_bounds__(256) pool3_nhwc_kernel(const float* __restrict__ x, int H, int W, int x_ctot, int x_coff,
+                                                         int CQ, int stride, int pad, int kind, int Ho, int Wo, long long total,
+                                                         float* __restrict__ y, int y_ctot, int y_coff) {
   pdl_sync();
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const size_t total = (size_t)P * C * Ho * Wo;
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
-  const int c = (int)(i % C);
-  const int ow = (int)((i / C) % Wo);
-  const int oh = (int)((i / ((size_t)C * Wo)) % Ho);
-  const int p = (int)(i / ((size_t)C * Wo * Ho));
-  const float* xp = x + (size_t)p * H * W * ctot + coff + c;
-  float m = -INFINITY;
+  const int cq = (int)(i % CQ);
+  const long long pix = i / CQ;                   // (img * Ho + oh) * Wo + ow
+  const int ow = (int)(pix % Wo);
+  const int oh = (int)((pix / Wo) % Ho);
+  const long long img = pix / ((long long)Wo * Ho);
+  const float* xp = x + img * H * W * (long long)x_ctot + x_coff + 4 * cq;
+  const int y0 = oh * stride - pad, x0 = ow * stride - pad;
+  float4 m = kind == 0 ? make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY) : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
   for (int a = 0; a < 3; ++a) {
-    const int y = oh * 2 + a;
-    if (y >= H) break;
+    const int yy = y0 + a;
+    if (yy < 0 || yy >= H) continue;
+#pragma unroll
     for (int b = 0; b < 3; ++b) {
-      const int xx = ow * 2 + b;
-      if (xx >= W) break;
-      m = fmaxf(m, __ldg(xp + (size_t)(y * W + xx) * ctot));
+      const int xx = x0 + b;
+      if (xx < 0 || xx >= W) continue;
+      const float4 v = __ldg(reinterpret_cast<const float4*>(xp + (long long)(yy * W + xx) * x_ctot));
+      if (kind == 0) {
+        m.x = fmaxf(m.x, v.x); m.y = fmaxf(m.y, v.y); m.z = fmaxf(m.z, v.z); m.w = fmaxf(m.w, v.w);
+      } else {
+        m.x += v.x; m.y += v.y; m.z += v.z; m.w += v.w;
+      }
     }
   }
-  out[i] = m;   // [P, Ho, Wo, C]
+  if (kind != 0) {
+    m.x /= 9.f; m.y /= 9.f; m.z /= 9.f; m.w /= 9.f;
+  }
+  *reinterpret_cast<float4*>(y + pix * y_ctot + y_coff + 4 * cq) = m;
+}
+
+// NCHW image batch [n, c, hw] -> channels-last [n, hw, c_pad], channels >= c zero: one thread per pixel, the c reads are
+// coalesced across the warp, the c_pad / 4 float4 stores are contiguous per thread
+__global__ void __launch_bounds__(256) image_to_nhwc_kernel(const float* __restrict__ src, float* __restrict__ dst, int c, int hw,
+                                                            int c_pad, long long total) {
+  pdl_sync();
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const long long img = i / hw;
+  const int p = (int)(i - img * hw);
+  const float* s = src + img * c * (long long)hw + p;
+  float* d = dst + i * c_pad;
+  for (int q = 0; q < c_pad; q += 4) {
+    float4 v;
+    v.x = q + 0 < c ? __ldg(s + (long long)(q + 0) * hw) : 0.f;
+    v.y = q + 1 < c ? __ldg(s + (long long)(q + 1) * hw) : 0.f;
+    v.z = q + 2 < c ? __ldg(s + (long long)(q + 2) * hw) : 0.f;
+    v.w = q + 3 < c ? __ldg(s + (long long)(q + 3) * hw) : 0.f;
+    *reinterpret_cast<float4*>(d + q) = v;
+  }
 }
 
 // ---------------------------------------------------------------------------- fused heads (SURVEY K6)
@@ -404,17 +440,36 @@ extern "C" int offk_avgpool_drop_bwd(const float* dpooled, int P, int C, int HW,
   return OFFK_LAUNCH_CHECK("avgpool_drop_bwd");
 }
 
-extern "C" int offk_maxpool3s2_fwd(const float* x, int P, int C, int H, int W, int x_ctot, int x_coff, float* out,
-                                   void* stream) {
-  OFFK_REQUIRE(x && out && P > 0 && C > 0 && H >= 3 && W >= 3 && x_coff >= 0 && x_coff + C <= x_ctot,
-               "maxpool: bad args");
-  int Ho = (H - 3 + 1) / 2 + 1, Wo = (W - 3 + 1) / 2 + 1;  // ceil((H-3)/2)+1 ...
-  if ((Ho - 1) * 2 >= H) --Ho;                             // ... and the last window must start inside the input
-  if ((Wo - 1) * 2 >= W) --Wo;
-  const size_t total = (size_t)P * C * Ho * Wo;
-  (void)launch_pdl(maxpool3s2_fwd_kernel, dim3(blocks_for(total, 256)), dim3(256), 0, as_stream(stream), x, P, C, H, W, x_ctot, x_coff, Ho, Wo,
-                                                                               out);
-  return OFFK_LAUNCH_CHECK("maxpool3s2_fwd");
+extern "C" int offk_pool3_nhwc(const float* x, int n_img, int H, int W, int x_ctot, int x_coff, int C, int stride, int pad,
+                               int kind, float* y, int y_ctot, int y_coff, void* stream) {
+  OFFK_REQUIRE(x && y && n_img > 0 && H > 0 && W > 0 && C > 0 && stride >= 1 && pad >= 0 && 2 * pad < 3 &&
+                   (kind == OFFK_POOL_MAX || kind == OFFK_POOL_AVG),
+               "pool3_nhwc: bad args");
+  OFFK_REQUIRE(C % 4 == 0 && x_ctot % 4 == 0 && x_coff % 4 == 0 && y_ctot % 4 == 0 && y_coff % 4 == 0 && x_coff + C <= x_ctot &&
+                   y_coff + C <= y_ctot && ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15u) == 0,
+               "pool3_nhwc: channel slices must be 16-byte aligned quads");
+  // ceil mode: ceil((H + 2 pad - 3) / stride) + 1 windows, the last of which must start inside the input or its left padding
+  int Ho = (H + 2 * pad - 3 + stride - 1) / stride + 1, Wo = (W + 2 * pad - 3 + stride - 1) / stride + 1;
+  if ((Ho - 1) * stride >= H + pad) --Ho;
+  if ((Wo - 1) * stride >= W + pad) --Wo;
+  OFFK_REQUIRE(Ho >= 1 && Wo >= 1, "pool3_nhwc: input smaller than the window");
+  // count_include_pad divides by 9 only while every window stays inside the padded input
+  OFFK_REQUIRE(kind == OFFK_POOL_MAX || ((Ho - 1) * stride + 3 <= H + 2 * pad && (Wo - 1) * stride + 3 <= W + 2 * pad),
+               "pool3_nhwc: an average window runs past the padded input");
+  const long long total = (long long)n_img * Ho * Wo * (C / 4);
+  (void)launch_pdl(pool3_nhwc_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, as_stream(stream), x, H, W, x_ctot,
+                   x_coff, C / 4, stride, pad, kind, Ho, Wo, total, y, y_ctot, y_coff);
+  return OFFK_LAUNCH_CHECK("pool3_nhwc");
+}
+
+extern "C" int offk_image_to_nhwc(const float* src, float* dst, int n_img, int c, int hw, int c_pad, void* stream) {
+  OFFK_REQUIRE(src && dst && n_img > 0 && hw > 0 && c > 0 && c <= c_pad && c_pad % 4 == 0 &&
+                   (reinterpret_cast<uintptr_t>(dst) & 15u) == 0,
+               "image_to_nhwc: bad args (0 < c <= c_pad, c_pad %% 4 == 0, 16-byte aligned dst)");
+  const long long total = (long long)n_img * hw;
+  (void)launch_pdl(image_to_nhwc_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, as_stream(stream), src, dst, c, hw,
+                   c_pad, total);
+  return OFFK_LAUNCH_CHECK("image_to_nhwc");
 }
 
 extern "C" int offk_head_fwd(const float* x, int P, int C, int HW, int x_ctot, int x_coff, int drop_mode, const uint8_t* keep_mask,

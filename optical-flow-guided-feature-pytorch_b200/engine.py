@@ -172,10 +172,10 @@ class TGemm(Gemm):
         t.precision = eng.prec
         t.bk = bk if (wgrad and x_layout != "nchw") else 0
         if eng.presplit and not wgrad:
-            # B is a weight matrix inside the parameter buffer or the per-step weight copies: its residuals sit at the same
-            # offset of the twin buffer
+            # B is a weight matrix inside one of the owner's weight buffers: its residuals sit at the same offset of the
+            # twin buffer
             bp = kw["b_src"].data_ptr()
-            for hi, lo in ((eng.params_flat, eng.params_lo), (eng.wc_flat, eng.wc_lo)):
+            for hi, lo in eng.lo_twins:
                 if hi.data_ptr() <= bp < hi.data_ptr() + hi.numel() * 4:
                     t.b_lo_delta = (lo.data_ptr() - hi.data_ptr()) // 4
                     self.reads.append(lo)
@@ -210,66 +210,11 @@ class TGemm(Gemm):
         L.check(lib.offk_tma_gemm(C.byref(self.tdesc), stream), self.name)
 
 
-class OFFEngine:
-    """Plan + buffers for one (batch, length) shape on one GPU.
-
-    variant: 'rgb'  learned depth-wise 3x3 spatial gradient + bias, per-pair logits (RGB_OFF.py)
-             'flow' fixed diagonal Sobel, segment consensus over the L-1 pairs (Flow_OFF.py / RGB_OFF_v2.py)
-    precision: 'fp32' = fp32-parity mode ON THE TENSOR CORES (OFFK_PREC_TF32X3: error-compensated 3xTF32 tcgen05 MMAs,
-               fp32 accumulate; the reference's arithmetic is fp32, RGB_OFF.py:597), 'tf32' = one kind::tf32 MMA per
-               product (the fast mode, tolerance stated separately)
-    """
-
-    def __init__(self, batch: int, length: int, variant: str = "rgb", device="cuda", precision: str = "tf32",
-                 index_mode: str = "reference_flat", consensus=None, tap_grads: bool = False):
-        assert variant in ("rgb", "flow") and length >= 2 and batch >= 1
-        self.lib = L.lib()
-        self.B, self.Lseg, self.variant = batch, length, variant
-        self.N, self.P = batch * length, batch * (length - 1)
-        self.device = torch.device(device)
-        self.prec = {"fp32": L.PREC_TF32X3, "tf32": L.PREC_TF32}[precision]
-        self.precision = precision
-        self.index_mode = {"reference_flat": L.INDEX_REFERENCE_FLAT, "aligned": L.INDEX_ALIGNED}[index_mode]
-        self.consensus = (variant != "rgb") if consensus is None else bool(consensus)
-        self.tap_grads = tap_grads
-        self.single_stream = False       # True: issue every lane on the caller's stream (profiling / debugging)
-        self._tab_cache = {}
-        self._keep = []
-        self.generation = 0
-
-        # ---- parameters: one flat buffer, reference-named views
-        self.layout, self.n_flat = S.flat_layout(variant)
-        # fp32 (3xTF32) mode: the tf32 residuals of the weights are produced once per step into a twin buffer directly behind
-        # the parameters, so that the GEMMs receive both weight tiles by TMA (offk.h: b_lo_delta) instead of splitting them in
-        # shared memory in every CTA and K-block
-        self.presplit = self.prec == L.PREC_TF32X3
-        self._params_all = torch.zeros(self.n_flat * (2 if self.presplit else 1), device=self.device)
-        self.params_flat = self._params_all[:self.n_flat]
-        self.params_lo = self._params_all[self.n_flat:] if self.presplit else None
-        self.grads_flat = torch.zeros(self.n_flat, device=self.device)
-        self.params = OrderedDict((n, self._view(self.params_flat, n)) for n in S.param_shapes(variant))
-        self.grads = OrderedDict((n, self._view(self.grads_flat, n)) for n in S.param_shapes(variant))
-        if variant == "flow":
-            # frozen util.SobelFilter_Diagonal taps (util.py:61), [32,1,3,3]
-            k = torch.tensor([[0., 1., 0.], [-1., 0., 1.], [0., -1., 0.]], device=self.device)
-            self.sobel_w = k.expand(S.DOWN_C, 1, 3, 3).contiguous()
-
-        self._alloc()
-        self._build()
-
-    # ------------------------------------------------------------------ helpers
-    def _view(self, flat, name):
-        off, shape = self.layout[name]
-        return flat[off:off + int(np.prod(shape))].view(shape)
-
-    def _unit_w(self, flat, tag):
-        off, _ = self.layout[f"motion_conv_gen_{tag}.weight"]
-        cin = S.LEVELS[tag][0]
-        return flat[off:off + S.UNIT_C * cin].view(S.UNIT_C, cin)
-
-    def _unit_b(self, flat, tag):
-        off, _ = self.layout[f"motion_conv_gen_{tag}.bias"]
-        return flat[off:off + S.UNIT_C]
+class GemmOwner:
+    """What a bound Gemm / TGemm needs from the plan that owns it: ``lib``, ``device``, ``prec``, ``presplit`` (3xTF32 with
+    the weights' tf32 residuals in twin buffers), ``lo_twins`` ([(weights, residuals)] buffer pairs for b_lo_delta), the
+    table cache and ``flops_fwd``; and the forward-conv launch policy (``_conv_fwd``).  OFFEngine and the BN-Inception
+    extractor plan (extractor.py) are the two owners."""
 
     def _tables(self, key, spc: T.GemmSpec):
         if key not in self._tab_cache:
@@ -277,117 +222,6 @@ class OFFEngine:
             self._tab_cache[key] = {k: torch.from_numpy(v).to(dev) for k, v in T.padded_tables(spc).items()}
         return self._tab_cache[key]
 
-    def _buf(self, name, *shape):
-        t = torch.zeros(*shape, device=self.device)
-        self.buf[name] = t
-        return t
-
-    def load_params(self, prm: dict):
-        """Copy reference-named tensors (a state_dict subset) into the flat buffer."""
-        with torch.no_grad():
-            for n, v in self.params.items():
-                v.copy_(prm[n].to(self.device, torch.float32))
-
-    # ------------------------------------------------------------------ buffers
-    def _alloc(self):
-        P, N = self.P, self.N
-        self.buf = {}
-        for tag, (cin, s) in S.LEVELS.items():
-            self._buf("gd_" + tag, N, s, s, S.UNIT_C)
-            self._buf("dgd_" + tag, N, s, s, S.UNIT_C)
-        for st, (ctot, s, _) in S.STAGES.items():
-            self._buf("F" + st, P, s, s, ctot)
-            self._buf("dF" + st, P, s, s, ctot)
-        a = lambda n, c, s: (self._buf(n, P, s, s, c), self._buf("d_" + n, P, s, s, c))
-        a("t28", 64, 14)
-        self._buf("t28r", P, 14, 14, 64)          # relu(t28): conv1_trans_28a consumes the activated copy (RGB_OFF.py:658-659)
-        a("tmp28", 64, 14)
-        for blk in "abc":
-            a("h1_28" + blk, 64, 14)
-            a("h2_28" + blk, 64, 14)
-        a("br28", 256, 14)
-        a("s28a", 256, 14)
-        a("s28b", 256, 14)
-        a("t14", 128, 7)
-        a("tmp14", 128, 7)
-        for blk in "ab":
-            a("h1_14" + blk, 128, 7)
-            a("h2_14" + blk, 128, 7)
-        a("ex14", 512, 7)
-        a("s14a", 512, 7)
-        a("h3_14b", 512, 7)
-        a("t7", 256, 7)
-        a("tmp7", 256, 7)
-        a("h1_7", 256, 7)
-        a("h2_7", 256, 7)
-        a("br7", 1024, 7)
-        a("s7", 1024, 7)
-        self._buf("p28", P, 7, 7, 256)
-        for k, c in (("7", 1024), ("14", 512), ("28", 256)):
-            self._buf("pool" + k, P, c)
-            self._buf("fc" + k, P, S.NUM_CLASSES)
-            if self.consensus:
-                self._buf("cfc" + k, self.B, S.NUM_CLASSES)
-        # two input sets: while one is being consumed (forward AND backward read the taps) the other can be filled by
-        # an asynchronous host->device copy (stage_taps)
-        self.tap_sets = [OrderedDict((tag, torch.zeros(N, cin, s, s, device=self.device)) for tag, (cin, s) in S.LEVELS.items())
-                         for _ in range(2)]
-        self.taps = self.tap_sets[0]
-        self._tap_set = 0
-        self._tap_users = {tag: [] for tag in S.LEVELS}      # bound GEMMs whose A operand is the tap
-        self._copy_stream = None
-        if self.tap_grads:
-            self.tap_grad = OrderedDict((tag, torch.zeros_like(t)) for tag, t in self.taps.items())
-        # Per-step weight re-layouts, produced by ONE gather-copy launch (wc_flat[i] = params_flat[wc_idx[i]]):
-        #   wp[name] : OHWI [cout, kh, kw, cin] copies of the KxK conv weights (K order of the channels-last implicit GEMM)
-        #   wd[name] : [cin, kh, kw, cout] copies with flipped taps of every stride-1 conv = the B operand of its
-        #              data-gradient GEMM (dX = dY * W^T as a forward conv over dY)
-        # dwp[name]: OHWI accumulators of the KxK weight gradients (un-permuted into grads_flat after the backward)
-        self.wp, self.dwp, self.wd = {}, {}, {}
-        kxk = [(name, cout, cin, k) for name, cout, cin, k, _, _ in S.STAGE_CONVS if k > 1]
-        total = sum(cout * cin * k * k for _, cout, cin, k in kxk)
-        self.dwp_flat = torch.zeros(total, device=self.device)
-        idx, off, views = [], 0, []
-        for name, cout, cin, k, stride, pad in S.STAGE_CONVS:
-            p_off = self.layout[name + ".weight"][0]
-            oihw = p_off + np.arange(cout * cin * k * k, dtype=np.int64).reshape(cout, cin, k, k)
-            if k > 1:
-                idx.append(oihw.transpose(0, 2, 3, 1).reshape(-1))
-                views.append(("wp", name, off, (cout, k, k, cin)))
-                off += oihw.size
-            if stride == 1:
-                idx.append(p_off + T.dgrad_class_weight_index(cout, cin, k, 1, pad, 0, 0))
-                views.append(("wd", name, off, (cin, k * k * cout)))
-                off += oihw.size
-            else:
-                # one [cin, R, Q, cout] block per stride-parity class (a, b) of the input pixel
-                for a in range(stride):
-                    for b in range(stride):
-                        sub = p_off + T.dgrad_class_weight_index(cout, cin, k, stride, pad, a, b)
-                        idx.append(sub)
-                        views.append(("wd", (name, a, b), off, (cin, sub.size // cin)))
-                        off += sub.size
-        self.wc_idx = torch.from_numpy(np.concatenate(idx).astype(np.int32)).to(self.device)
-        off = (off + 3) // 4 * 4
-        self._wc_all = torch.zeros(off * (2 if self.presplit else 1), device=self.device)
-        self.wc_flat = self._wc_all[:off]
-        self.wc_lo = self._wc_all[off:] if self.presplit else None
-        for kind, name, o, shape in views:
-            getattr(self, kind)[name] = self.wc_flat[o:o + int(np.prod(shape))].view(shape)
-        off = 0
-        for name, cout, cin, k in kxk:
-            n = cout * cin * k * k
-            self.dwp[name] = self.dwp_flat[off:off + n].view(cout, k, k, cin)
-            off += n
-        # dropout state (filled per forward call)
-        self.drop_mode = L.DROP_NONE
-        self.drop_seed = 0
-        self.masks = None
-        self.seed_state = torch.zeros(1, dtype=torch.int64, device=self.device)   # per-step dropout seed (device word)
-        self._graphs = {}                # (pass, tap set, dropout mode) -> torch.cuda.CUDAGraph
-        self._cap_stream = None
-
-    # ------------------------------------------------------------------ plan
     def _conv_fwd(self, name, x, y, geom, w, b, *, relu=False, relu_cols=None, addend=None,
                   add_tabs=None, relu_post=False, x_layout="nhwc", no_split=False, aux=None):
         """One TMA-fed launch (TGemm); a geometry without a TMA-fed form is an error.
@@ -459,8 +293,196 @@ class OFFEngine:
         self.flops_fwd += g.flops
         return g
 
+
+class OFFEngine(GemmOwner):
+    """Plan + buffers for one (batch, length) shape on one GPU.
+
+    tap_layout: 'nchw' (the reference's layout) or 'channels_last': both tap sets are [N, C, S, S] tensors in
+               torch.channels_last memory format (what the fused BN-Inception extractor writes), and every unit reads its
+               tap through dense / im2col tensor maps in place, as the NCHW plan does for the 7x7 levels through a copy
+
+    variant: 'rgb'  learned depth-wise 3x3 spatial gradient + bias, per-pair logits (RGB_OFF.py)
+             'flow' fixed diagonal Sobel, segment consensus over the L-1 pairs (Flow_OFF.py / RGB_OFF_v2.py)
+    precision: 'fp32' = fp32-parity mode ON THE TENSOR CORES (OFFK_PREC_TF32X3: error-compensated 3xTF32 tcgen05 MMAs,
+               fp32 accumulate; the reference's arithmetic is fp32, RGB_OFF.py:597), 'tf32' = one kind::tf32 MMA per
+               product (the fast mode, tolerance stated separately)
+    """
+
+    def __init__(self, batch: int, length: int, variant: str = "rgb", device="cuda", precision: str = "tf32",
+                 index_mode: str = "reference_flat", consensus=None, tap_grads: bool = False, tap_layout: str = "nchw"):
+        assert variant in ("rgb", "flow") and length >= 2 and batch >= 1
+        if tap_layout not in ("nchw", "channels_last"):
+            raise ValueError(f"tap_layout: 'nchw' or 'channels_last', not {tap_layout!r}")
+        if tap_grads and tap_layout == "channels_last":
+            # the channels-last taps come from the frozen fused extractor (train_off.py:39-46): nothing consumes their gradient
+            raise ValueError("tap_grads=True needs tap_layout='nchw': channels-last taps come from the frozen extractor")
+        self.tap_layout = tap_layout
+        self.lib = L.lib()
+        self.B, self.Lseg, self.variant = batch, length, variant
+        self.N, self.P = batch * length, batch * (length - 1)
+        self.device = torch.device(device)
+        self.prec = {"fp32": L.PREC_TF32X3, "tf32": L.PREC_TF32}[precision]
+        self.precision = precision
+        self.index_mode = {"reference_flat": L.INDEX_REFERENCE_FLAT, "aligned": L.INDEX_ALIGNED}[index_mode]
+        self.consensus = (variant != "rgb") if consensus is None else bool(consensus)
+        self.tap_grads = tap_grads
+        self.single_stream = False       # True: issue every lane on the caller's stream (profiling / debugging)
+        self._tab_cache = {}
+        self._keep = []
+        self.generation = 0
+
+        # ---- parameters: one flat buffer, reference-named views
+        self.layout, self.n_flat = S.flat_layout(variant)
+        # fp32 (3xTF32) mode: the tf32 residuals of the weights are produced once per step into a twin buffer directly behind
+        # the parameters, so that the GEMMs receive both weight tiles by TMA (offk.h: b_lo_delta) instead of splitting them in
+        # shared memory in every CTA and K-block
+        self.presplit = self.prec == L.PREC_TF32X3
+        self._params_all = torch.zeros(self.n_flat * (2 if self.presplit else 1), device=self.device)
+        self.params_flat = self._params_all[:self.n_flat]
+        self.params_lo = self._params_all[self.n_flat:] if self.presplit else None
+        self.grads_flat = torch.zeros(self.n_flat, device=self.device)
+        self.params = OrderedDict((n, self._view(self.params_flat, n)) for n in S.param_shapes(variant))
+        self.grads = OrderedDict((n, self._view(self.grads_flat, n)) for n in S.param_shapes(variant))
+        if variant == "flow":
+            # frozen util.SobelFilter_Diagonal taps (util.py:61), [32,1,3,3]
+            k = torch.tensor([[0., 1., 0.], [-1., 0., 1.], [0., -1., 0.]], device=self.device)
+            self.sobel_w = k.expand(S.DOWN_C, 1, 3, 3).contiguous()
+
+        self._alloc()
+        self._build()
+
+    # ------------------------------------------------------------------ helpers
+    def _view(self, flat, name):
+        off, shape = self.layout[name]
+        return flat[off:off + int(np.prod(shape))].view(shape)
+
+    def _unit_w(self, flat, tag):
+        off, _ = self.layout[f"motion_conv_gen_{tag}.weight"]
+        cin = S.LEVELS[tag][0]
+        return flat[off:off + S.UNIT_C * cin].view(S.UNIT_C, cin)
+
+    def _unit_b(self, flat, tag):
+        off, _ = self.layout[f"motion_conv_gen_{tag}.bias"]
+        return flat[off:off + S.UNIT_C]
+
+    def _buf(self, name, *shape):
+        t = torch.zeros(*shape, device=self.device)
+        self.buf[name] = t
+        return t
+
+    def load_params(self, prm: dict):
+        """Copy reference-named tensors (a state_dict subset) into the flat buffer."""
+        with torch.no_grad():
+            for n, v in self.params.items():
+                v.copy_(prm[n].to(self.device, torch.float32))
+
+    # ------------------------------------------------------------------ buffers
+    def _alloc(self):
+        P, N = self.P, self.N
+        self.buf = {}
+        for tag, (cin, s) in S.LEVELS.items():
+            self._buf("gd_" + tag, N, s, s, S.UNIT_C)
+            self._buf("dgd_" + tag, N, s, s, S.UNIT_C)
+        for st, (ctot, s, _) in S.STAGES.items():
+            self._buf("F" + st, P, s, s, ctot)
+            self._buf("dF" + st, P, s, s, ctot)
+        a = lambda n, c, s: (self._buf(n, P, s, s, c), self._buf("d_" + n, P, s, s, c))
+        a("t28", 64, 14)
+        self._buf("t28r", P, 14, 14, 64)          # relu(t28): conv1_trans_28a consumes the activated copy (RGB_OFF.py:658-659)
+        a("tmp28", 64, 14)
+        for blk in "abc":
+            a("h1_28" + blk, 64, 14)
+            a("h2_28" + blk, 64, 14)
+        a("br28", 256, 14)
+        a("s28a", 256, 14)
+        a("s28b", 256, 14)
+        a("t14", 128, 7)
+        a("tmp14", 128, 7)
+        for blk in "ab":
+            a("h1_14" + blk, 128, 7)
+            a("h2_14" + blk, 128, 7)
+        a("ex14", 512, 7)
+        a("s14a", 512, 7)
+        a("h3_14b", 512, 7)
+        a("t7", 256, 7)
+        a("tmp7", 256, 7)
+        a("h1_7", 256, 7)
+        a("h2_7", 256, 7)
+        a("br7", 1024, 7)
+        a("s7", 1024, 7)
+        self._buf("p28", P, 7, 7, 256)
+        for k, c in (("7", 1024), ("14", 512), ("28", 256)):
+            self._buf("pool" + k, P, c)
+            self._buf("fc" + k, P, S.NUM_CLASSES)
+            if self.consensus:
+                self._buf("cfc" + k, self.B, S.NUM_CLASSES)
+        # two input sets: while one is being consumed (forward AND backward read the taps) the other can be filled by
+        # an asynchronous host->device copy (stage_taps)
+        if self.tap_layout == "channels_last":      # [N, C, S, S] views of [N, S, S, C] storage
+            tap = lambda cin, s: torch.zeros(N, s, s, cin, device=self.device).permute(0, 3, 1, 2)
+        else:
+            tap = lambda cin, s: torch.zeros(N, cin, s, s, device=self.device)
+        self.tap_sets = [OrderedDict((tag, tap(cin, s)) for tag, (cin, s) in S.LEVELS.items()) for _ in range(2)]
+        self.taps = self.tap_sets[0]
+        self._tap_set = 0
+        self._tap_users = {tag: [] for tag in S.LEVELS}      # bound GEMMs whose A operand is the tap
+        self._copy_stream = None
+        if self.tap_grads:
+            self.tap_grad = OrderedDict((tag, torch.zeros_like(t)) for tag, t in self.taps.items())
+        # Per-step weight re-layouts, produced by ONE gather-copy launch (wc_flat[i] = params_flat[wc_idx[i]]):
+        #   wp[name] : OHWI [cout, kh, kw, cin] copies of the KxK conv weights (K order of the channels-last implicit GEMM)
+        #   wd[name] : [cin, kh, kw, cout] copies with flipped taps of every stride-1 conv = the B operand of its
+        #              data-gradient GEMM (dX = dY * W^T as a forward conv over dY)
+        # dwp[name]: OHWI accumulators of the KxK weight gradients (un-permuted into grads_flat after the backward)
+        self.wp, self.dwp, self.wd = {}, {}, {}
+        kxk = [(name, cout, cin, k) for name, cout, cin, k, _, _ in S.STAGE_CONVS if k > 1]
+        total = sum(cout * cin * k * k for _, cout, cin, k in kxk)
+        self.dwp_flat = torch.zeros(total, device=self.device)
+        idx, off, views = [], 0, []
+        for name, cout, cin, k, stride, pad in S.STAGE_CONVS:
+            p_off = self.layout[name + ".weight"][0]
+            oihw = p_off + np.arange(cout * cin * k * k, dtype=np.int64).reshape(cout, cin, k, k)
+            if k > 1:
+                idx.append(oihw.transpose(0, 2, 3, 1).reshape(-1))
+                views.append(("wp", name, off, (cout, k, k, cin)))
+                off += oihw.size
+            if stride == 1:
+                idx.append(p_off + T.dgrad_class_weight_index(cout, cin, k, 1, pad, 0, 0))
+                views.append(("wd", name, off, (cin, k * k * cout)))
+                off += oihw.size
+            else:
+                # one [cin, R, Q, cout] block per stride-parity class (a, b) of the input pixel
+                for a in range(stride):
+                    for b in range(stride):
+                        sub = p_off + T.dgrad_class_weight_index(cout, cin, k, stride, pad, a, b)
+                        idx.append(sub)
+                        views.append(("wd", (name, a, b), off, (cin, sub.size // cin)))
+                        off += sub.size
+        self.wc_idx = torch.from_numpy(np.concatenate(idx).astype(np.int32)).to(self.device)
+        off = (off + 3) // 4 * 4
+        self._wc_all = torch.zeros(off * (2 if self.presplit else 1), device=self.device)
+        self.wc_flat = self._wc_all[:off]
+        self.wc_lo = self._wc_all[off:] if self.presplit else None
+        self.lo_twins = [(self.params_flat, self.params_lo), (self.wc_flat, self.wc_lo)]
+        for kind, name, o, shape in views:
+            getattr(self, kind)[name] = self.wc_flat[o:o + int(np.prod(shape))].view(shape)
+        off = 0
+        for name, cout, cin, k in kxk:
+            n = cout * cin * k * k
+            self.dwp[name] = self.dwp_flat[off:off + n].view(cout, k, k, cin)
+            off += n
+        # dropout state (filled per forward call)
+        self.drop_mode = L.DROP_NONE
+        self.drop_seed = 0
+        self.masks = None
+        self.seed_state = torch.zeros(1, dtype=torch.int64, device=self.device)   # per-step dropout seed (device word)
+        self._graphs = {}                # (pass, tap set, dropout mode) -> torch.cuda.CUDAGraph
+        self._cap_stream = None
+
+    # ------------------------------------------------------------------ plan
     def _conv_wgrad(self, name, x, dy, geom, dw, db, *, x_layout="nhwc", tap_copy=False):
-        """tap_copy: x is the channels-last copy of a unit's tap (the 7x7 levels), which is TMA-fed like the NCHW tap."""
+        """tap_copy: x is a unit's channels-last tap (or, in the NCHW plan, the channels-last copy of a 7x7 tap), which is
+        TMA-fed like the NCHW tap."""
         # dW is accumulated in the k order of the implicit GEMM (OHWI: consecutive accumulator rows = consecutive
         # addresses, so the split-K reductions coalesce) and un-permuted once at the end; writing OIHW directly
         # (dw_layout="oihw") was measured slower: the strided atomics cost more than the permute pass
@@ -564,16 +586,22 @@ class OFFEngine:
             gd, dgd = bf["gd_" + tag], bf["dgd_" + tag]
             # K1: gen (ReLU) and down (linear) 1x1 convs as ONE GEMM with 160 output channels
             # 7x7 taps: a 196-byte channel stride is not a legal TMA stride -> one channels-last copy of the tap per
-            # step feeds both the forward GEMM (dense tensor map) and the weight gradient (im2col_t), all TMA-fed
-            via_copy = (s * s) % 4 != 0 and cin % 32 == 0
+            # step feeds both the forward GEMM (dense tensor map) and the weight gradient (im2col_t), all TMA-fed.
+            # Channels-last taps take that route in place, at every level.
+            cl = self.tap_layout == "channels_last"
+            via_copy = (s * s) % 4 != 0 and cin % 32 == 0 and not cl
             if via_copy:
                 tapT = self._buf("tapT_" + tag, N, s, s, cin)
 
                 def kt(stream, tag=tag, tapT=tapT, cin=cin, hw=s * s):
                     L.check(lib.offk_nchw_to_nhwc(_ptr(self.taps[tag]), _ptr(tapT), N, cin, hw, stream), "tapT_" + tag)
                 fwd.append(_nm(kt, "tapT_" + tag, writes=[tapT], lane=fl))
-                k1 = self._conv_fwd("unit_" + tag, tapT, gd, geom, self._unit_w(self.params_flat, tag),
+            x_cl = self.taps[tag] if cl else (tapT if via_copy else None)
+            if x_cl is not None:
+                k1 = self._conv_fwd("unit_" + tag, x_cl, gd, geom, self._unit_w(self.params_flat, tag),
                                     self._unit_b(self.params_flat, tag), relu_cols=S.GEN_C, x_layout="nhwc", no_split=True)
+                if cl:
+                    self._tap_users[tag].append(getattr(k1, "gemm", k1))
             else:
                 k1 = self._conv_fwd("unit_" + tag, self.taps[tag], gd, geom, self._unit_w(self.params_flat, tag),
                                     self._unit_b(self.params_flat, tag), relu_cols=S.GEN_C, x_layout="nchw")
@@ -601,9 +629,11 @@ class OFFEngine:
             io.dw = dw3.data_ptr() if dw3 is not None else None
             io.dbias = db3.data_ptr() if db3 is not None else None
             # K4: weight / bias gradient of the fused 1x1 (no dX for the frozen taps unless asked, train_off.py:39-46)
-            if via_copy:
-                k4 = self._conv_wgrad("unit_" + tag, tapT, dgd, geom, self._unit_w(self.grads_flat, tag),
+            if x_cl is not None:
+                k4 = self._conv_wgrad("unit_" + tag, x_cl, dgd, geom, self._unit_w(self.grads_flat, tag),
                                       self._unit_b(self.grads_flat, tag), x_layout="nhwc", tap_copy=True)
+                if cl:
+                    self._tap_users[tag].append(k4)
             else:
                 k4 = self._conv_wgrad("unit_" + tag, self.taps[tag], dgd, geom,
                                       self._unit_w(self.grads_flat, tag), self._unit_b(self.grads_flat, tag), x_layout="nchw")
@@ -706,8 +736,8 @@ class OFFEngine:
             fwd.append(self._add_into_slice(bf["s14a"], bf["h3_14b"], bf["F7"], 832, 320, 512, 49))
 
         # ---- heads 28 / 14 (RGB_OFF.py:783-793)
-        fwd.append(_nm(lambda stream: L.check(lib.offk_maxpool3s2_fwd(_ptr(bf["F14"]), P, 256, 14, 14, 1056, 800,
-                                                                       _ptr(bf["p28"]), stream), "maxpool28"), "maxpool28",
+        fwd.append(_nm(lambda stream: L.check(lib.offk_pool3_nhwc(_ptr(bf["F14"]), P, 14, 14, 1056, 800, 256, 2, 0, L.POOL_MAX,
+                                                                   _ptr(bf["p28"]), 256, 0, stream), "maxpool28"), "maxpool28",
                        reads=[bf["F14"]], writes=[bf["p28"]], lane=1))
         # each head = ONE launch: avgpool 7x7 -> dropout -> Linear (-> segment consensus)   (SURVEY K6)
         fwd.append(_on(self._head_fwd("28", bf["p28"], 256, 256, 0, "fc_action_motion_28"), 1))

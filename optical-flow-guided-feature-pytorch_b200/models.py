@@ -4,9 +4,11 @@ and RGB_OFF_v2.py:43-58,1378-1392.
 
 Only the OFF section (RGB_OFF.py:596-860 / Flow_OFF.py:606-884) is implemented here -- it runs on liboffk through
 ``OFFSubNetwork``.  The frozen BN-Inception feature extractor (RGB_OFF.py:43-263,362-594; train_off.py:39-57 keeps it
-in eval mode without gradients) is not part of the accelerated path: pass ``backbone="bninception"`` for the built-in
+in eval mode without gradients) is optional: pass ``backbone="bninception"`` for the built-in
 table-driven restatement on stock torch ops (``off_b200/backbone.py``; the model is then a complete drop-in: images in,
-the reference's 593 / 576 state_dict entries), or pass any module mapping the
+the reference's 593 / 576 state_dict entries), ``backbone="bninception_fused"`` for the same extractor on liboffk
+(``off_b200/extractor.py``: CUDA fp32 images of exactly ``batch*length`` frames, BatchNorm folded from its running
+statistics, the taps written channels-last straight into the OFF engine's input buffers), or pass any module mapping the
 image batch ``[batch*length, 3 | 10, 224, 224]`` to ``(taps, score)`` where ``taps`` holds the nine Inception outputs
 '3a'..'5b' (``inception_3a_output_out`` ... ``inception_5b_output_out``, RGB_OFF.py:395-590) and ``score`` is
 ``Feature_Generation_Score`` ``[batch*length, num_classes]`` (:592-594).  Without a backbone the forward methods take
@@ -44,15 +46,22 @@ class BNInception_OFF(nn.Module):
         self.consensus_type = "avg"
         self.consensus = ConsensusModule(self.consensus_type, dim=1)          # Flow_OFF.py:47-48
         off_variant = "rgb" if variant == "rgb" else "flow"
+        if isinstance(backbone, str) and backbone not in ("bninception", "bninception_fused"):
+            raise ValueError("backbone: a module, None, 'bninception' (the built-in TSN BN-Inception extractor on stock torch "
+                             "ops) or 'bninception_fused' (the same extractor on liboffk, writing channels-last taps)")
+        fused = backbone == "bninception_fused"
         # not registered as a child: its parameter holders are re-registered below under the reference's names
         object.__setattr__(self, "off", OFFSubNetwork(batch, length, off_variant, precision=precision, index_mode=index_mode,
-                                                      tap_grads=tap_grads, device=device))
+                                                      tap_grads=tap_grads, device=device,
+                                                      tap_layout="channels_last" if fused else "nchw"))
         for name, mod in self.off.named_children():
             setattr(self, name, mod)                  # motion_conv_gen_3a ... fc_action_motion_14 (+ sobel_edge_diagonal)
         self._off_children = tuple(n for n, _ in self.off.named_children())
-        if isinstance(backbone, str):
-            if backbone != "bninception":
-                raise ValueError("backbone: a module, None, or 'bninception' (the built-in TSN BN-Inception extractor)")
+        if fused:
+            from .extractor import FusedBNInception
+            backbone = FusedBNInception(num_classes, 10 if variant == "flow" else 3, batch * length, precision, device,
+                                        taps=self.off.engine.tap_sets[0])
+        elif isinstance(backbone, str):
             from .backbone import BNInceptionBackbone
             backbone = BNInceptionBackbone(num_classes, in_channels=10 if variant == "flow" else 3).to(device)
         self._attach_backbone(backbone)
@@ -106,6 +115,8 @@ class BNInception_OFF(nn.Module):
                 raise RuntimeError("BNInception_OFF was built without a backbone: pass the nine Inception taps "
                                    "('3a'..'5b'), or construct it with backbone=<module returning (taps, score)>")
             return input, None, None
+        if hasattr(self.backbone, "plan"):            # FusedBNInception: its pass is replayed as a graph with the OFF passes
+            self.backbone.use_graphs = self.off.use_graphs
         out = self.backbone(input)
         taps, score = out[0], out[1]
         extra = out[2] if len(out) > 2 else None

@@ -116,18 +116,19 @@ class OFFSubNetwork(nn.Module):
     logits ``[batch*(length-1), 101]``; variant='flow' (also RGB_OFF_v2): fixed diagonal Sobel and segment consensus
     ``[batch, 101]``.  Dropout follows ``self.training`` (p = 0.8, RGB_OFF.py:356); pass ``masks`` to inject keep-masks.
     ``precision``: 'fp32' = fp32-parity arithmetic on the tensor cores (3xTF32), 'tf32' = single-MMA tf32 (the default here,
-    the fast mode).  ``use_graphs``: replay each pass as one captured CUDA graph.
+    the fast mode).  ``use_graphs``: replay each pass as one captured CUDA graph.  ``tap_layout='channels_last'``: the
+    engine's tap buffers are channels-last (what ``FusedBNInception`` writes in place); other taps are copied into them.
     """
 
     def __init__(self, batch: int, length: int, variant: str = "rgb", precision: str = "tf32",
                  index_mode: str = "reference_flat", consensus=None, tap_grads: bool = False, device="cuda",
-                 use_graphs=None):
+                 use_graphs=None, tap_layout: str = "nchw"):
         super().__init__()
         self.batch, self.length, self.variant = batch, length, variant
         # forward / backward as one captured CUDA graph each (same kernels, no per-launch host cost); OFFK_GRAPHS=1 turns it
         # on for modules that do not say
         self.use_graphs = (os.environ.get("OFFK_GRAPHS", "0") == "1") if use_graphs is None else bool(use_graphs)
-        self.engine = OFFEngine(batch, length, variant, device, precision, index_mode, consensus, tap_grads)
+        self.engine = OFFEngine(batch, length, variant, device, precision, index_mode, consensus, tap_grads, tap_layout)
         self._seed = 0
         groups = OrderedDict()
         for name in S.param_shapes(variant):
