@@ -22,279 +22,12 @@ import torch
 from . import _lib as L
 from . import spec as S
 from . import tables as T
-
-_SM_TARGET = 148
-_PICK_A = 128           # _pick_tile_n: per-CTA cost ~ _PICK_A + bn (A rows + B rows of a K-block)
-_WGRAD_FIXED_KB = 10    # _wgrad_split: fixed cost of a weight-gradient CTA, in K-blocks of 32 pixels
-_TF32_WANT_CTAS = _SM_TARGET    # _auto_tile_n: CTAs a TMA-fed GEMM without split-K aims for in the tf32 mode
-_X3_WANT_CTAS = 40      # ... and in the 3xTF32 mode
-_FINISH_MIN_TILES = 100     # output tiles from which a split-K conv finishes in-kernel (_conv_fwd)
+from .plan import (_OUT_TABLES, _SM_TARGET, _FreeGeom, Gemm, LaunchPlan, Schedule, TGemm, _gkey, _kernels, _nm, _on,
+                   _pick_tile_n, _ptr, _wgrad_split)
+from .plan import _auto_tile_n, _names  # noqa: F401  (re-exported: bench.py and the tests import them from here)
 
 
-def _ptr(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
-
-
-class _FreeGeom:
-    """im2col geometry with a caller-given output grid and separate top / left padding (OFFK_TGEMM_FREE_GEOM)."""
-
-    def __init__(self, **kw):
-        self.__dict__.update(kw)
-
-
-def _pick_tile_n(M: int, N: int, slots: int = 2 * _SM_TARGET) -> int:
-    """N tile (multiple of 16, <= 256; the last tile may be partial) of a GEMM without split-K: the one that minimises
-    rounds x per-CTA cost, rounds = ceil(CTAs / resident CTA slots) and cost ~ 128 + bn (rows of A and B a K-block moves
-    through shared memory).  Wave quantisation matters: 37 x 11 tiles of 96 columns are 1.4 rounds, 37 x 8 of 144 are one."""
-    mt = math.ceil(M / 128)
-    best, best_cost = 0, None
-    for bn in range(256, 15, -16):
-        if bn > (N + 15) // 16 * 16:
-            continue
-        nt = math.ceil(N / bn)
-        cost = math.ceil(mt * nt / slots) * (_PICK_A + bn) * (1.0 if mt * nt >= _SM_TARGET else _SM_TARGET / (mt * nt)) ** 0.5
-        if best_cost is None or cost < best_cost - 1e-9:
-            best, best_cost = bn, cost
-    return best
-
-
-def _wgrad_split(tiles: int, kb: int, slots: int, bk: int = 32) -> int:
-    """Split-K factor of a weight-gradient GEMM with `tiles` output tiles and `kb` K-blocks of `bk` pixels: the one that
-    minimises rounds x (K-blocks per CTA + fixed cost), rounds = ceil(CTAs / resident CTA slots); an under-filled round is
-    charged as idle SMs.  The fixed cost (prologue, first TMA round trip, adding the tile into dW) is worth ~10 K-blocks of
-    32 pixels (profiles/timeline_*_r02z.txt); the result is insensitive to it between 5 and 20 (profiles/env_r03j.log)."""
-    fixed = _WGRAD_FIXED_KB * 32 / bk
-    cost = lambda s_: math.ceil(tiles * s_ / slots) * (math.ceil(kb / s_) + fixed) * max(1.0, _SM_TARGET / (tiles * s_))
-    return min(range(1, max(1, kb // 4) + 1), key=lambda s_: (cost(s_), s_))
-
-
-class Gemm:
-    """One bound gather-GEMM launch (descriptor + device tables kept alive)."""
-
-    def __init__(self, eng: "OFFEngine", spc: T.GemmSpec, key, *, a_src, b_src, out, bias=None, relu_pre_cols=0,
-                 gate=None, gate_tabs=None, gate_col0=0, gate_first=False, addend=None,
-                 add_tabs=None, relu_post=False, atomic=False, ones_out=None, split_k=1, tile_n=0, name="",
-                 finish=False, aux=None, out_vec=None):
-        if spc.a_mode is None or spc.b_mode is None:
-            raise ValueError(f"{name}: an operand of this {spc.kind} GEMM has no 16-byte load form (tables.GemmSpec)")
-        self.eng, self.name, self.spec = eng, name, spc
-        tabs = eng._tables(key, spc)
-        d = L.OffkGemm()
-        d.M, d.N, d.K = spc.M, spc.N, spc.K
-        d.a_src, d.a_row, d.a_col = a_src.data_ptr(), tabs["a_row"].data_ptr(), tabs["a_col"].data_ptr()
-        d.a_h, d.a_w = (spc.a_h, spc.a_w) if spc.a_h else (T.NO_BOX, T.NO_BOX)
-        d.a_ones_row, d.a_mode = spc.a_ones_row, spc.a_mode
-        d.b_src, d.b_row, d.b_col, d.b_mode = b_src.data_ptr(), tabs["b_row"].data_ptr(), tabs["b_col"].data_ptr(), spc.b_mode
-        d.out, d.out_row, d.out_col = out.data_ptr(), tabs["out_row"].data_ptr(), tabs["out_col"].data_ptr()
-        d.bias = bias.data_ptr() if bias is not None else None
-        d.relu_pre_cols = relu_pre_cols
-        d.gate = gate.data_ptr() if gate is not None else None
-        d.gate_row = gate_tabs[0].data_ptr() if gate_tabs else None
-        d.gate_col = gate_tabs[1].data_ptr() if gate_tabs else None
-        d.gate_col0, d.gate_first = gate_col0, int(gate_first)
-        d.addend = addend.data_ptr() if addend is not None else None
-        d.add_row = add_tabs[0].data_ptr() if add_tabs else None
-        d.add_col = add_tabs[1].data_ptr() if add_tabs else None
-        d.relu_post, d.atomic_out = int(relu_post), int(atomic)
-        d.ones_row_out = ones_out.data_ptr() if ones_out is not None else None
-        if tile_n == 0 and split_k == 1:
-            tile_n = _auto_tile_n(spc.M, spc.N, isinstance(self, TGemm), eng.prec == L.PREC_TF32X3)
-        d.split_k, d.tile_n = split_k, tile_n
-        d.out_vec = spc.out_vec if out_vec is None else out_vec
-        counter = None
-        if finish:                         # split-K finished in-kernel by the last CTA of each output tile (offk.h)
-            bn = tile_n if tile_n else (256 if spc.N > 256 else (spc.N + 15) // 16 * 16)
-            counter = torch.zeros(math.ceil(spc.M / 128) * math.ceil(spc.N / bn), dtype=torch.int32, device=eng.device)
-            d.finish_counter = counter.data_ptr()
-        if aux is not None:                # (aux_out, aux_row table or None, aux_col0, aux_addend or None)
-            d.aux_out = aux[0].data_ptr()
-            d.aux_row = aux[1].data_ptr() if aux[1] is not None else None
-            d.aux_col0 = aux[2]
-            d.aux_addend = aux[3].data_ptr() if aux[3] is not None else None
-        T.check_modes(spc)
-        self.desc = d
-        self._keep = (tabs, a_src, b_src, out, bias, gate, gate_tabs, addend, add_tabs, ones_out, counter, aux)
-        self.flops = 2.0 * spc.M * spc.N * spc.K
-        self.launches = [name]
-        self.reads = [a_src, b_src, addend, gate, bias, aux[3] if aux else None]
-        self.writes = [out, ones_out, aux[0] if aux else None]
-        self.lane = 0
-
-    def set_a_src(self, ptr):
-        self.desc.a_src = ptr
-
-    def __call__(self, stream):
-        L.check(self.eng.lib.offk_gather_gemm(C.byref(self.desc), self.eng.prec, stream), self.name)
-
-
-class TGemm(Gemm):
-    """A forward conv / FC on a channels-last input as ONE TMA-fed launch (offk_tma_gemm): A through a dense 2-D
-    tensor map (1x1, stride 1) or TMA im2col mode (KxK), B = the [cout, K] weight matrix.  Same epilogue fields and
-    output tables as the gather-GEMM it stands in for."""
-
-    @staticmethod
-    def eligible(geom: T.ConvGeom, x_layout="nhwc") -> bool:
-        if x_layout == "nchw":      # the taps, read in place as an MN-major operand: 1x1 conv over whole frames
-            return (T._is1x1(geom) and geom.cin % 32 == 0 and geom.x_coff == 0 and geom.x_ctot == geom.cin
-                    and (geom.hin * geom.win) % 4 == 0)
-        return geom.cin % 32 == 0 and geom.x_ctot % 4 == 0 and geom.x_coff % 4 == 0 and geom.kdim % 4 == 0
-
-    @staticmethod
-    def wgrad_eligible(geom: T.ConvGeom, x_layout="nhwc") -> bool:
-        """Weight gradient with both operands TMA-fed: A = im2col(x)^T (channels-last) or the NCHW tap, B = dY."""
-        y_ok = geom.y_ctot % 4 == 0 and geom.y_coff % 4 == 0 and geom.cout % 4 == 0
-        if x_layout == "nchw":
-            return (y_ok and T._is1x1(geom) and geom.x_coff == 0 and geom.x_ctot == geom.cin
-                    and (geom.hin * geom.win) % 4 == 0)
-        return y_ok and geom.cin % 32 == 0 and geom.x_ctot % 4 == 0 and geom.x_coff % 4 == 0
-
-    def __init__(self, eng, spc, key, geom: T.ConvGeom, x_layout="nhwc", wgrad=False, bk=0, **kw):
-        super().__init__(eng, spc, key, **kw)
-        t = L.OffkTGemm()
-        C.memmove(C.byref(t.g), C.byref(self.desc), C.sizeof(L.OffkGemm))
-        one = geom.kh == 1 and geom.kw == 1 and geom.stride == 1 and geom.pad == 0
-        if wgrad:
-            t.a_kind = L.TMA_A_NCHW_T if x_layout == "nchw" else L.TMA_A_IM2COL_T
-        elif x_layout == "nchw":
-            t.a_kind = L.TMA_A_NCHW
-        elif one:
-            t.a_kind, t.lda = L.TMA_A_DENSE, geom.x_ctot
-            t.g.a_src = kw["a_src"].data_ptr() + 4 * geom.x_coff
-        else:
-            t.a_kind = L.TMA_A_IM2COL
-        t.a_coff = geom.x_coff
-        if not wgrad and spc.out_vec == 1 and spc.M > 1:
-            # linear output rows: a plain epilogue may leave through TMA tile stores (offk.h: out_ld)
-            r = np.asarray(spc.out_row, dtype=np.int64)
-            ld = int(r[1] - r[0])
-            if ld > 0 and r[0] == 0 and np.array_equal(r, np.arange(spc.M, dtype=np.int64) * ld):
-                t.out_ld, t.out_c0 = ld, int(spc.out_col[0])
-        t.precision = eng.prec
-        t.bk = bk if (wgrad and x_layout != "nchw") else 0
-        if eng.presplit and not wgrad:
-            # B is a weight matrix inside one of the owner's weight buffers: its residuals sit at the same offset of the
-            # twin buffer
-            bp = kw["b_src"].data_ptr()
-            for hi, lo in eng.lo_twins:
-                if hi.data_ptr() <= bp < hi.data_ptr() + hi.numel() * 4:
-                    t.b_lo_delta = (lo.data_ptr() - hi.data_ptr()) // 4
-                    self.reads.append(lo)
-        t.n_img, t.hin, t.win, t.ctot, t.cin = geom.n_img, geom.hin, geom.win, geom.x_ctot, geom.cin
-        t.kh, t.kw, t.stride, t.pad, t.hout, t.wout = geom.kh, geom.kw, geom.stride, geom.pad, geom.hout, geom.wout
-        if isinstance(geom, _FreeGeom):
-            t.geom_flags, t.pad_w = L.TGEMM_FREE_GEOM, geom.pad_w
-        if wgrad:                         # B = dY[pixel, cout slice], row-major
-            t.b_kind, t.ldb = L.TMA_B_DENSE_T, geom.y_ctot
-            t.g.b_src = kw["b_src"].data_ptr() + 4 * geom.y_coff
-        else:
-            t.b_kind, t.ldb = L.TMA_B_DENSE, geom.kdim
-        self.tdesc = t
-        self._by_src = {}                 # a_src pointer -> prepared descriptor (the two tap sets alternate)
-
-    def set_a_src(self, ptr):
-        if self.tdesc.g.a_src == ptr:
-            return
-        self._by_src[self.tdesc.g.a_src] = self.tdesc
-        t = self._by_src.get(ptr)
-        if t is None:
-            t = L.OffkTGemm()
-            C.memmove(C.byref(t), C.byref(self.tdesc), C.sizeof(L.OffkTGemm))
-            t.g.a_src, t.prepared = ptr, 0
-        self.tdesc = t
-        self.desc.a_src = ptr
-
-    def __call__(self, stream):
-        lib = self.eng.lib
-        if not self.tdesc.prepared:                                  # tensor maps are encoded on first use (needs a driver)
-            L.check(lib.offk_tma_gemm_prepare(C.byref(self.tdesc)), self.name + " (prepare)")
-        L.check(lib.offk_tma_gemm(C.byref(self.tdesc), stream), self.name)
-
-
-class GemmOwner:
-    """What a bound Gemm / TGemm needs from the plan that owns it: ``lib``, ``device``, ``prec``, ``presplit`` (3xTF32 with
-    the weights' tf32 residuals in twin buffers), ``lo_twins`` ([(weights, residuals)] buffer pairs for b_lo_delta), the
-    table cache and ``flops_fwd``; and the forward-conv launch policy (``_conv_fwd``).  OFFEngine and the BN-Inception
-    extractor plan (extractor.py) are the two owners."""
-
-    def _tables(self, key, spc: T.GemmSpec):
-        if key not in self._tab_cache:
-            dev = self.device
-            self._tab_cache[key] = {k: torch.from_numpy(v).to(dev) for k, v in T.padded_tables(spc).items()}
-        return self._tab_cache[key]
-
-    def _conv_fwd(self, name, x, y, geom, w, b, *, relu=False, relu_cols=None, addend=None,
-                  add_tabs=None, relu_post=False, x_layout="nhwc", no_split=False, aux=None):
-        """One TMA-fed launch (TGemm); a geometry without a TMA-fed form is an error.
-        aux = (aux_out, aux_row table | None, aux_col0, aux_addend | None): second output max(v + aux_addend, 0) written by
-        the GEMM epilogue (offk.h); only honoured with the float4 epilogue (out_vec) -- the returned step has
-        .aux_fused = True then."""
-        spc = T.conv_fwd_spec(geom, x_layout, "nhwc")
-        m_tiles, kb = math.ceil(spc.M / 128), math.ceil(spc.K / 32)
-        n_tiles = max(1, math.ceil(spc.N / 256))
-        split = 1
-        if addend is None and m_tiles * n_tiles < 200 and kb >= 32:
-            # split-K factor: minimise rounds x K-blocks per CTA, rounds = ceil(CTAs / resident CTA slots) (two CTAs per SM in
-            # the tf32 mode, one in the 3xTF32 mode whose stages are twice as large); ties go to the smaller factor.
-            # 147 tiles: 2 splits = 294 CTAs = one round (3 splits were 1.49 rounds at 31 % tensor-pipe activity).
-            slots = _SM_TARGET * (1 if self.prec == L.PREC_TF32X3 else 2)
-            tiles = m_tiles * n_tiles
-            split = min(range(1, max(1, kb // 8) + 1),
-                        key=lambda s_: (math.ceil(tiles * s_ / slots) * math.ceil(kb / s_) * (1 if tiles * s_ >= 0.9 * _SM_TARGET else 4), s_))
-        cols = (geom.cout if relu else 0) if relu_cols is None else relu_cols
-        if not TGemm.eligible(geom, x_layout):
-            raise ValueError(f"{name}: this conv geometry has no TMA-fed form (TGemm.eligible)")
-        mk = lambda *a, **k: TGemm(*a, geom=geom, x_layout=x_layout, **k)
-        if x_layout == "nchw" or no_split:
-            split = 1                     # per-frame M tiles already fill the machine (N * ceil(hw/128) CTAs)
-        fuse = spc.out_vec
-        # in-kernel finishing pays when there are enough output tiles for the finishing CTAs to keep the machine busy
-        # (motion_conv_trans_28: 147 tiles, same time as the bare split-K GEMM, bias_act and ReLU copy for free); with the
-        # 37-tile 7x7 layers the fences + a finishing pass by 37 CTAs cost 9-27 us more than a separate full-grid bias_act
-        # pass (measured, profiles/launches_tf32_r02g*.txt), so those keep the two-kernel form
-        fin_ok = fuse and m_tiles * n_tiles >= _FINISH_MIN_TILES
-        if split > 1 and fin_ok:
-            # split-K partial tiles are added into the zeroed output; the last CTA of each tile applies bias / ReLU (and
-            # writes the second output) in place: no separate bias_act pass
-            g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, bias=b, relu_pre_cols=cols,
-                   split_k=split, name=name, finish=True, aux=aux)
-
-            def run(stream, g=g, y=y):
-                L.check(self.lib.offk_fill_zero(_ptr(y), y.numel(), stream), name + ".zero")
-                g(stream)
-            assert geom.y_coff == 0 and geom.y_ctot == geom.cout
-            self.flops_fwd += g.flops
-            run.name, run.flops, run.gemm, run.aux_fused = name, g.flops, g, aux is not None
-            run.launches = [name + ".zero", name + ".splitk"]
-            run.reads, run.writes, run.lane = g.reads, g.writes, 0
-            return run
-        if split > 1:
-            g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, split_k=split, name=name)
-            hw = geom.hout * geom.wout
-
-            def run(stream, g=g, y=y, b=b, geom=geom, hw=hw, cols=cols):
-                L.check(self.lib.offk_fill_zero(_ptr(y), y.numel(), stream), name + ".zero")
-                g(stream)
-                L.check(self.lib.offk_bias_act(_ptr(y), _ptr(b), geom.n_img, geom.cout, hw, geom.y_ctot, geom.y_coff,
-                                               cols, stream), name + ".bias_act")
-            assert geom.y_coff == 0 and geom.y_ctot == geom.cout
-            self.flops_fwd += g.flops
-            run._split = True
-            run.name = name
-            run.flops = g.flops
-            run.launches = [name + ".zero", name + ".splitk", name + ".bias_act"]
-            run.gemm = g
-            run.reads, run.writes, run.lane = g.reads, g.writes, 0
-            return run
-        # nchw TMA: one N tile (re-reading the tap per N tile would multiply the HBM traffic of an HBM-bound GEMM)
-        tn = (spc.N + 15) // 16 * 16 if (x_layout == "nchw" and spc.N <= 256) else 0
-        g = mk(self, spc, ("fwd", x_layout, _gkey(geom)), a_src=x, b_src=w, out=y, bias=b, relu_pre_cols=cols,
-               addend=addend, add_tabs=add_tabs, relu_post=relu_post, tile_n=tn, name=name, aux=aux if fuse else None)
-        g.aux_fused = bool(fuse and aux is not None)
-        self.flops_fwd += g.flops
-        return g
-
-
-class OFFEngine(GemmOwner):
+class OFFEngine(LaunchPlan):
     """Plan + buffers for one (batch, length) shape on one GPU.
 
     tap_layout: 'nchw' (the reference's layout) or 'channels_last': both tap sets are [N, C, S, S] tensors in
@@ -316,30 +49,20 @@ class OFFEngine(GemmOwner):
         if tap_grads and tap_layout == "channels_last":
             # the channels-last taps come from the frozen fused extractor (train_off.py:39-46): nothing consumes their gradient
             raise ValueError("tap_grads=True needs tap_layout='nchw': channels-last taps come from the frozen extractor")
+        super().__init__(device, precision)
         self.tap_layout = tap_layout
-        self.lib = L.lib()
         self.B, self.Lseg, self.variant = batch, length, variant
         self.N, self.P = batch * length, batch * (length - 1)
-        self.device = torch.device(device)
-        self.prec = {"fp32": L.PREC_TF32X3, "tf32": L.PREC_TF32}[precision]
         self.precision = precision
         self.index_mode = {"reference_flat": L.INDEX_REFERENCE_FLAT, "aligned": L.INDEX_ALIGNED}[index_mode]
         self.consensus = (variant != "rgb") if consensus is None else bool(consensus)
         self.tap_grads = tap_grads
         self.single_stream = False       # True: issue every lane on the caller's stream (profiling / debugging)
-        self._tab_cache = {}
-        self._keep = []
         self.generation = 0
 
         # ---- parameters: one flat buffer, reference-named views
         self.layout, self.n_flat = S.flat_layout(variant)
-        # fp32 (3xTF32) mode: the tf32 residuals of the weights are produced once per step into a twin buffer directly behind
-        # the parameters, so that the GEMMs receive both weight tiles by TMA (offk.h: b_lo_delta) instead of splitting them in
-        # shared memory in every CTA and K-block
-        self.presplit = self.prec == L.PREC_TF32X3
-        self._params_all = torch.zeros(self.n_flat * (2 if self.presplit else 1), device=self.device)
-        self.params_flat = self._params_all[:self.n_flat]
-        self.params_lo = self._params_all[self.n_flat:] if self.presplit else None
+        self.params_flat, self.params_lo = self._weights(self.n_flat)
         self.grads_flat = torch.zeros(self.n_flat, device=self.device)
         self.params = OrderedDict((n, self._view(self.params_flat, n)) for n in S.param_shapes(variant))
         self.grads = OrderedDict((n, self._view(self.grads_flat, n)) for n in S.param_shapes(variant))
@@ -459,11 +182,7 @@ class OFFEngine(GemmOwner):
                         views.append(("wd", (name, a, b), off, (cin, sub.size // cin)))
                         off += sub.size
         self.wc_idx = torch.from_numpy(np.concatenate(idx).astype(np.int32)).to(self.device)
-        off = (off + 3) // 4 * 4
-        self._wc_all = torch.zeros(off * (2 if self.presplit else 1), device=self.device)
-        self.wc_flat = self._wc_all[:off]
-        self.wc_lo = self._wc_all[off:] if self.presplit else None
-        self.lo_twins = [(self.params_flat, self.params_lo), (self.wc_flat, self.wc_lo)]
+        self.wc_flat, self.wc_lo = self._weights((off + 3) // 4 * 4)
         for kind, name, o, shape in views:
             getattr(self, kind)[name] = self.wc_flat[o:o + int(np.prod(shape))].view(shape)
         off = 0
@@ -477,7 +196,6 @@ class OFFEngine(GemmOwner):
         self.masks = None
         self.seed_state = torch.zeros(1, dtype=torch.int64, device=self.device)   # per-step dropout seed (device word)
         self._graphs = {}                # (pass, tap set, dropout mode) -> torch.cuda.CUDAGraph
-        self._cap_stream = None
 
     # ------------------------------------------------------------------ plan
     def _conv_wgrad(self, name, x, dy, geom, dw, db, *, x_layout="nhwc", tap_copy=False):
@@ -528,7 +246,7 @@ class OFFEngine(GemmOwner):
             if addend is not None and add_geom is not None:
                 # addend lives in a differently-shaped buffer: tables of the same logical (img, c, y, x) element
                 aspec = T.conv_dgrad_specs(add_geom, "nhwc", "nhwc", "nhwc")[i]
-                t = self._tables(("dgrad", "nhwc", _gkey(add_geom), i), aspec)
+                t = self._tables(("dgrad", "nhwc", _gkey(add_geom), i), aspec, _OUT_TABLES)
                 add_tabs = (t["out_row"], t["out_col"])
             kw_ = dict(a_src=dy, b_src=w, out=dx, gate=gate, gate_col0=gate_col0, gate_first=gate_first, addend=addend,
                        add_tabs=add_tabs, name=f"{name}.dgrad{i}")
@@ -564,7 +282,6 @@ class OFFEngine(GemmOwner):
     def _build(self):
         P, N, B, Lg = self.P, self.N, self.B, self.Lseg
         bf, pr, gr = self.buf, self.params, self.grads
-        self.flops_fwd = self.flops_bwd = 0.0
         fwd, bwd_stage = [], []
         lib = self.lib
 
@@ -598,13 +315,13 @@ class OFFEngine(GemmOwner):
                 fwd.append(_nm(kt, "tapT_" + tag, writes=[tapT], lane=fl))
             x_cl = self.taps[tag] if cl else (tapT if via_copy else None)
             if x_cl is not None:
-                k1 = self._conv_fwd("unit_" + tag, x_cl, gd, geom, self._unit_w(self.params_flat, tag),
-                                    self._unit_b(self.params_flat, tag), relu_cols=S.GEN_C, x_layout="nhwc", no_split=True)
+                k1, = self._conv_fwd("unit_" + tag, x_cl, gd, geom, self._unit_w(self.params_flat, tag),
+                                     self._unit_b(self.params_flat, tag), relu_cols=S.GEN_C, x_layout="nhwc", no_split=True)
                 if cl:
                     self._tap_users[tag].append(getattr(k1, "gemm", k1))
             else:
-                k1 = self._conv_fwd("unit_" + tag, self.taps[tag], gd, geom, self._unit_w(self.params_flat, tag),
-                                    self._unit_b(self.params_flat, tag), relu_cols=S.GEN_C, x_layout="nchw")
+                k1, = self._conv_fwd("unit_" + tag, self.taps[tag], gd, geom, self._unit_w(self.params_flat, tag),
+                                     self._unit_b(self.params_flat, tag), relu_cols=S.GEN_C, x_layout="nchw")
                 self._tap_users[tag].append(getattr(k1, "gemm", k1))
             fwd.append(_on(k1, fl))
             # K2 / K3 descriptors: fused spatial stencil + temporal difference + dropout + cat, into the stage buffer
@@ -688,18 +405,13 @@ class OFFEngine(GemmOwner):
                   x_ctot=0, x_coff=0, y_ctot=0, y_coff=0, lane=0, aux=None):
             """forward conv; returns geom for the gradient wiring."""
             geom = geom_of(name, P, s_in, x_ctot, x_coff, y_ctot, y_coff)
-            fwd.append(_on(self._conv_fwd(name, x, y, geom, W(name), Bv(name), relu=relu, addend=addend,
-                                          relu_post=relu_post, aux=aux), lane))
+            fwd.extend(_on(st, lane) for st in self._conv_fwd(name, x, y, geom, W(name), Bv(name), relu=relu, addend=addend,
+                                                              relu_post=relu_post, aux=aux))
             return geom
 
         # ---- resolution 28 (RGB_OFF.py:655-685)
-        # pre-ReLU output kept for the branch (:665); its ReLU'd copy (:658) is the epilogue's second output
-        g_t28 = layer("motion_conv_trans_28", bf["F28"], bf["t28"], 28, aux=(bf["t28r"], None, 0, None))
-        if not getattr(fwd[-1], "aux_fused", False):
-            n28 = bf["t28"].numel()
-            fwd.append(_nm(lambda stream: L.check(lib.offk_relu_gate(_ptr(bf["t28"]), _ptr(bf["t28"]), n28, _ptr(bf["t28r"]),
-                                                                      stream), "relu_t28"), "relu_t28",
-                           reads=[bf["t28"]], writes=[bf["t28r"]]))
+        # pre-ReLU output kept for the branch (:665); its ReLU'd copy (:658) is the second output
+        g_t28 = layer("motion_conv_trans_28", bf["F28"], bf["t28"], 28, aux=(bf["t28r"], 64, 0, None, "relu_t28"))
         g_c1a = layer("motion_conv1_trans_28a", bf["t28r"], bf["h1_28a"], 14, relu=True)
         g_c2a = layer("motion_conv2_trans_28a", bf["h1_28a"], bf["h2_28a"], 14, relu=True)
         g_bra = layer("motion_conv_branch_28a", bf["t28"], bf["br28"], 14, lane=2)
@@ -713,8 +425,8 @@ class OFFEngine(GemmOwner):
         g_c3c = geom_of("motion_conv3_trans_28c", P, 14, y_ctot=1056, y_coff=800)
         g_s28b_as_f14 = T.ConvGeom(P, 256, 14, 14, 256, y_ctot=256)  # tables for the s28b addend (plain [P,14,14,256])
         spc_add = T.conv_fwd_spec(g_s28b_as_f14, "nhwc", "nhwc")
-        tabs_add = self._tables(("fwd", "nhwc", _gkey(g_s28b_as_f14)), spc_add)
-        fwd.append(self._conv_fwd("motion_conv3_trans_28c", bf["h2_28c"], bf["F14"], g_c3c,
+        tabs_add = self._tables(("fwd", "nhwc", _gkey(g_s28b_as_f14)), spc_add, _OUT_TABLES)
+        fwd.extend(self._conv_fwd("motion_conv3_trans_28c", bf["h2_28c"], bf["F14"], g_c3c,
                                   W("motion_conv3_trans_28c"), Bv("motion_conv3_trans_28c"), addend=bf["s28b"],
                                   add_tabs=(tabs_add["out_row"], tabs_add["out_col"]), relu_post=True))
 
@@ -727,13 +439,9 @@ class OFFEngine(GemmOwner):
         g_14b1 = layer("motion_conv1_trans_14b", bf["s14a"], bf["h1_14b"], 7, relu=True)
         g_14b2 = layer("motion_conv2_trans_14b", bf["h1_14b"], bf["h2_14b"], 7, relu=True)
         # 3x3 + ReLU (:316,:778), kept for the backward gate; sum_14b = relu(s14a + h3_14b) -> 7-stage fusion buffer channels
-        # [320,832) (:779-780, cat :832) is the same epilogue's second output
-        g_f7slice = T.ConvGeom(P, 512, 7, 7, 512, y_ctot=832, y_coff=320)
-        tabs_f7 = self._tables(("fwd", "nhwc", _gkey(g_f7slice)), T.conv_fwd_spec(g_f7slice, "nhwc", "nhwc"))
+        # [320,832) (:779-780, cat :832) is the second output
         g_14b3 = layer("motion_conv3_trans_14b", bf["h2_14b"], bf["h3_14b"], 7, relu=True,
-                       aux=(bf["F7"], tabs_f7["out_row"], 0, bf["s14a"]))      # the row table carries the channel offset 320
-        if not getattr(fwd[-1], "aux_fused", False):
-            fwd.append(self._add_into_slice(bf["s14a"], bf["h3_14b"], bf["F7"], 832, 320, 512, 49))
+                       aux=(bf["F7"], 832, 320, bf["s14a"], "sum_14b"))
 
         # ---- heads 28 / 14 (RGB_OFF.py:783-793)
         fwd.append(_nm(lambda stream: L.check(lib.offk_pool3_nhwc(_ptr(bf["F14"]), P, 14, 14, 1056, 800, 256, 2, 0, L.POOL_MAX,
@@ -857,8 +565,6 @@ class OFFEngine(GemmOwner):
         post = [_nm(lambda stream: L.check(lib.offk_permute_weight_batch(len(kxk), self._unperm, 2, stream), "unpermute"),
                     "unpermute_kxk_weight_grads", reads=[self.dwp_flat], writes=[gr[n + ".weight"] for n, _, _, _ in kxk], lane=1)]
         self.fwd_steps = pre + fwd
-        # kernels of liboffk launched per pass (cudaMemsetAsync zero-fills are not kernels)
-        count = lambda steps: sum(len([n for n in _names(st) if not _is_memset(n)]) for st in steps)
         # gradient accumulators start from zero (split-K / atomic accumulation); grads_flat only when asked
         self._zero_grads = True
         gflat, dwflat = self.grads_flat, self.dwp_flat
@@ -870,8 +576,9 @@ class OFFEngine(GemmOwner):
         self.bwd_stage_steps = zero + bwd_stage + post
         self.bwd_unit_steps = bwd_units
         self.bwd_steps = self.bwd_stage_steps + self.bwd_unit_steps
-        self.launches_fwd = count(self.fwd_steps)
-        self.launches_bwd = count(self.bwd_steps)
+        self.steps = self.fwd_steps + self.bwd_steps
+        self.launches_fwd = len(_kernels(self.fwd_steps))
+        self.launches_bwd = len(_kernels(self.bwd_steps))
         # parameters and taps are read-only inside a pass: never a hazard
         ro = [self.params_flat] + [t for ts in self.tap_sets for t in ts.values()]
         if self.variant == "flow":
@@ -889,11 +596,6 @@ class OFFEngine(GemmOwner):
         self.stage_range = (self.unit_range[1], self.n_flat)    # stage convs + FC heads
 
     # ------------------------------------------------------------------ small step factories
-    def _add_into_slice(self, a, b, dst, ctot, coff, c, hw):
-        P, lib = self.P, self.lib
-        return _nm(lambda stream: L.check(lib.offk_add_relu_slice(_ptr(a), _ptr(b), _ptr(dst), ctot, coff, P, c, hw, 1,
-                                                                   stream), "sum_14b"), "sum_14b", reads=[a, b], writes=[dst])
-
     @staticmethod
     def _site_salt(site):
         """Constant 64-bit salt of dropout call site ``site`` (12 per forward, RGB_OFF.py:612..:845): splitmix64(site).
@@ -1026,31 +728,8 @@ class OFFEngine(GemmOwner):
         key = (which, self._tap_set, self.drop_mode)
         g = self._graphs.get(key)
         if g is None:
-            g = self._graphs[key] = self._capture(which)
+            g = self._graphs[key] = self._capture(lambda: self._issue(which))
         g.replay()
-
-    def _capture(self, which):
-        """Capture one pass (all lanes: the side streams fork from and join the capturing stream through the schedule's
-        events, so the graph keeps the multi-stream concurrency of the eager plan)."""
-        main = torch.cuda.current_stream(self.device)
-        if self._cap_stream is None:
-            self._cap_stream = torch.cuda.Stream(device=self.device)
-        cap = self._cap_stream
-        cap.wait_stream(main)
-        with torch.cuda.stream(cap):
-            self._issue(which)          # eager once on this stream: tensor maps encoded, kernel attributes set
-        cap.synchronize()
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g, stream=cap):
-            self._issue(which)
-        main.wait_stream(cap)
-        return g
-
-    def launch_names(self):
-        """One name per device launch of forward() + backward(), in issue order (for annotating ncu launch lists)."""
-        out = [n for st in self.fwd_steps for n in _names(st)]
-        out += [n for st in self.bwd_steps for n in _names(st)]    # (the d_out copies are cudaMemcpyAsync, not kernels)
-        return [n for n in out if not _is_memset(n)]
 
     def backward(self, g7: torch.Tensor, g14: torch.Tensor, zero_grads: bool = True, after_stage=None, after_unit=None,
                  graph: bool = False):
@@ -1099,122 +778,3 @@ class OFFEngine(GemmOwner):
         for s_ in streams[1:]:
             if s_ is not streams[0]:
                 streams[0].wait_stream(s_)
-
-
-def _auto_tile_n(M: int, N: int, tma: bool = False, x3: bool = False) -> int:
-    """N tile of a GEMM launched without split-K; 0 = the kernel's default (widest legal tile).
-    TMA-fed: two CTAs fit an SM and one CTA's epilogue should overlap another's main loop, so aim for >= 2 x 148 CTAs
-    with the widest tile that gets there (re-reading A per N tile is one cheap TMA instruction).
-    Gather-fed: the A gather is the expensive part and is repeated per N tile, so only narrow the tile when the grid
-    would otherwise leave most SMs idle (the 7x7-resolution layers: 37 M tiles)."""
-    mt = math.ceil(M / 128)
-    bn0 = (N + 15) // 16 * 16 if N <= 256 else 256
-    want, enough = (120, 140)
-    if tma:         # (2 x 148 before the MMA issue path was fixed: narrow tiles were issue-bound then; profiles/env_r03t.log)
-        want = enough = _TF32_WANT_CTAS
-    if tma and x3:
-        # 3xTF32: one CTA per SM, and every extra N tile repeats the A tile AND its residual pass (motion_conv_trans_28,
-        # 147 x 1 tiles of 64: two tiles of 32 took 586 us against 371 us; unit_5a, 56 M tiles: five tiles of 32 columns
-        # 38 us against ~20 for one of 160).  Only the 37-tile 7x7 layers are narrowed (sweep: profiles/env_r03s.log)
-        want = enough = _X3_WANT_CTAS
-    if mt * math.ceil(N / bn0) >= want:
-        return 0
-    best = 0
-    for bn in (128, 64, 32):
-        if bn < bn0 and N % bn == 0:
-            best = bn
-            if mt * (N // bn) >= enough:
-                break
-    return best
-
-
-def _is_memset(name):
-    return name.endswith(".zero") or name.startswith("zero ")
-
-
-def _nm(fn, name, reads=(), writes=(), lane=0):
-    """Annotate a plan step: launch name, the buffers it reads / writes (for cross-stream hazard analysis), its lane."""
-    fn.launches = [name]
-    fn.reads, fn.writes, fn.lane = list(reads), list(writes), lane
-    return fn
-
-
-def _on(step, lane):
-    step.lane = lane
-    return step
-
-
-def _span(t):
-    return (t.data_ptr(), t.data_ptr() + t.numel() * t.element_size())
-
-
-class Schedule:
-    """A fixed list of steps spread over a few CUDA streams ("lanes").  Steps on one lane run in issue order; a step
-    that touches a buffer last written (or still being read) by a step on another lane waits on an event recorded
-    behind that step.  The hazards (RAW / WAW / WAR on byte ranges) are derived from the steps' declared reads and
-    writes, so lane assignment is purely a performance choice: any assignment is correct."""
-
-    def __init__(self, steps, ignore=()):
-        self.steps = list(steps)
-        n = len(self.steps)
-        self.n_lanes = 1 + max((getattr(st, "lane", 0) for st in self.steps), default=0)
-        ign = [_span(t) for t in ignore]
-
-        def spans(ts):
-            out = []
-            for t in ts:
-                if t is None:
-                    continue
-                sp = _span(t)
-                if any(lo <= sp[0] and sp[1] <= hi for lo, hi in ign):
-                    continue                      # read-only inputs (parameters, taps): never a hazard
-                out.append(sp)
-            return out
-
-        rd = [spans(getattr(st, "reads", ())) for st in self.steps]
-        wr = [spans(getattr(st, "writes", ())) for st in self.steps]
-        hit = lambda A, B: any(a[0] < b[1] and b[0] < a[1] for a in A for b in B)
-        lanes = [getattr(st, "lane", 0) for st in self.steps]
-        self.lanes = lanes
-        covered = [[-1] * self.n_lanes for _ in range(self.n_lanes)]   # covered[a][b]: latest step of lane b that a awaited
-        self.waits = [[] for _ in range(n)]
-        record = set()
-        for i in range(n):
-            need = {}
-            for j in range(i):
-                if lanes[j] == lanes[i] or j <= covered[lanes[i]][lanes[j]]:
-                    continue
-                if hit(wr[j], rd[i]) or hit(wr[j], wr[i]) or hit(rd[j], wr[i]):
-                    need[lanes[j]] = j
-            for lane_j, j in need.items():
-                self.waits[i].append(j)
-                covered[lanes[i]][lane_j] = j
-                record.add(j)
-        self.record = record
-        self.events = {j: torch.cuda.Event() for j in record}
-
-    def run(self, streams, lo=0, hi=None, on_step=None):
-        """Issue steps [lo, hi) on ``streams`` (torch.cuda.Stream per lane; lane 0 = the caller's stream).
-        ``on_step(step, stream)`` is called after each step has been issued."""
-        hi = len(self.steps) if hi is None else hi
-        handles = [C.c_void_p(st.cuda_stream) for st in streams]
-        for i in range(lo, hi):
-            lane = self.lanes[i]
-            for j in self.waits[i]:
-                streams[lane].wait_event(self.events[j])
-            self.steps[i](handles[lane])
-            if i in self.record:
-                self.events[i].record(streams[lane])
-            if on_step is not None:
-                on_step(self.steps[i], streams[lane])
-
-
-def _names(step):
-    ls = getattr(step, "launches", None)
-    if ls is not None:
-        return list(ls)
-    return [getattr(step, "name", None) or getattr(step, "__name__", "step")]
-
-
-def _gkey(g: T.ConvGeom):
-    return (g.n_img, g.cin, g.hin, g.win, g.cout, g.kh, g.kw, g.stride, g.pad, g.x_ctot, g.x_coff, g.y_ctot, g.y_coff)

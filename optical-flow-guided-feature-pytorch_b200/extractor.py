@@ -7,7 +7,7 @@ for a fixed number of frames.
   flat buffer (plus their tf32 residuals behind it in the fp32 mode, as in the OFF engine).  The fold is redone before a
   forward whenever a parameter or buffer of the module changed since the last one (``load_state_dict``, an optimizer, ...).
 * The image batch is converted to channels-last with 4 (RGB) or 12 (flow) channels, so the 7x7 stem is a gather-fed GEMM
-  with 16-byte channel groups; every other conv is one TMA-fed GEMM (``engine.TGemm``) with bias + ReLU in its epilogue,
+  with 16-byte channel groups; every other conv is one TMA-fed GEMM (``plan.TGemm``) with bias + ReLU in its epilogue,
   writing its channel slice of the module's channels-last output: the Inception concatenations cost nothing.
 * The nine tap modules write straight into the tap buffers of the OFF engine the extractor is paired with (its first input
   set, channels-last), so the OFF forward reads them in place.
@@ -27,7 +27,7 @@ import torch
 from . import _lib as L
 from . import tables as T
 from .backbone import BNInceptionBackbone, TAPS, _NORMAL, _ORDER, _REDUCE
-from .engine import Gemm, GemmOwner, Schedule, _nm, _ptr
+from .plan import Gemm, LaunchPlan, Schedule, _nm, _ptr
 
 IMG = 224                                      # input resolution of the TSN BN-Inception (RGB_OFF.py:362)
 
@@ -42,23 +42,15 @@ def _module_channels(tag):
     return cin, n3 + d + cin, size, size // 2
 
 
-class ExtractorPlan(GemmOwner):
+class ExtractorPlan(LaunchPlan):
     """Buffers, folded weights and launch list of one ``FusedBNInception`` forward over ``n_frames`` images."""
 
     def __init__(self, net: BNInceptionBackbone, n_frames: int, in_channels: int, num_classes: int, precision: str,
                  device, taps=None):
-        self.lib = L.lib()
-        self.device = torch.device(device)
-        if self.device.type == "cuda" and self.device.index is None:
-            # "cuda" means the current device; tensors report it with its index ("cuda:0"), which the checks compare against
-            self.device = torch.device("cuda", torch.cuda.current_device())
+        super().__init__(device, precision)
         self.N = n_frames
         self.cin, self.c_pad = in_channels, (in_channels + 3) // 4 * 4
         self.num_classes = num_classes
-        self.prec = {"fp32": L.PREC_TF32X3, "tf32": L.PREC_TF32}[precision]
-        self.presplit = self.prec == L.PREC_TF32X3
-        self._tab_cache = {}
-        self.flops_fwd = 0.0
         N, dev = n_frames, self.device
 
         # ---- folded weights: name -> (offset, cout, kh, kw, cin of the weight rows), OHWI; biases in their own buffer
@@ -75,11 +67,7 @@ class ExtractorPlan(GemmOwner):
         self.fc_off, self.fc_boff = off, boff
         off += (num_classes * 1024 + 3) // 4 * 4
         boff += (num_classes + 3) // 4 * 4
-        # fp32 mode: the tf32 residuals of the weights directly behind them (offk.h: b_lo_delta)
-        self._w_all = torch.zeros(off * (2 if self.presplit else 1), device=dev)
-        self.w_flat = self._w_all[:off]
-        self.w_lo = self._w_all[off:] if self.presplit else None
-        self.lo_twins = [(self.w_flat, self.w_lo)]
+        self.w_flat, self.w_lo = self._weights(off)
         self.b_flat = torch.zeros(boff, device=dev)
         self.folded_key = None
 
@@ -132,8 +120,7 @@ class ExtractorPlan(GemmOwner):
         geom = T.ConvGeom(self.N, cin, s_in, s_in, cout, k, k, conv.stride[0], conv.padding[0], y_ctot=y_ctot, y_coff=y_coff)
         w, b = self._w(name)
         # split-K accumulates into a zeroed buffer of its own; a channel slice of a concatenation is written once
-        step = self._conv_fwd(name, x, y, geom, w, b, relu=True, no_split=geom.y_ctot != cout)
-        self.steps.append(step)
+        self.steps += self._conv_fwd(name, x, y, geom, w, b, relu=True, no_split=geom.y_ctot != cout)
         return geom
 
     def _pool(self, name, x, s_in, c, stride, pad, kind, y, y_ctot, y_coff):
@@ -202,16 +189,11 @@ class ExtractorPlan(GemmOwner):
         gfc = T.ConvGeom(N, 1024, 1, 1, self.num_classes)
         wfc = self.w_flat[self.fc_off:self.fc_off + self.num_classes * 1024].view(self.num_classes, 1024)
         bfc = self.b_flat[self.fc_boff:self.fc_boff + self.num_classes]
-        self.steps.append(self._conv_fwd("last_linear", pooled, bf["score"], gfc, wfc, bfc, no_split=True))
+        self.steps += self._conv_fwd("last_linear", pooled, bf["score"], gfc, wfc, bfc, no_split=True)
         # parameters are read-only inside a pass; the image is written by the conversion step only
         self.sched = Schedule(self.steps, ignore=[self.w_flat, self.b_flat] + ([self.w_lo] if self.presplit else []))
         self._graph = None
         self._graph_src = None
-        self._cap_stream = None
-
-    def launch_names(self):
-        return [n for st in self.steps for n in getattr(st, "launches", [getattr(st, "name", "step")])
-                if not n.endswith(".zero")]
 
     # ------------------------------------------------------------------ weights
     @torch.no_grad()
@@ -235,27 +217,18 @@ class ExtractorPlan(GemmOwner):
                                                 C.c_void_p(main.cuda_stream)), "extractor weight residuals")
 
     # ------------------------------------------------------------------ run
+    def _issue(self):
+        self.sched.run([torch.cuda.current_stream(self.device)])
+
     def run(self, x, graph=False):
-        main = torch.cuda.current_stream(self.device)
         if not graph:
             self._src = x
-            self.sched.run([main])
+            self._issue()
             return
         if self._graph is None:
             self._graph_src = torch.empty_like(x)
             self._src = self._graph_src
-            if self._cap_stream is None:
-                self._cap_stream = torch.cuda.Stream(device=self.device)
-            cap = self._cap_stream
-            cap.wait_stream(main)
-            with torch.cuda.stream(cap):
-                self.sched.run([cap])     # eager once on this stream: tensor maps encoded, kernel attributes set
-            cap.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g, stream=cap):
-                self.sched.run([cap])
-            main.wait_stream(cap)
-            self._graph = g
+            self._graph = self._capture(self._issue)
         if x.data_ptr() != self._graph_src.data_ptr():
             self._graph_src.copy_(x)
         self._graph.replay()

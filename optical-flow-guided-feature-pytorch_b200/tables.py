@@ -270,12 +270,18 @@ def emulate_dgrad_class(g: ConvGeom, spec: GemmSpec, dy_nhwc: np.ndarray, w_oihw
     return out.reshape(-1, g.cin)
 
 
-def check_modes(spec: GemmSpec):
-    """Assert the promises behind the vector load / store modes (contiguity, alignment, shared validity)."""
+def check_modes(spec: GemmSpec, gather: bool = True):
+    """Assert the promises behind the vector store mode and, for a gather-fed launch (``gather``), behind the vector load
+    modes (contiguity, alignment, shared validity)."""
     def quads(tab, n):
         t = tab[: n - n % 4].reshape(-1, 4)
         return t
 
+    if spec.out_vec:
+        assert spec.N % 4 == 0 and (spec.out_col == spec.out_col[0] + np.arange(spec.N)).all()
+        assert spec.out_col[0] % 4 == 0 and (spec.out_row % 4 == 0).all()
+    if not gather:
+        return
     if spec.a_mode == LOAD_VEC_K:
         assert spec.K % 4 == 0
         q = quads(spec.a_col, spec.K)
@@ -298,9 +304,6 @@ def check_modes(spec: GemmSpec):
         assert spec.N % 4 == 0
         q = quads(spec.b_row, spec.N)
         assert (q == q[:, :1] + np.arange(4)).all() and (q[:, 0] % 4 == 0).all() and (spec.b_col % 4 == 0).all()
-    if spec.out_vec:
-        assert spec.N % 4 == 0 and (spec.out_col == spec.out_col[0] + np.arange(spec.N)).all()
-        assert spec.out_col[0] % 4 == 0 and (spec.out_row % 4 == 0).all()
 
 
 NO_BOX = 32767          # a_h / a_w value meaning "every real element is valid"

@@ -34,7 +34,7 @@ def _stock_conv_flops(cin):
 
 @pytest.mark.parametrize("cin", [3, 10])
 def test_fused_extractor_plan_builds_without_a_gpu(cin):
-    from off_b200 import engine as E
+    from off_b200 import plan as PL
     from off_b200.backbone import BNInceptionBackbone
     from off_b200.extractor import FusedBNInception
     n = 6
@@ -47,14 +47,14 @@ def test_fused_extractor_plan_builds_without_a_gpu(cin):
     # launch list: the image conversion, ONE gather-fed stem GEMM, one TMA-fed GEMM per other conv of backbone.py's table,
     # the two stem pools and one pool per Inception module, the global pool and last_linear
     steps = {getattr(st, "name", None) or st.launches[0]: st for st in plan.steps}
-    gathers = [st for st in plan.steps if isinstance(st, E.Gemm) and not isinstance(st, E.TGemm)]
+    gathers = [st for st in plan.steps if isinstance(st, PL.Gemm) and not isinstance(st, PL.TGemm)]
     assert [g.name for g in gathers] == ["conv1_7x7_s2"]
     assert gathers[0].spec.a_mode == gathers[0].spec.b_mode == 2           # LOAD_VEC_K x LOAD_VEC_K
     convs = [name for name, m in stock.named_children() if isinstance(m, torch.nn.Conv2d)]
     assert len(convs) == 69
     for name in convs[1:]:
         st = steps[name]
-        assert isinstance(getattr(st, "gemm", st), E.TGemm), name
+        assert isinstance(getattr(st, "gemm", st), PL.TGemm), name
     pools = [n for n in steps if (n.startswith("inception_") and n.endswith("_pool")) or n in ("pool1", "pool2")]
     assert pools == ["pool1", "pool2"] + [f"inception_{t}_pool" for t in ("3a", "3b", "3c", "4a", "4b", "4c", "4d", "4e",
                                                                            "5a", "5b")]

@@ -411,18 +411,18 @@ def test_builtin_backbone_matches_the_reference_taps(variant):
 
 
 def test_launch_policies_are_wave_aware():
-    """Host-side tile / split-K policies (engine.py): pure functions of the problem shape, pinned here on the shapes whose
+    """Host-side tile / split-K policies (plan.py): pure functions of the problem shape, pinned here on the shapes whose
     measurements motivated them (DESIGN.md 3.2, finding 5)."""
     import off_b200  # noqa: F401
-    from off_b200 import engine as E
+    from off_b200 import plan as PL
     # 3xTF32 (one CTA per SM): a second N tile repeats the A tile and its residual pass -- only the 37-tile 7x7 layers narrow
-    assert E._auto_tile_n(56 * 128, 160, True, True) == 0            # unit_5a: one tile of 160 columns, not five of 32
-    assert E._auto_tile_n(147 * 128, 64, True, True) == 0            # motion_conv_trans_28: 147 x 1, not 147 x 2
-    assert E._auto_tile_n(37 * 128, 256, True, True) == 128          # 7x7 stage: 37 x 2
-    assert E._auto_tile_n(37 * 128, 1024, True, True) == 0           # 37 x 4 tiles of 256 already
+    assert PL._auto_tile_n(56 * 128, 160, True, True) == 0           # unit_5a: one tile of 160 columns, not five of 32
+    assert PL._auto_tile_n(147 * 128, 64, True, True) == 0           # motion_conv_trans_28: 147 x 1, not 147 x 2
+    assert PL._auto_tile_n(37 * 128, 256, True, True) == 128         # 7x7 stage: 37 x 2
+    assert PL._auto_tile_n(37 * 128, 1024, True, True) == 0          # 37 x 4 tiles of 256 already
     # weight gradients: CTAs = tiles x split lands on whole rounds of the resident slots
-    assert E._wgrad_split(3, 3600, 148) == 49                        # unit_3a.wgrad: 147 CTAs, one round (was 3 x 98)
-    assert E._wgrad_split(3, 3600, 296) == 98                        # tf32 mode: two CTAs per SM
-    s = E._wgrad_split(123, 294, 148, 64)                            # motion_conv_trans_28.wgrad, 64-pixel K-blocks
+    assert PL._wgrad_split(3, 3600, 148) == 49                       # unit_3a.wgrad: 147 CTAs, one round (was 3 x 98)
+    assert PL._wgrad_split(3, 3600, 296) == 98                       # tf32 mode: two CTAs per SM
+    s = PL._wgrad_split(123, 294, 148, 64)                           # motion_conv_trans_28.wgrad, 64-pixel K-blocks
     assert 123 * s <= 148 * math.ceil(123 * s / 148) and (148 * math.ceil(123 * s / 148) - 123 * s) < 15
-    assert E._wgrad_split(1, 588, 148) == 147                        # a single-tile 1x1 layer still fills the machine
+    assert PL._wgrad_split(1, 588, 148) == 147                       # a single-tile 1x1 layer still fills the machine

@@ -106,7 +106,7 @@ def from_images(B, Lg, variant, backbone, precision, iters, warmup, dev):
 
 def maxpool28_ab(B, Lg, precision, parent_lib, iters, warmup, rounds, dev):
     """The OFF training step with the maxpool28 launch on either kernel; the rest of the plan is the same object."""
-    from off_b200 import _lib as L, engine as E, spec as S
+    from off_b200 import _lib as L, plan as PL, spec as S
     from off_b200.modules import OFFSubNetwork
     import off_oracle as O
     old = C.CDLL(parent_lib)
@@ -114,13 +114,13 @@ def maxpool28_ab(B, Lg, precision, parent_lib, iters, warmup, rounds, dev):
     old.offk_maxpool3s2_fwd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
     net = OFFSubNetwork(B, Lg, "rgb", precision=precision, device=dev)
     eng = net.engine
-    i = [k for k, st in enumerate(eng.fwd_sched.steps) if E._names(st) == ["maxpool28"]][0]
+    i = [k for k, st in enumerate(eng.fwd_sched.steps) if PL._names(st) == ["maxpool28"]][0]
     new_step = eng.fwd_sched.steps[i]
     f14, p28, P = eng.buf["F14"], eng.buf["p28"], eng.P
 
     def old_fn(stream):
-        L.check(old.offk_maxpool3s2_fwd(E._ptr(f14), P, 256, 14, 14, 1056, 800, E._ptr(p28), stream), "maxpool3s2")
-    old_step = E._nm(old_fn, "maxpool28", reads=new_step.reads, writes=new_step.writes, lane=new_step.lane)
+        L.check(old.offk_maxpool3s2_fwd(PL._ptr(f14), P, 256, 14, 14, 1056, 800, PL._ptr(p28), stream), "maxpool3s2")
+    old_step = PL._nm(old_fn, "maxpool28", reads=new_step.reads, writes=new_step.writes, lane=new_step.lane)
     taps = {k: v.to(dev) for k, v in O.make_taps(3, B, Lg).items()}
     target = torch.randint(0, 101, (B * (Lg - 1),), device=dev)
 

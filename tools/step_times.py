@@ -9,7 +9,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import off_b200  # noqa
-from off_b200 import engine as E
+from off_b200 import engine as E, plan as PL
 
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 48
 Lg = int(sys.argv[2]) if len(sys.argv) > 2 else 3
@@ -31,7 +31,7 @@ for _ in range(2):
     eng.forward(train=True, seed=1)
     eng.backward(g7, g14)
 steps = list(eng.fwd_steps) + list(eng.bwd_steps)
-names = ["+".join(E._names(s)) for s in steps]
+names = ["+".join(PL._names(s)) for s in steps]
 acc = [0.0] * len(steps)
 st = torch.cuda.current_stream()
 h = C.c_void_p(st.cuda_stream)
