@@ -84,12 +84,13 @@ int offk_device_info(int* sm_count, int* cc_major, int* cc_minor, long long* l2_
  * Epilogue, in this order, each step optional:
  *   v = D[m,n] + bias[n]
  *   v = max(v,0)                         if n <  relu_pre_cols
- *   v = gate[g] > 0 ? v : 0              if gate && gate_first  && n >= gate_col0   (ReLU')
- *   v = v + addend[a_row + a_col]        if addend
- *   v = gate[g] > 0 ? v : 0              if gate && !gate_first && n >= gate_col0
+ *   v = gate[o] > 0 ? v : 0              if gate && gate_first  && n >= gate_col0   (ReLU')
+ *   v = v + addend[add_row[m] + add_col[n]]   if addend
+ *   v = gate[o] > 0 ? v : 0              if gate && !gate_first && n >= gate_col0
  *   v = max(v,0)                         if relu_post
- *   out = v   (atomic add when split_k > 1 or atomic_out; then bias / activations are NOT applied)
- * gate / addend use (gate_row,gate_col) / (add_row,add_col) or, when NULL, the out tables.
+ *   out[o] = v   (atomic add when split_k > 1 or atomic_out; then bias / activations are NOT applied)
+ * o = out_row[m] + out_col[n]: the gate is read at the output's own element.  A NULL add_row / add_col stands for the
+ * out table.
  *
  * Table padding contract (so the kernels never bounds-check an index): a_row has ceil(M/128)*128 entries, a_col
  * and b_col have ceil(K/32)*32 + 64 entries, b_row has ceil(N/256)*256 entries.  Padding entries of a_row /
@@ -131,8 +132,6 @@ typedef struct offk_gemm {
   const float* bias;      /* [N] or NULL */
   int32_t relu_pre_cols;
   const float* gate;
-  const int32_t* gate_row;
-  const int32_t* gate_col;
   int32_t gate_col0;
   int32_t gate_first;
   const float* addend;
@@ -155,7 +154,7 @@ typedef struct offk_gemm {
    *   zero-initialised `out`; the last one to arrive re-reads the summed tile and applies the epilogue above (bias, ReLU
    *   prefix, gate, addend, ReLU) in place -- so bias / activation ARE applied although split_k > 1.
    * aux_out: a second output written where the final value v of an element is produced (directly, or by the split-K
-   *   finisher):  aux_out[aux_row[m] + aux_col0 + n] = max(v + aux_addend[out_row[m] + out_col[n]], 0)
+   *   finisher):  aux_out[aux_row[m] + n] = max(v + aux_addend[out_row[m] + out_col[n]], 0)
    *   (aux_row NULL: the out_row table; aux_addend NULL: 0).  RGB_OFF.py:658 (the ReLU'd copy of motion_conv_trans_28's
    *   pre-activation output, which :665 also consumes raw) and :779-780,832 (sum_14b = relu(sum_14a + relu(conv3_14b)) written
    *   into the 7x7 fusion buffer while the inner ReLU output is kept for the backward pass). */
@@ -163,8 +162,6 @@ typedef struct offk_gemm {
   float* aux_out;
   const int32_t* aux_row;
   const float* aux_addend;
-  int32_t aux_col0;
-  int32_t reserved2;
 } offk_gemm_t;
 
 int offk_gather_gemm(const offk_gemm_t* g, int precision, void* stream);
@@ -276,8 +273,8 @@ typedef struct offk_stencil {
   uint64_t seed;
   const uint8_t* keep_mask; /* [P, K*Cs, H, W] (NCHW order) for OFFK_DROP_MASK */
   const uint64_t* seed_dev; /* OFFK_DROP_SEED: NULL, or a device word added to `seed` when the kernel runs -- the per-step
-                               part of the seed then lives in device memory (offk_seed_set / offk_seed_advance), so a
-                               captured CUDA graph draws fresh masks on every replay while `seed` stays the call site's salt */
+                               part of the seed then lives in device memory (offk_seed_set), so a captured CUDA graph
+                               draws fresh masks on every replay while `seed` stays the call site's salt */
 } offk_stencil_t;
 
 int offk_stencil_diff_fwd(const offk_stencil_t* s, const float* g, const float* d, const float* w,
@@ -324,16 +321,9 @@ int offk_stencil_diff_bwd(const offk_stencil_t* s, const float* dout, const floa
 int offk_avgpool_drop_fwd(const float* x, int P, int C, int HW, int x_ctot, int x_coff, int drop_mode,
                           const uint8_t* keep_mask, uint64_t seed, const uint64_t* seed_dev, float drop_p, float keep_scale,
                           float* out, void* stream);
-/* dx[p, coff+c, :] = gate( dx_in + drop'(dpooled[p,c]) / HW ) ; dx_in = dx itself when accumulate != 0,
- * gate = (act[p, coff+c, :] > 0) when act != NULL (ReLU' of the producer). dpooled may be NULL (gate only). */
-int offk_avgpool_drop_bwd(const float* dpooled, int P, int C, int HW, int ctot, int coff, int drop_mode,
-                          const uint8_t* keep_mask, uint64_t seed, const uint64_t* seed_dev, float drop_p, float keep_scale,
-                          const float* act, int accumulate, float* dx, void* stream);
 /* seed_dev (may be NULL) as in offk_stencil_t: the effective seed is seed + *seed_dev, read when the kernel runs.
- * offk_seed_set stores `value` into the device word; offk_seed_advance replaces it by the next value of a splitmix64
- * sequence (the first node of a captured training step: every replay gets its own dropout masks). */
+ * offk_seed_set stores `value` into the device word. */
 int offk_seed_set(uint64_t* state, uint64_t value, void* stream);
-int offk_seed_advance(uint64_t* state, void* stream);
 /* One head in ONE launch (SURVEY K6): global_pool -> dropout -> fc_action_motion* (-> ConsensusModule('avg') over the T
  * frame pairs of a clip): RGB_OFF.py:784-787, 790-793, 844-847; Flow_OFF.py:867-876; basic_ops.py:21-22.
  *   pooled[p, c]  = drop( mean_hw x[p, hw, x_coff + c] )                (written when non-NULL: the backward needs it)
@@ -389,9 +379,8 @@ int offk_add_relu_slice(const float* a, const float* b, float* dst, int dst_ctot
 
 /* Conv weights: the reference's OIHW [cout,cin,kh,kw] <-> OHWI [cout,kh,kw,cin], the K order of the channels-last
  * implicit GEMM.  to_ohwi = 1: dst(OHWI) = src(OIHW) (before forward); 0: dst(OIHW) = src(OHWI);
- * 2: dst(OIHW) += src(OHWI) (weight gradients) */
-int offk_permute_weight(const float* src, float* dst, int cout, int cin, int kh, int kw, int to_ohwi, void* stream);
-/* n (<= 16) weights in ONE launch, same to_ohwi for all (the OHWI -> OIHW accumulation of every KxK weight gradient
+ * 2: dst(OIHW) += src(OHWI) (weight gradients).
+ * n (<= 16) weights in ONE launch, same to_ohwi for all (the OHWI -> OIHW accumulation of every KxK weight gradient
  * after the backward pass) */
 typedef struct offk_permute {
   const float* src;

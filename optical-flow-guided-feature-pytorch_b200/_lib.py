@@ -32,14 +32,12 @@ class OffkGemm(C.Structure):
         ("b_src", C.c_void_p), ("b_row", C.c_void_p), ("b_col", C.c_void_p), ("b_mode", C.c_int32),
         ("out", C.c_void_p), ("out_row", C.c_void_p), ("out_col", C.c_void_p),
         ("bias", C.c_void_p), ("relu_pre_cols", C.c_int32),
-        ("gate", C.c_void_p), ("gate_row", C.c_void_p), ("gate_col", C.c_void_p),
-        ("gate_col0", C.c_int32), ("gate_first", C.c_int32),
+        ("gate", C.c_void_p), ("gate_col0", C.c_int32), ("gate_first", C.c_int32),
         ("addend", C.c_void_p), ("add_row", C.c_void_p), ("add_col", C.c_void_p),
         ("relu_post", C.c_int32), ("atomic_out", C.c_int32),
         ("ones_row_out", C.c_void_p),
         ("split_k", C.c_int32), ("tile_n", C.c_int32), ("out_vec", C.c_int32), ("reserved", C.c_int32),
         ("finish_counter", C.c_void_p), ("aux_out", C.c_void_p), ("aux_row", C.c_void_p), ("aux_addend", C.c_void_p),
-        ("aux_col0", C.c_int32), ("reserved2", C.c_int32),
     ]
 
 
@@ -109,14 +107,11 @@ _PROTOS = {
     "offk_stencil_diff_bwd_batch": (C.c_int, [C.c_int, C.POINTER(OffkStencil), C.POINTER(OffkStencilIO), _P]),
     "offk_avgpool_drop_fwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_uint64, _P,
                                         C.c_float, C.c_float, _P, _P]),
-    "offk_avgpool_drop_bwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_uint64, _P,
-                                        C.c_float, C.c_float, _P, C.c_int, _P, _P]),
     "offk_head_fwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_uint64, _P, C.c_float,
                                 C.c_float, _P, _P, C.c_int, C.c_int, _P, _P, _P, _P]),
     "offk_head_bwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_uint64, _P, C.c_float,
                                 C.c_float, _P, C.c_int, C.c_int, _P, _P, C.c_int, _P, _P, _P, _P]),
     "offk_seed_set": (C.c_int, [_P, C.c_uint64, _P]),
-    "offk_seed_advance": (C.c_int, [_P, _P]),
     "offk_pool3_nhwc": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                   _P, C.c_int, C.c_int, _P]),
     "offk_segment_mean_fwd": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, _P]),
@@ -132,7 +127,6 @@ _PROTOS = {
     "offk_gather_copy": (C.c_int, [_P, _P, _P, C.c_longlong, _P]),
     "offk_tf32_residual": (C.c_int, [_P, _P, C.c_longlong, _P]),
     "offk_permute_weight_batch": (C.c_int, [C.c_int, C.POINTER(OffkPermute), C.c_int, _P]),
-    "offk_permute_weight": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "offk_drop_keep_host": (C.c_int, [C.c_uint64, C.c_uint64, C.c_float]),
     "offk_ce_loss_fwd_bwd": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_float, _P, _P, _P]),
     "offk_grad_sumsq": (C.c_int, [_P, C.c_longlong, _P, _P]),

@@ -6,13 +6,12 @@ namespace offk {
 
 // Per-row state of the epilogue (one accumulator row m).
 struct EpiRow {
-  int out, gate, add;
+  int out, add;
   bool ones;
 };
 __device__ __forceinline__ EpiRow epi_row(const offk_gemm_t& g, int m) {
   EpiRow r;
   r.out = g.out_row[m];
-  r.gate = g.gate ? (g.gate_row ? g.gate_row[m] : r.out) : 0;
   r.add = g.addend ? (g.add_row ? g.add_row[m] : r.out) : 0;
   r.ones = (m == g.a_ones_row);
   return r;
@@ -33,7 +32,7 @@ __device__ __forceinline__ void epi_store(const offk_gemm_t& g, const EpiRow& r,
   if (n < g.relu_pre_cols) v = fmaxf(v, 0.f);
   float gate = 1.f;
   const bool gated = g.gate && n >= g.gate_col0;
-  if (gated) gate = __ldg(g.gate + (r.gate + (g.gate_col ? g.gate_col[n] : oc)));
+  if (gated) gate = __ldg(g.gate + (r.out + oc));
   if (gated && g.gate_first) v = gate > 0.f ? v : 0.f;
   if (g.addend) v += __ldg(g.addend + (r.add + (g.add_col ? g.add_col[n] : oc)));
   if (gated && !g.gate_first) v = gate > 0.f ? v : 0.f;

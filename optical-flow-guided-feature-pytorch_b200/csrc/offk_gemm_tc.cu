@@ -212,10 +212,6 @@ struct LoaderB {
   }
 };
 
-#ifdef OFFK_DEBUG_DUMP
-__device__ float* g_offk_dump = nullptr;   // bring-up only: CTA (0,0,0) copies its stage-0 shared memory here
-#endif
-
 // ---------------------------------------------------------------------------- kernel
 // X3 = OFFK_PREC_TF32X3: every stage holds [A | B | A_lo | B_lo].  Each producer thread turns the chunks it copied itself
 // into their tf32 residuals (offk_tc.cuh) once its cp.async groups have landed -- `la` K-blocks behind the issue front --
@@ -366,13 +362,12 @@ gather_gemm_tc_kernel(const offk_gemm_t g, int bn, int stages, int kb_per_split,
     const int m = m0 + quad * 32 + lane;
     const bool mvalid = m < g.M;
     // table entries first: they are in flight while the last MMAs retire
-    EpiRow er = {0, 0, 0, false};
+    EpiRow er = {0, 0, false};
     if (mvalid) er = epi_row(g, m);
     const bool atomic = (g.split_k > 1) || g.atomic_out;
     const bool vec = g.out_vec == 1 && !er.ones;
     // out_vec contract: column tables are contiguous (col[n] = col[0] + n)
     const int oc0 = __ldg(g.out_col);
-    const int gc0 = g.gate ? (g.gate_col ? __ldg(g.gate_col) : oc0) : 0;
     const int ac0 = g.addend ? (g.add_col ? __ldg(g.add_col) : oc0) : 0;
     mbar_wait(smem_u32(&sh->accum_full), 0u);
     tc_fence_after();
@@ -390,7 +385,7 @@ gather_gemm_tc_kernel(const offk_gemm_t g, int bn, int stages, int kb_per_split,
           const int n = nb + 4 * j;
           ad[j] = f4zero(); gt[j] = make_float4(1.f, 1.f, 1.f, 1.f);
           if (n < g.N && !atomic) {
-            if (g.gate && n >= g.gate_col0) gt[j] = ldg128(g.gate + (er.gate + gc0 + n));
+            if (g.gate && n >= g.gate_col0) gt[j] = ldg128(g.gate + (er.out + oc0 + n));
             if (g.addend) ad[j] = ldg128(g.addend + (er.add + ac0 + n));
           }
         }
@@ -412,22 +407,8 @@ gather_gemm_tc_kernel(const offk_gemm_t g, int bn, int stages, int kb_per_split,
             asm volatile("red.global.add.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(o), "f"(x.x), "f"(x.y), "f"(x.z), "f"(x.w) : "memory");
             continue;
           }
-          const bool gated = g.gate && n >= g.gate_col0;
-          if (g.bias) {
-            const float4 b = ldg128(g.bias + n);
-            x.x += b.x; x.y += b.y; x.z += b.z; x.w += b.w;
-          }
-          if (n < g.relu_pre_cols) x = f4relu(x);
-          const float4 t = gt[j];
-          if (gated && g.gate_first) {
-            x.x = t.x > 0.f ? x.x : 0.f; x.y = t.y > 0.f ? x.y : 0.f; x.z = t.z > 0.f ? x.z : 0.f; x.w = t.w > 0.f ? x.w : 0.f;
-          }
-          x.x += ad[j].x; x.y += ad[j].y; x.z += ad[j].z; x.w += ad[j].w;
-          if (gated && !g.gate_first) {
-            x.x = t.x > 0.f ? x.x : 0.f; x.y = t.y > 0.f ? x.y : 0.f; x.z = t.z > 0.f ? x.z : 0.f; x.w = t.w > 0.f ? x.w : 0.f;
-          }
-          if (g.relu_post) x = f4relu(x);
-          *reinterpret_cast<float4*>(o) = x;
+          const float4 bias4 = g.bias ? ldg128(g.bias + n) : f4zero();
+          *reinterpret_cast<float4*>(o) = epi_act4(g, x, n, bias4, gt[j], ad[j], g.gate && n >= g.gate_col0);
         }
       } else if (mvalid) {
         if (atomic && !er.ones) {
@@ -444,12 +425,6 @@ gather_gemm_tc_kernel(const offk_gemm_t g, int bn, int stages, int kb_per_split,
       }
     }
   }
-#ifdef OFFK_DEBUG_DUMP
-  if (g_offk_dump && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && warp < 8) {
-    const float* sp = reinterpret_cast<const float*>(smem_raw + (smem_base - smem_u32(smem_raw)));
-    for (uint32_t i = tid; i < stage_bytes / 4; i += TC_PRODUCERS) g_offk_dump[i] = sp[i];
-  }
-#endif
   tc_fence_before();
   __syncthreads();
   if (warp == 8) {
@@ -532,7 +507,3 @@ int launch_gemm_tc(const offk_gemm_t& g, cudaStream_t st, bool x3) {
 }
 
 }  // namespace offk
-
-#ifdef OFFK_DEBUG_DUMP
-extern "C" int offk_debug_set_dump(float* p) { return (int)cudaMemcpyToSymbol(offk::g_offk_dump, &p, sizeof(p)); }
-#endif

@@ -136,27 +136,18 @@ struct TmShared {
   float bias[256];                 // the tile's bias values (vector epilogue)
 };
 
-// Final value of 4 consecutive elements (one accumulator row, columns n..n+3): the epilogue of offk.h, then the optional
-// second output.  out_base / aux_base: element offsets of the row in `out` / `aux_out` (column 0).
+// Final value of 4 consecutive elements (one accumulator row, columns n..n+3): the epilogue of offk.h (epi_act4), then the
+// optional second output.  out_base / aux_base: element offsets of the row in `out` / `aux_out` (column 0).
 __device__ __forceinline__ float4 epi_final4(const offk_gemm_t& g, float4 v, int n, const float4& bias4, const float4& t,
                                              const float4& ad, bool gated, int out_base, int aux_base) {
-  v.x += bias4.x; v.y += bias4.y; v.z += bias4.z; v.w += bias4.w;
-  if (n < g.relu_pre_cols) v = f4relu(v);               // relu_pre_cols is a multiple of 4 on this path
-  if (gated && g.gate_first) {
-    v.x = t.x > 0.f ? v.x : 0.f; v.y = t.y > 0.f ? v.y : 0.f; v.z = t.z > 0.f ? v.z : 0.f; v.w = t.w > 0.f ? v.w : 0.f;
-  }
-  v.x += ad.x; v.y += ad.y; v.z += ad.z; v.w += ad.w;
-  if (gated && !g.gate_first) {
-    v.x = t.x > 0.f ? v.x : 0.f; v.y = t.y > 0.f ? v.y : 0.f; v.z = t.z > 0.f ? v.z : 0.f; v.w = t.w > 0.f ? v.w : 0.f;
-  }
-  if (g.relu_post) v = f4relu(v);
+  v = epi_act4(g, v, n, bias4, t, ad, gated);
   if (g.aux_out) {
     float4 a = v;
     if (g.aux_addend) {
       const float4 x = ldg128(g.aux_addend + (out_base + n));
       a.x += x.x; a.y += x.y; a.z += x.z; a.w += x.w;
     }
-    *reinterpret_cast<float4*>(g.aux_out + (aux_base + g.aux_col0 + n)) = f4relu(a);
+    *reinterpret_cast<float4*>(g.aux_out + (aux_base + n)) = f4relu(a);
   }
   return v;
 }
@@ -180,7 +171,6 @@ __device__ __noinline__ void splitk_finish(const offk_gemm_t& g, uint32_t* flag_
   if (!*flag) return;
   __threadfence();
   const int oc0 = __ldg(g.out_col);
-  const int gc0 = g.gate ? (g.gate_col ? __ldg(g.gate_col) : oc0) : 0;
   const int ac0 = g.addend ? (g.add_col ? __ldg(g.add_col) : oc0) : 0;
   const int c4n = bn >> 2;                                 // float4 columns of the tile
   // thread -> (row, float4 column): consecutive threads walk a row (coalesced), 256 threads cover 256 / c4n rows per pass
@@ -193,7 +183,7 @@ __device__ __noinline__ void splitk_finish(const offk_gemm_t& g, uint32_t* flag_
     float* o = g.out + (er.out + oc0 + n);
     const float4 v = __ldcg(reinterpret_cast<const float4*>(o));
     const float4 bias4 = g.bias ? ldg128(g.bias + n) : f4zero();
-    const float4 t = gated ? ldg128(g.gate + (er.gate + gc0 + n)) : make_float4(1.f, 1.f, 1.f, 1.f);
+    const float4 t = gated ? ldg128(g.gate + (er.out + oc0 + n)) : make_float4(1.f, 1.f, 1.f, 1.f);
     const float4 ad4 = g.addend ? ldg128(g.addend + (er.add + ac0 + n)) : f4zero();
     *reinterpret_cast<float4*>(o) = epi_final4(g, v, n, bias4, t, ad4, gated, er.out + oc0, aux_base);
   }
@@ -624,21 +614,20 @@ tma_gemm_kernel(const __grid_constant__ CUtensorMap tma, const __grid_constant__
       const int rsub = lane >> 3, cq = lane & 7;                 // read-back: 4 rows per warp pass, 8 float4 per row
       const int nchunks = (bn + 31) >> 5;
       const int oc0 = __ldg(g.out_col);
-      const int gc0 = g.gate ? (g.gate_col ? __ldg(g.gate_col) : oc0) : 0;
       const int ac0 = g.addend ? (g.add_col ? __ldg(g.add_col) : oc0) : 0;
       // The four output rows this thread stores, their table entries and the column bases are fetched while the main
       // loop still runs (they sat on the critical path of every chunk before).  out_vec contract: the column tables are
       // contiguous, col[n] = col[0] + n.
-      int r_out[TC_BM / 32], r_gate[TC_BM / 32], r_add[TC_BM / 32], r_aux[TC_BM / 32];
+      int r_out[TC_BM / 32], r_add[TC_BM / 32], r_aux[TC_BM / 32];
       bool r_ok[TC_BM / 32];
 #pragma unroll
       for (int it = 0; it < TC_BM / 32; ++it) {
         const int m = m0 + it * 32 + ew * 4 + rsub;
         r_ok[it] = m < m_lim;
-        r_out[it] = r_gate[it] = r_add[it] = r_aux[it] = 0;
+        r_out[it] = r_add[it] = r_aux[it] = 0;
         if (r_ok[it]) {
           const EpiRow er = epi_row(g, m);
-          r_out[it] = er.out; r_gate[it] = er.gate; r_add[it] = er.add;
+          r_out[it] = er.out; r_add[it] = er.add;
           r_aux[it] = g.aux_out ? (g.aux_row ? __ldg(g.aux_row + m) : er.out) : 0;
         }
       }
@@ -675,7 +664,7 @@ tma_gemm_kernel(const __grid_constant__ CUtensorMap tma, const __grid_constant__
           gt[it] = make_float4(1.f, 1.f, 1.f, 1.f);
           ad[it] = f4zero();
           if (nvalid && r_ok[it] && !atomic) {
-            if (gated) gt[it] = ldg128(g.gate + (r_gate[it] + gc0 + n));
+            if (gated) gt[it] = ldg128(g.gate + (r_out[it] + oc0 + n));
             if (g.addend) ad[it] = ldg128(g.addend + (r_add[it] + ac0 + n));
           }
         }
@@ -730,7 +719,7 @@ tma_gemm_kernel(const __grid_constant__ CUtensorMap tma, const __grid_constant__
     } else {
       const int m = m0 + quad * 32 + lane;
       const bool mvalid = m < m_lim;
-      EpiRow er = {0, 0, 0, false};
+      EpiRow er = {0, 0, false};
       if (mvalid) er = epi_row(g, m);
       split_loop();
       mbar_wait(smem_u32(&sh->accum_full), 0u);
@@ -1001,7 +990,7 @@ extern "C" int offk_tma_gemm(const offk_tgemm_t* t, void* stream) {
   OFFK_REQUIRE(g.out_vec == 1 || (!g.finish_counter && !g.aux_out), "tma_gemm: finish_counter / aux_out need out_vec = 1");
   OFFK_REQUIRE(!g.finish_counter || (g.split_k > 1 && !g.atomic_out), "tma_gemm: finish_counter is for split_k > 1 without atomic_out");
   OFFK_REQUIRE(!g.aux_out || g.finish_counter || (g.split_k <= 1 && !g.atomic_out), "tma_gemm: aux_out needs a final value (no raw accumulation)");
-  if (g.aux_out) OFFK_REQUIRE((reinterpret_cast<uintptr_t>(g.aux_out) & 15u) == 0 && (g.aux_col0 & 3) == 0, "tma_gemm: aux_out alignment");
+  if (g.aux_out) OFFK_REQUIRE((reinterpret_cast<uintptr_t>(g.aux_out) & 15u) == 0, "tma_gemm: aux_out alignment");
   const int bn = t->prepared;
   TmGeom geo;
   geo.a_kind = t->a_kind; geo.a_coff = t->a_coff; geo.cblocks = t->cin > 0 ? t->cin / TC_BK : 1; geo.kw = t->kw > 0 ? t->kw : 1;

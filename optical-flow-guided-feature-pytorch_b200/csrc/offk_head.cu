@@ -13,9 +13,9 @@ __device__ __forceinline__ float keep_factor(int mode, const uint8_t* mask, uint
 }
 
 // the per-step word of the dropout seed lives in device memory (offk.h: seed_dev)
-__global__ void seed_update_kernel(uint64_t* state, uint64_t value, int advance) {
+__global__ void seed_update_kernel(uint64_t* state, uint64_t value) {
   pdl_sync();
-  *state = advance ? *state + 0x9E3779B97F4A7C15ull : value;   // a Weyl sequence; drop_hash64 does the mixing
+  *state = value;
 }
 
 // thread per (p, c); x is channels-last [P, HW, ctot]: consecutive threads read consecutive channels
@@ -32,27 +32,6 @@ __global__ void avgpool_drop_fwd_kernel(const float* __restrict__ x, int P, int 
   for (int h = 0; h < HW; ++h) s += __ldg(xp + (size_t)h * ctot);
   const float k = keep_factor(mode, mask, seed, drop_threshold16(drop_p), (size_t)i, scale);
   out[i] = (s / (float)HW) * k;
-}
-
-__global__ void avgpool_drop_bwd_kernel(const float* __restrict__ dpooled, int P, int C, int HW, int ctot, int coff,
-                                        int mode, const uint8_t* __restrict__ mask, uint64_t seed,
-                                        const uint64_t* __restrict__ seed_dev, float drop_p,
-                                        float scale, const float* __restrict__ act, int accumulate,
-                                        float* __restrict__ dx) {
-  pdl_sync();
-  if (seed_dev) seed += __ldg(seed_dev);
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const size_t total = (size_t)P * C * HW;
-  if (i >= total) return;
-  const int c = (int)(i % C);
-  const size_t ph = i / C;            // p*HW + hw
-  const size_t pc = (ph / HW) * C + c;
-  const size_t o = ph * ctot + coff + c;
-  float v = 0.f;
-  if (dpooled) v = __ldg(dpooled + pc) * keep_factor(mode, mask, seed, drop_threshold16(drop_p), pc, scale) / (float)HW;
-  if (accumulate) v += dx[o];
-  if (act) v = __ldg(act + o) > 0.f ? v : 0.f;
-  dx[o] = v;
 }
 
 // 3x3 pool over a channel slice of a channels-last tensor, ceil-mode output, one thread per (output pixel, channel quad):
@@ -377,12 +356,6 @@ __device__ __forceinline__ void permute_weight_block(const float* __restrict__ s
     }
   }
 }
-__global__ void __launch_bounds__(256)
-permute_weight_kernel(const float* __restrict__ src, float* __restrict__ dst, int cout, int cin, int rq, int to_ohwi) {
-  pdl_sync();
-  extern __shared__ float tile[];                       // [32][rq] in OIHW order (rq is odd on this path: no conflicts)
-  permute_weight_block(src, dst, cin, rq, to_ohwi, blockIdx.y, blockIdx.x * 32, tile);
-}
 // several weights in one launch: block -> (weight, output channel, 32-channel group)
 constexpr int PW_MAX = 16;
 struct PermuteBatch {
@@ -410,13 +383,8 @@ using namespace offk;
 
 extern "C" int offk_seed_set(uint64_t* state, uint64_t value, void* stream) {
   OFFK_REQUIRE(state != nullptr, "seed_set: null state");
-  (void)launch_pdl(seed_update_kernel, dim3(1), dim3(1), 0, as_stream(stream), state, value, 0);
+  (void)launch_pdl(seed_update_kernel, dim3(1), dim3(1), 0, as_stream(stream), state, value);
   return OFFK_LAUNCH_CHECK("seed_set");
-}
-extern "C" int offk_seed_advance(uint64_t* state, void* stream) {
-  OFFK_REQUIRE(state != nullptr, "seed_advance: null state");
-  (void)launch_pdl(seed_update_kernel, dim3(1), dim3(1), 0, as_stream(stream), state, (uint64_t)0, 1);
-  return OFFK_LAUNCH_CHECK("seed_advance");
 }
 
 extern "C" int offk_avgpool_drop_fwd(const float* x, int P, int C, int HW, int x_ctot, int x_coff, int drop_mode,
@@ -427,17 +395,6 @@ extern "C" int offk_avgpool_drop_fwd(const float* x, int P, int C, int HW, int x
   (void)launch_pdl(avgpool_drop_fwd_kernel, dim3(blocks_for((size_t)P * C, 128)), dim3(128), 0, as_stream(stream), 
       x, P, C, HW, x_ctot, x_coff, drop_mode, keep_mask, seed, seed_dev, drop_p, keep_scale, out);
   return OFFK_LAUNCH_CHECK("avgpool_drop_fwd");
-}
-
-extern "C" int offk_avgpool_drop_bwd(const float* dpooled, int P, int C, int HW, int ctot, int coff, int drop_mode,
-                                     const uint8_t* keep_mask, uint64_t seed, const uint64_t* seed_dev, float drop_p,
-                                     float keep_scale, const float* act, int accumulate, float* dx, void* stream) {
-  OFFK_REQUIRE(dx && P > 0 && C > 0 && HW > 0 && coff >= 0 && coff + C <= ctot, "avgpool_bwd: bad args");
-  OFFK_REQUIRE(drop_mode != OFFK_DROP_MASK || keep_mask, "avgpool_bwd: mask missing");
-  const size_t total = (size_t)P * C * HW;
-  (void)launch_pdl(avgpool_drop_bwd_kernel, dim3(blocks_for(total, 256)), dim3(256), 0, as_stream(stream), 
-      dpooled, P, C, HW, ctot, coff, drop_mode, keep_mask, seed, seed_dev, drop_p, keep_scale, act, accumulate, dx);
-  return OFFK_LAUNCH_CHECK("avgpool_drop_bwd");
 }
 
 extern "C" int offk_pool3_nhwc(const float* x, int n_img, int H, int W, int x_ctot, int x_coff, int C, int stride, int pad,
@@ -632,14 +589,4 @@ extern "C" int offk_permute_weight_batch(int n, const offk_permute_t* items, int
   OFFK_REQUIRE(blk < 2147483647LL, "permute_weight_batch: grid too large");
   (void)launch_pdl(permute_weight_batch_kernel, dim3((unsigned)blk), dim3(256), (size_t)32 * rq_max * sizeof(float), as_stream(stream), pb, to_ohwi);
   return OFFK_LAUNCH_CHECK("permute_weight_batch");
-}
-
-extern "C" int offk_permute_weight(const float* src, float* dst, int cout, int cin, int kh, int kw, int to_ohwi,
-                                   void* stream) {
-  OFFK_REQUIRE(src && dst && cout > 0 && cin > 0 && kh > 0 && kw > 0, "permute_weight: bad args");
-  OFFK_REQUIRE(kh * kw <= 256 && cout <= 65535, "permute_weight: filter too large");
-  dim3 grid((cin + 31) / 32, cout);
-  (void)launch_pdl(permute_weight_kernel, dim3(grid), dim3(256), (size_t)32 * kh * kw * sizeof(float), as_stream(stream), src, dst, cout, cin,
-                                                                                                 kh * kw, to_ohwi);
-  return OFFK_LAUNCH_CHECK("permute_weight");
 }

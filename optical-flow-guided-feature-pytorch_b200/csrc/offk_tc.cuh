@@ -309,35 +309,22 @@ __device__ __forceinline__ void epi_rows_contiguous(const offk_gemm_t& g, uint32
   }
 }
 
-// 4 consecutive output columns of one accumulator row, contiguous in memory (NHWC): float4 everywhere.
-__device__ __forceinline__ void epi_store4(const offk_gemm_t& g, const EpiRow& r, int n, float4 v, bool atomic) {
-  const int oc = g.out_col[n];
-  float* o = g.out + (r.out + oc);
-  if (atomic) {
-    asm volatile("red.global.add.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(o), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
-                 : "memory");
-    return;
-  }
-  if (g.bias) {
-    const float4 b = ldg128(g.bias + n);
-    v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
-  }
-  if (n < g.relu_pre_cols) v = f4relu(v);   // relu_pre_cols is a multiple of 4 on this path
-  const bool gated = g.gate && n >= g.gate_col0;
-  float4 gt = make_float4(1.f, 1.f, 1.f, 1.f);
-  if (gated) gt = ldg128(g.gate + (r.gate + (g.gate_col ? g.gate_col[n] : oc)));
+// The epilogue of offk.h on 4 consecutive columns n..n+3 of one accumulator row (out_vec = 1): the float4 form of
+// epi_store's op chain.  The caller fetches the operands -- bias4, gate values t and add4 are 0, 1 and 0 where absent --
+// and gated = the gate applies to these columns.
+__device__ __forceinline__ float4 epi_act4(const offk_gemm_t& g, float4 v, int n, const float4& bias4, const float4& t,
+                                           const float4& add4, bool gated) {
+  v.x += bias4.x; v.y += bias4.y; v.z += bias4.z; v.w += bias4.w;
+  if (n < g.relu_pre_cols) v = f4relu(v);               // relu_pre_cols is a multiple of 4 on this path
   if (gated && g.gate_first) {
-    v.x = gt.x > 0.f ? v.x : 0.f; v.y = gt.y > 0.f ? v.y : 0.f; v.z = gt.z > 0.f ? v.z : 0.f; v.w = gt.w > 0.f ? v.w : 0.f;
+    v.x = t.x > 0.f ? v.x : 0.f; v.y = t.y > 0.f ? v.y : 0.f; v.z = t.z > 0.f ? v.z : 0.f; v.w = t.w > 0.f ? v.w : 0.f;
   }
-  if (g.addend) {
-    const float4 a = ldg128(g.addend + (r.add + (g.add_col ? g.add_col[n] : oc)));
-    v.x += a.x; v.y += a.y; v.z += a.z; v.w += a.w;
-  }
+  v.x += add4.x; v.y += add4.y; v.z += add4.z; v.w += add4.w;
   if (gated && !g.gate_first) {
-    v.x = gt.x > 0.f ? v.x : 0.f; v.y = gt.y > 0.f ? v.y : 0.f; v.z = gt.z > 0.f ? v.z : 0.f; v.w = gt.w > 0.f ? v.w : 0.f;
+    v.x = t.x > 0.f ? v.x : 0.f; v.y = t.y > 0.f ? v.y : 0.f; v.z = t.z > 0.f ? v.z : 0.f; v.w = t.w > 0.f ? v.w : 0.f;
   }
   if (g.relu_post) v = f4relu(v);
-  *reinterpret_cast<float4*>(o) = v;
+  return v;
 }
 
 

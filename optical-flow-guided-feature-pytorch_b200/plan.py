@@ -88,7 +88,7 @@ def _auto_tile_n(M: int, N: int, tma: bool = False, x3: bool = False) -> int:
 
 
 def _bind_epilogue(step, plan, spc: T.GemmSpec, d, tabs, *, tma, a_src, b_src, out, bias=None, relu_pre_cols=0,
-                   gate=None, gate_tabs=None, gate_col0=0, gate_first=False, addend=None, add_tabs=None, relu_post=False,
+                   gate=None, gate_col0=0, gate_first=False, addend=None, add_tabs=None, relu_post=False,
                    atomic=False, ones_out=None, split_k=1, tile_n=0, name="", finish=False, aux=None, out_vec=None):
     """Fill the fields of offk_gemm_t ``d`` that the gather-fed and the TMA-fed kernel read alike (problem size, operand
     sources, output tables, epilogue, split-K), and annotate ``step`` as a plan step."""
@@ -98,8 +98,6 @@ def _bind_epilogue(step, plan, spc: T.GemmSpec, d, tabs, *, tma, a_src, b_src, o
     d.bias = bias.data_ptr() if bias is not None else None
     d.relu_pre_cols = relu_pre_cols
     d.gate = gate.data_ptr() if gate is not None else None
-    d.gate_row = gate_tabs[0].data_ptr() if gate_tabs else None
-    d.gate_col = gate_tabs[1].data_ptr() if gate_tabs else None
     d.gate_col0, d.gate_first = gate_col0, int(gate_first)
     d.addend = addend.data_ptr() if addend is not None else None
     d.add_row = add_tabs[0].data_ptr() if add_tabs else None
@@ -115,12 +113,12 @@ def _bind_epilogue(step, plan, spc: T.GemmSpec, d, tabs, *, tma, a_src, b_src, o
         bn = tile_n if tile_n else (256 if spc.N > 256 else (spc.N + 15) // 16 * 16)
         counter = torch.zeros(math.ceil(spc.M / 128) * math.ceil(spc.N / bn), dtype=torch.int32, device=plan.device)
         d.finish_counter = counter.data_ptr()
-    if aux is not None:                # (aux_out, aux_row table or None, aux_addend or None); aux_col0 stays 0
+    if aux is not None:                # (aux_out, aux_row table or None, aux_addend or None)
         d.aux_out = aux[0].data_ptr()
         d.aux_row = aux[1].data_ptr() if aux[1] is not None else None
         d.aux_addend = aux[2].data_ptr() if aux[2] is not None else None
     step.plan, step.name, step.spec = plan, name, spc
-    step._keep = (tabs, a_src, b_src, out, bias, gate, gate_tabs, addend, add_tabs, ones_out, counter, aux)
+    step._keep = (tabs, a_src, b_src, out, bias, gate, addend, add_tabs, ones_out, counter, aux)
     step.flops = 2.0 * spc.M * spc.N * spc.K
     step.launches = [name]
     step.reads = [a_src, b_src, addend, gate, bias, aux[2] if aux else None]
@@ -150,8 +148,8 @@ class Gemm:
 class TGemm:
     """A conv / FC on a channels-last input (or an NCHW tap) as ONE TMA-fed launch (offk_tma_gemm): A through a dense
     2-D tensor map (1x1, stride 1) or TMA im2col mode (KxK), B = the [cout, K] weight matrix; or the weight gradient with
-    A = im2col(x)^T / the NCHW tap and B = dY.  The epilogue reads the output tables (and the gate / addend / aux tables
-    a caller passes); the gather tables and load modes of offk_gemm_t stay 0."""
+    A = im2col(x)^T / the NCHW tap and B = dY.  The epilogue reads the output tables (and the addend / aux tables a caller
+    passes); the gather tables and load modes of offk_gemm_t stay 0."""
 
     @staticmethod
     def eligible(geom: T.ConvGeom, x_layout="nhwc") -> bool:

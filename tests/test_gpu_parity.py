@@ -796,8 +796,8 @@ def test_tma_gemm_split_k_finisher_and_second_output(dev, prec, tol, split, with
     if split > 1:
         d.finish_counter = counter.data_ptr()
     if with_aux:
-        # the row table of a channel-slice geometry already carries the slice offset (64): aux_col0 is an EXTRA column offset
-        d.aux_out, d.aux_row, d.aux_col0, d.aux_addend = aux.data_ptr(), aux_row.data_ptr(), 0, addend.data_ptr()
+        # the row table of a channel-slice geometry carries the slice offset (64)
+        d.aux_out, d.aux_row, d.aux_addend = aux.data_ptr(), aux_row.data_ptr(), addend.data_ptr()
     t.a_kind = L.TMA_A_IM2COL
     t.n_img, t.hin, t.win, t.ctot, t.cin = n, h, h, cin, cin
     t.kh, t.kw, t.stride, t.pad, t.hout, t.wout = k, k, 1, 1, h, h
